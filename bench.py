@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Default workload = BASELINE.json config 3: 10-word discrete HMM (N=4, M=256) Baum-Welch over
 100 000 synthetic sequences per word at T=200 (200 M frames per EM iteration), per GPU (weak
@@ -16,6 +16,11 @@ codewords resident in HBM; `e2e` = the same through the public packed-array API
 launching stream; `cpu_baseline` = the CPU oracle (numpy port of the reference) on a bounded
 sample using all host cores; secondary blocks `vq_encode`, `lbg`, `score` for the other
 BASELINE configs.
+
+--dump-outputs DIR writes what the timed iterations computed, as a caller of the resident trainer would
+read it after the last timed step (pi, A, B, the per-iteration log-likelihood statistic of every word and
+the per-sequence log-likelihoods of the last E-step), to DIR/<name>.npy; the inputs depend only on the
+arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -31,6 +36,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree (which may be read-only)
 sys.path.insert(0, ROOT)
 
 HBM_FALLBACK_GBS = 6650.0  # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
@@ -359,12 +365,15 @@ class Env:
 PHASES = ("bw_forward", "bw_exact", "bw_backward", "bw_reduce", "bw_allreduce", "bw_mstep")
 
 
-def time_baum_welch(env: Env, bw, steps: int, warmup: int, sampler=None):
+def time_baum_welch(env: Env, bw, steps: int, warmup: int, sampler=None, on_timed=None):
     """W untimed warm-up iterations, then `steps` iterations queued back to back between barrier + synchronize,
     CUDA events on the launching stream, profiling events OFF (this is `value`); then the same number of
-    iterations once more with the library's per-launch events on, for the per-kernel times of the roofline."""
+    iterations once more with the library's per-launch events on, for the per-kernel times of the roofline.
+    on_timed(bw) is called between the two, outside the timed region."""
     torch, lib, _lib = env.torch, env.lib, env._lib
-    cap = 1 << 14  # max_iterations of the calls below: never reached (a word that reaches it stops being trained)
+    done = int(bw.history(1)[1].max(initial=0))  # iterations the model already ran (max_iterations counts them too)
+    # max_iterations of the calls below: never reached (a word that reaches it stops being trained)
+    cap = max(1 << 14, done + warmup + 2 * steps + 1)
     bw.iterate(warmup, -1.0, cap, sync_each=False)
     env.barrier()
     l0 = lib.hmmb_launch_count()
@@ -376,6 +385,8 @@ def time_baum_welch(env: Env, bw, steps: int, warmup: int, sampler=None):
         env.barrier()
     ms = env.max_over_ranks(ev0.elapsed_time(ev1))
     launches = int(lib.hmmb_launch_count() - l0)
+    if on_timed is not None:
+        on_timed(bw)
     _lib.check(lib.hmmb_set_profiling(1))
     _lib.check(lib.hmmb_phase_reset())
     env.barrier()
@@ -388,6 +399,30 @@ def time_baum_welch(env: Env, bw, steps: int, warmup: int, sampler=None):
             phases[name] = {"ms_per_launch": pms / n, "launches": n}
     _lib.check(lib.hmmb_set_profiling(0))
     return ms / steps, launches, phases
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def bw_outputs(bw, iterations: int):
+    """What a caller of the resident trainer reads back after `iterations` EM iterations: the model, the
+    per-iteration log-likelihood statistic of every word and the per-sequence log-likelihoods of the last E-step."""
+    pi, A, B = bw.params()
+    hist, _ = bw.history(iterations)
+    return {"pi": pi, "A": A, "B": B, "ll_hist": hist, "seq_ll": bw.seq_ll()}
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Every array as out_dir/<name>.npy in float64, DUMP_LIMIT_BYTES in all at most: an array larger than its
+    share is cut to a fixed, seeded sample of its rows (leading axis), the same rows on every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // len(arrays) - 4096  # (room for the .npy header)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            rows = np.random.default_rng(0).choice(len(a), max(1, share // (a.nbytes // len(a))), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def bw_roofline(workload, family, phases, frames_rank, N, M, hbm_peak, peak_src):
@@ -649,7 +684,12 @@ def main():
     ap.add_argument("--workload", default="bw_c3", choices=list(WORKLOADS))
     ap.add_argument("--scale", type=float, default=1.0, help="fraction of the workload's sequences (debug)")
     ap.add_argument("--no-extras", action="store_true", help="headline + e2e only (no config 4 / strong / parity / shard / VQ / LBG / scoring / CPU blocks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     cfg = dict(WORKLOADS[args.workload])
     cfg["S"] = max(1, int(round(cfg["S"] * args.scale)))
     if args.impl == "reference":
@@ -698,7 +738,10 @@ def main():
         time.sleep(1.0)  # nvidia-smi needs about a second to start printing
     # single GPU: NVML thread every ~2 ms during the timed region; several ranks: an nvidia-smi child of rank 0
     clk = ClockSampler(local_rank) if world == 1 else None
-    ms_per_step, gpu_launches, phases = time_baum_welch(env, bw, args.steps, args.warmup, sampler=clk)
+    on_timed = None
+    if args.dump_outputs and rank == 0:
+        on_timed = lambda b: dump_outputs(args.dump_outputs, bw_outputs(b, args.warmup + args.steps))
+    ms_per_step, gpu_launches, phases = time_baum_welch(env, bw, args.steps, args.warmup, sampler=clk, on_timed=on_timed)
     if smi:
         time.sleep(0.05)
         smi.stop()
