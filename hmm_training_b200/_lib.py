@@ -11,7 +11,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("HMMB_LIB_PATH") or os.path.join(_HERE, "libhmmb200.so")  # override: kernel experiments
+LIB_PATH = os.path.join(_HERE, "libhmmb200.so")
 
 HMMB_OK = 0
 ERR_CUDA, ERR_ARG, ERR_OOM, ERR_EMPTY, ERR_RANGE, ERR_UNSUPPORTED = -1, -2, -3, -4, -5, -6

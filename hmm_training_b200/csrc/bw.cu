@@ -1,7 +1,6 @@
 // Host side of the Baum-Welch trainer and the forward scorer: sequence sorting/blocking,
 // device layout, the EM loop, and the C ABI declared in include/hmmb200.h.
 #include <algorithm>
-#include <chrono>
 #include <cstdlib>
 #include <functional>
 #include <memory>
@@ -54,14 +53,6 @@ __global__ void k_fill_i32(int32_t *p, int64_t n, int32_t v) {
 }
 
 // ---------------------------------------------------------------- scoring kernels
-// is every model's A upper-bidiagonal?  (device flag written by k_check_bidiag)
-__global__ void k_check_bidiag(const double *__restrict__ A, int W, int N, int32_t *__restrict__ not_bidiag) {
-    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < W * N * N; e += gridDim.x * blockDim.x) {
-        const int ij = e % (N * N), i = ij / N, j = ij % N;
-        if (j != i && j != i + 1 && A[e] > 0.0) *not_bidiag = 1;
-    }
-}
-
 // VECB: per-state error bound of the forward recursion (needed for utterances of thousands of frames); the scalar
 // bound is ~10 instructions per step cheaper and enough below SCORE4_SCALAR_BOUND_MAX_T frames (bw4_kernels.cuh)
 constexpr int SCORE4_SCALAR_BOUND_MAX_T = 1000;
@@ -99,9 +90,7 @@ k_score4(const Blk *__restrict__ blks, int nblk, int blocks_per_cta, const uint4
 // (score4_lean_run) for models that allow it; 8 warps per CTA, one model per CTA, M <= SCORE4R_MAX_M.
 // Shared memory: [M * 8] double2 (b0, b1), [M * 8] double2 (b2, b3), [M] per-codeword max, [M] support masks.
 constexpr int SCORE4R_WARPS = 8;
-#ifndef SCORE4R_MIN_CTAS
-#define SCORE4R_MIN_CTAS 2
-#endif
+constexpr int SCORE4R_MIN_CTAS = 2;
 constexpr int SCORE4R_REP = 8;
 constexpr int SCORE4R_MAX_M = 256;  // 64 KB of replicated B^T: three CTAs per SM
 template <bool BIDIAG, bool VECB>
@@ -269,7 +258,6 @@ struct EarlyUpload {
     int issued = 0;                 // chunks already queued on the copy stream
     size_t hi[MAX_CHUNKS] = {};     // end byte of each chunk
     cudaEvent_t ev[MAX_CHUNKS] = {};
-    cudaEvent_t t0 = nullptr;       // HMMB_TIMING: start of the upload (copy stream)
     bool active() const { return nchunk > 0; }
     // queue chunks [issued, upto) on the copy stream.  The first chunks go out before the host-side
     // sorting / blocking (PCIe works while the host does), the rest only after the (small)
@@ -306,27 +294,20 @@ struct PendingPrepare {
     int cta_end[MAX_STAGES] = {};    // CTA work items [.., cta_end) only touch those blocks
 };
 
-// stages of the pipelined first E-step (HMMB_PIPE_STAGES overrides).  The tail of a fit call behind the last upload chunk
+// Stages of the pipelined first E-step (N = 4 and left-to-right).  The tail of a fit call behind the last upload chunk
 // is the last stage's repack + forward + backward, and a stage launches whole work items: with the resident iterations'
 // list (two items per SM, one fat backward CTA each) a stage of config 3 kept a quarter of the SMs busy for the 1.5 ms one
 // item takes, and more stages only made that worse (4 stages 6.1 ms per fit call, 8 stages 8.0).  With the finer list the
 // staged E-step launches from (SeqSet::cta_begin_fine, about eight items per SM) the picture turns: 4 stages 5.75 ms,
-// 8 stages 5.50.
-static int pipeline_stages() {
-    const char *e = getenv("HMMB_PIPE_STAGES");
-    return e ? std::max(1, std::min(atoi(e), (int)PendingPrepare::MAX_STAGES)) : 8;
-}
-// left-to-right kernels (config 4, 200 MB of codewords + 131 MB of parameters up): 2 stages 16.1 ms per fit call,
-// 4 stages 14.0 - 14.6, 8 stages 13.85
-static int ltr_pipeline_stages() {
-    const char *e = getenv("HMMB_PIPE_STAGES");
-    return e ? std::max(1, std::min(atoi(e), (int)PendingPrepare::MAX_STAGES)) : 8;
-}
+// 8 stages 5.50.  Left-to-right kernels (config 4, 200 MB of codewords + 131 MB of parameters up): 2 stages 16.1 ms per
+// fit call, 4 stages 14.0 - 14.6, 8 stages 13.85.
+constexpr int PIPE_STAGES = 8;
+static_assert(PIPE_STAGES <= PendingPrepare::MAX_STAGES, "one upload chunk per stage");
 static int score_stages(bool want_ll) {
-    // 1 M utterances x 10 models, pinned buffers (scripts/score_stage_probe.py), 2 / 3 / 4 / 6 / 8 stages: 5.11 / 4.66 / 4.50 /
-    // 4.35 / 4.41 ms with the log-likelihood matrix going back stage by stage, 4.17 / 3.95 / 3.82 / 4.01 / 3.95 ms argmax only
-    const char *e = getenv("HMMB_SCORE_STAGES");
-    return e ? std::max(1, std::min(atoi(e), (int)PendingPrepare::MAX_STAGES)) : (want_ll ? 6 : 4);
+    // 1 M utterances x 10 models, pinned buffers, 2 / 3 / 4 / 6 / 8 stages: 5.11 / 4.66 / 4.50 / 4.35 / 4.41 ms with the
+    // log-likelihood matrix going back stage by stage, 4.17 / 3.95 / 3.82 / 4.01 / 3.95 ms argmax only (the probe script
+    // that swept this is in the history at commit 03a55a2)
+    return want_ll ? 6 : 4;
 }
 
 // ---------------------------------------------------------------- sequence set (shared by BW and scoring)
@@ -335,8 +316,6 @@ struct SeqSet {
     int N = 0, M = 0, NP = 0, sym_bytes = 1;
     bool special4 = false;            // blocked layout (32 same-word sequences per block), N = 4 kernels
     int ltr_ns = 0;                   // blocked layout for the left-to-right kernels with NS = ltr_ns states
-    bool peer_enc = false;            // packed entries carry the peer lane (trainer's N = 4 layout, M <= 256; bw4_kernels.cuh)
-    unsigned symmask() const { return peer_enc ? PEER_SYM_MASK : SYM_MASK; }
     bool blocked() const { return special4 || ltr_ns != 0; }
     std::vector<int32_t> order;       // sorted -> original
     std::vector<int64_t> seq_begin;   // per word [W+1] (sorted order)
@@ -396,13 +375,22 @@ static int h2d_join() {
 
 static int pick_np(int N) { return N <= 4 ? 4 : (N <= 8 ? 8 : (N <= 16 ? 16 : 32)); }
 
+// Is every one of the W row-major N x N matrices A upper-bidiagonal (a_ij > 0 only for j = i or j = i + 1, the
+// reference's left-to-right topology)?  Zeros of A stay zeros under re-estimation, so the answer holds for a whole fit;
+// it selects the kernel family.
+static bool upper_bidiagonal(const double *A, int W, int N) {
+    const size_t nA = (size_t)W * N * N;
+    for (size_t e = 0; e < nA; ++e) {
+        const int ij = (int)(e % (size_t)(N * N)), i = ij / N, j = ij % N;
+        if (j != i && j != i + 1 && A[e] > 0.0) return false;
+    }
+    return true;
+}
+
 // repack blocks [b0, b1) of the blocked layouts from the raw codewords (any input width)
 template <typename InT>
 static int launch_repack_typed(SeqSet &s, const InT *d_in, int b0, int b1, int *d_bad) {
-    if (s.peer_enc)
-        HMMB_LAUNCH("prepare", (k_repack_blocks4<InT, true>), b1 - b0, REPACK_WARPS * 32, 0, d_in, s.d_off, s.d_len, s.d_blks, b0, s.nblk, (uint4 *)s.d_obs, s.M, d_bad);
-    else
-        HMMB_LAUNCH("prepare", (k_repack_blocks4<InT, false>), b1 - b0, REPACK_WARPS * 32, 0, d_in, s.d_off, s.d_len, s.d_blks, b0, s.nblk, (uint4 *)s.d_obs, s.M, d_bad);
+    HMMB_LAUNCH("prepare", k_repack_blocks4<InT>, b1 - b0, REPACK_WARPS * 32, 0, d_in, s.d_off, s.d_len, s.d_blks, b0, s.nblk, (uint4 *)s.d_obs, s.M, d_bad);
     return HMMB_OK;
 }
 static int launch_repack_range(SeqSet &s, const void *d_in, int idx_bytes, int b0, int b1, int *d_bad) {
@@ -461,17 +449,13 @@ static int launch_prepare(SeqSet &s, const InT *d_in, int64_t nsym, int *d_bad, 
 // Sort sequences by (word, length desc), build blocks / CTA work items, move the codewords
 // to the device in the layout the kernels read.  word_of_seq == nullptr: a single "word"
 // (scoring: every utterance is scored against every model).
-static double now_ms() {
-    return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
-}
-
 enum SeqLayout { LAYOUT_GENERIC = 0, LAYOUT_AUTO = 1, LAYOUT_LTR = 2 };
 
 // can the left-to-right kernels (bwltr_kernels.cuh) hold this model shape?
 static bool ltr_shape_ok(int N, int M) {
     if (N != 8 && N != 16) return false;
     if (M > LTR_MAX_SYM) return false;
-    const size_t stage = (size_t)LTR_WARPS * LTR_STAGE_BUFS * 32 * (N * 8 + 16);
+    const size_t stage = (size_t)LTR_WARPS * 32 * (N * 8 + 16);
     const size_t smem_b = (size_t)M * N * 8 + stage + (size_t)2 * N * 8 + (size_t)LTR_WARPS * 2 * N * 8 + 64;
     return smem_b <= ctx().smem_optin && !getenv("HMMB_FORCE_GENERIC") && !getenv("HMMB_NO_LTR");
 }
@@ -480,8 +464,6 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
                         const int32_t *word_of_seq, int64_t R, int W, int N, int M, int layout, bool defer = false,
                         const std::function<int()> *mid_hook = nullptr, int max_stages = 2) {
     Ctx &c = ctx();
-    const bool timing = getenv("HMMB_TIMING") != nullptr;
-    const double t0 = now_ms();
     if (R < 0 || W <= 0 || !offsets || (R > 0 && !obs)) { set_error("bad sequence arguments"); return HMMB_ERR_ARG; }
     if (N < 1 || N > HMMB_MAX_STATES) { set_error("N=%d outside supported range 1..%d", N, HMMB_MAX_STATES); return HMMB_ERR_UNSUPPORTED; }
     if (M < 1 || M > 65536) { set_error("M=%d outside supported range 1..65536", M); return HMMB_ERR_UNSUPPORTED; }
@@ -490,8 +472,6 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
     s.sym_bytes = M <= 256 ? 1 : 2;
     s.special4 = layout == LAYOUT_AUTO && N == 4 && M <= BW4_MAX_M && !getenv("HMMB_FORCE_GENERIC");
     s.ltr_ns = (layout == LAYOUT_LTR) ? N : 0;
-    // (the scorer builds its sets with word_of_seq == nullptr and keeps the plain codeword | rank entries)
-    s.peer_enc = BWD4_PEER_ENC && s.special4 && word_of_seq != nullptr && M <= PEER_MAX_M;
 
     std::unique_ptr<EarlyUpload> up_owner(new EarlyUpload());
     EarlyUpload &up = *up_owner;
@@ -511,10 +491,6 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
             event_put(fence);
             const int nchunk = (int)std::min<size_t>(EarlyUpload::MAX_CHUNKS, std::max<size_t>(1, in_bytes >> 24));
             up.src = src;
-            if (timing) {
-                cudaEventCreate(&up.t0);
-                cudaEventRecord(up.t0, c.copy_stream);
-            }
             for (int k = 0; k < nchunk; ++k) {
                 up.hi[k] = k == nchunk - 1 ? in_bytes : ((in_bytes / nchunk) * (k + 1)) & ~size_t(255);
                 up.ev[k] = event_get();
@@ -524,8 +500,7 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
             // eight); the metadata goes next in the DMA queue, the rest of the codewords behind it.  The first stage of the
             // pipelined E-step cannot start before the metadata has landed: with two chunks ahead of it (the default
             // until late in round 2) that was 1.8 ms into the call, with one 1.5 ms — 5.6 -> 5.4 ms per fit call
-            const char *fe = getenv("HMMB_UPLOAD_FIRST");
-            HMMB_TRY(up.issue(fe ? std::max(1, atoi(fe)) : std::max(1, nchunk / 8)));
+            HMMB_TRY(up.issue(std::max(1, nchunk / 8)));
             c.h2d_on_copy = true;
         }
     }
@@ -666,8 +641,7 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         // CTA work items: ~2 per SM (N = 4) / ~4 per SM (left-to-right kernels, one 8-warp CTA per SM), at least one
         // warp-round each
         // (N = 4: one fat backward CTA per SM, about two waves; the forward kernel splits every item over FWD4_SPLIT CTAs)
-        static const int bw4_items_per_sm = getenv("HMMB_BW4_ITEMS_PER_SM") ? std::max(1, atoi(getenv("HMMB_BW4_ITEMS_PER_SM"))) : 2;
-        const int target = s.special4 ? c.sm_count * bw4_items_per_sm : c.sm_count * 4;
+        const int target = s.special4 ? c.sm_count * 2 : c.sm_count * 4;
         int bpc = std::max(1, (s.nblk + target - 1) / target);
         if (bpc > 1 || !s.special4) bpc = (bpc + cta_warps - 1) / cta_warps * cta_warps;
         s.cta_begin.assign(nwords + 1, 0);
@@ -676,9 +650,8 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         // takes waves x rounds-per-item: items rounded up to whole rounds left config 3 with 280 items of 7 rounds on 2 x 148
         // CTA slots — 14 rounds per SM for 13.2 rounds of work, 16 SMs idle in the second wave.  296 items of 105.6 blocks
         // are 6 full rounds and one with 10 of the 16 warps busy, which is shorter than a full one.
-        static const bool exact_items = !(getenv("HMMB_BW4_EXACT_ITEMS") && atoi(getenv("HMMB_BW4_EXACT_ITEMS")) == 0);
         std::vector<int> items_of_word;
-        if (s.special4 && exact_items && (int64_t)s.nblk >= (int64_t)target * cta_warps * 2) {
+        if (s.special4 && (int64_t)s.nblk >= (int64_t)target * cta_warps * 2) {
             items_of_word.assign(nwords, 0);
             std::vector<std::pair<double, int>> rem;
             int64_t assigned = 0;
@@ -731,8 +704,8 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         s.ncta = (int)work.size();
         s.ncta_fwd = (int)work_fwd.size();
         if (s.special4 && defer) {
-            static const int fine_items_per_sm = getenv("HMMB_BW4_STAGE_ITEMS_PER_SM") ? std::max(1, atoi(getenv("HMMB_BW4_STAGE_ITEMS_PER_SM"))) : 8;
-            int bpf = std::max(1, (s.nblk + c.sm_count * fine_items_per_sm - 1) / (c.sm_count * fine_items_per_sm));
+            const int fine_items = c.sm_count * 8;  // about eight per SM (SeqSet::cta_begin_fine)
+            int bpf = std::max(1, (s.nblk + fine_items - 1) / fine_items);
             if (bpf > 1) bpf = (bpf + cta_warps - 1) / cta_warps * cta_warps;
             if (bpf < bpc) {
                 s.cta_begin_fine.assign(nwords + 1, 0);
@@ -753,7 +726,6 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         }
     }
 
-    const double t1 = now_ms();
     // ---- device buffers
     HMMB_TRY(dev_alloc(&s.d_meta, meta_bytes));
     s.d_off = reinterpret_cast<int64_t *>(s.d_meta);
@@ -833,9 +805,6 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         }
         p->up = std::move(up_owner);
         s.pend = std::move(p);
-        if (timing)
-            fprintf(stderr, "[hmmb] seqset_build: host sort/blocking %.2f ms, deferred prepare in %d stages (R=%lld, frames=%lld)\n",
-                    t1 - t0, s.pend->nstage, (long long)R, (long long)s.frames);
         return HMMB_OK;
     }
     int rc = HMMB_OK;
@@ -854,9 +823,6 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         if (e != cudaSuccess) rc = cuda_fail(e, "prepare sync", __FILE__, __LINE__);
     }
     dev_free(d_tmp);
-    if (timing)
-        fprintf(stderr, "[hmmb] seqset_build: host sort/blocking %.2f ms, upload + repack %.2f ms (R=%lld, frames=%lld)\n",
-                t1 - t0, now_ms() - t1, (long long)R, (long long)s.frames);
     if (rc != HMMB_OK) return rc;
     if (bad) {
         set_error("codeword out of range: some observation is >= M=%d (reference: IndexError)", M);
@@ -1067,17 +1033,9 @@ int hmmb_bw_create_ex(hmmb_bw_t **out, const void *obs, int idx_bytes, int obs_o
     const bool have_params = pi0 && A0 && B0;
     // Pipelined create for the left-to-right kernels (N = 8 / 16): pinned host codewords, initial parameters given
     // and every A upper-bidiagonal.  Only the blocked layout is built, and its repack is left to the first E-step.
-    bool ltr_pipe = false;
-    if (h->has_ltr && (flags & HMMB_BW_PIPELINE_UPLOAD) && have_params && !obs_on_device && R > 0 && offsets && obs &&
-        offsets[R] > offsets[0] && !getenv("HMMB_FORCE_DENSE_A") && !getenv("HMMB_NO_LTR_PIPELINE") &&
-        host_is_pinned((const char *)obs + (size_t)offsets[0] * idx_bytes)) {
-        ltr_pipe = true;
-        const size_t nA = (size_t)W * N * N;
-        for (size_t e = 0; e < nA && ltr_pipe; ++e) {
-            const int ij = (int)(e % (size_t)(N * N)), i = ij / N, j = ij % N;
-            if (j != i && j != i + 1 && A0[e] > 0.0) ltr_pipe = false;
-        }
-    }
+    const bool ltr_pipe = h->has_ltr && (flags & HMMB_BW_PIPELINE_UPLOAD) && have_params && !obs_on_device && R > 0 &&
+                          offsets && obs && offsets[R] > offsets[0] && !getenv("HMMB_FORCE_DENSE_A") &&
+                          host_is_pinned((const char *)obs + (size_t)offsets[0] * idx_bytes) && upper_bidiagonal(A0, W, N);
     if (h->has_ltr && !ltr_pipe && !obs_on_device && R > 0 && offsets && obs && offsets[R] > offsets[0]) {
         // both layouts are built from the codewords: upload them once
         const size_t in_bytes = (size_t)(offsets[R] - offsets[0]) * idx_bytes;
@@ -1108,8 +1066,8 @@ int hmmb_bw_create_ex(hmmb_bw_t **out, const void *obs, int idx_bytes, int obs_o
     if (ltr_pipe) {
         h->ltr_only = true;
         h->raw_idx_bytes = idx_bytes;
-        h->bpieces = getenv("HMMB_NO_B_PIECES") ? 0 : ltr_pipeline_stages();
-        rc = seqset_build(h->sl, obs, idx_bytes, 0, offsets, word_of_seq, R, W, N, M, LAYOUT_LTR, true, &finish, ltr_pipeline_stages());
+        h->bpieces = PIPE_STAGES;
+        rc = seqset_build(h->sl, obs, idx_bytes, 0, offsets, word_of_seq, R, W, N, M, LAYOUT_LTR, true, &finish, PIPE_STAGES);
         if (rc != HMMB_OK) return fail(rc);
         if (h->bpieces_issued > 0 && (!h->sl.pend || h->bpieces_issued < h->bpieces)) {
             // no staged E-step will wait for the pieces one by one: order the compute stream behind the last one
@@ -1130,7 +1088,7 @@ int hmmb_bw_create_ex(hmmb_bw_t **out, const void *obs, int idx_bytes, int obs_o
     } else {
         const bool pipeline = (flags & HMMB_BW_PIPELINE_UPLOAD) != 0 && !h->has_ltr;
         rc = seqset_build(h->s, obs, idx_bytes, obs_on_device, offsets, word_of_seq, R, W, N, M, LAYOUT_AUTO, pipeline,
-                          pipeline ? &finish : nullptr, pipeline_stages());
+                          pipeline ? &finish : nullptr, PIPE_STAGES);
         if (rc != HMMB_OK) return fail(rc);
         if (h->has_ltr) {
             rc = seqset_build(h->sl, obs, idx_bytes, obs_on_device, offsets, word_of_seq, R, W, N, M, LAYOUT_LTR);
@@ -1308,22 +1266,10 @@ static int bw_set_params_impl(hmmb_bw *h, const double *pi0, const double *A0, c
         HMMB_CUDA(cudaMemsetAsync(h->d_bzero, 0, (size_t)W * sizeof(int32_t), c.stream));
         HMMB_LAUNCH("bw_load", k_load_B, gb, 256, 0, tmp, N, M, h->d_Bt, h->d_bzero);
     }
-    {
-        // upper-bidiagonal A (the reference's left-to-right default) selects the 7-term kernels;
-        // zeros of A stay zeros under re-estimation, so the choice holds for the whole fit
-        h->bidiag = (N == 4);
-        for (size_t e = 0; e < nA && h->bidiag; ++e) {
-            const int ij = (int)(e % (size_t)(N * N)), i = ij / N, j = ij % N;
-            if (j != i && j != i + 1 && A0[e] > 0.0) h->bidiag = false;
-        }
-        if (getenv("HMMB_FORCE_DENSE_A")) h->bidiag = false;
-        h->use_ltr = h->has_ltr;
-        for (size_t e = 0; e < nA && h->use_ltr; ++e) {
-            const int ij = (int)(e % (size_t)(N * N)), i = ij / N, j = ij % N;
-            if (j != i && j != i + 1 && A0[e] > 0.0) h->use_ltr = false;
-        }
-        if (getenv("HMMB_FORCE_DENSE_A")) h->use_ltr = false;
-    }
+    // upper-bidiagonal A (the reference's left-to-right default) selects the 7-term N = 4 kernels and the
+    // left-to-right kernels for N = 8 / 16
+    h->bidiag = N == 4 && upper_bidiagonal(A0, W, N) && !getenv("HMMB_FORCE_DENSE_A");
+    h->use_ltr = h->has_ltr && upper_bidiagonal(A0, W, N) && !getenv("HMMB_FORCE_DENSE_A");
     if (h->ltr_only && !h->use_ltr) HMMB_TRY(bw_build_generic_lazily(h));
     HMMB_LAUNCH("bw_load", k_load_clamped, (unsigned)std::min<size_t>((nA + 255) / 256, 1024), 256, 0, tmp + nB, (int64_t)nA, h->d_A);
     HMMB_LAUNCH("bw_load", k_load_clamped, (unsigned)std::min<size_t>((nP + 255) / 256, 1024), 256, 0, tmp + nB + nA, (int64_t)nP, h->d_pi);
@@ -1399,7 +1345,7 @@ static int launch_exact(hmmb_bw *h) {
     SeqSet &s = h->cur();
     HMMB_LAUNCH("bw_exact", (k_bw_exact<SymT, BLOCKED>), h->exact_grid, BW_THREADS, 0, s.d_obs, BLOCKED ? s.d_foff : s.d_off,
                 s.d_len, s.d_word, s.R, h->N, h->M, h->d_pi, h->d_A, h->d_Bt, h->d_llseq, h->act_cur, h->d_flag,
-                h->d_exact_scratch, h->exact_stride, h->d_accum, h->astride, h->d_nexact, s.symmask());
+                h->d_exact_scratch, h->exact_stride, h->d_accum, h->astride, h->d_nexact, SYM_MASK);
     return HMMB_OK;
 }
 
@@ -1450,7 +1396,7 @@ static int launch_special_estep(hmmb_bw *h) {
         if (c1 <= c0) return HMMB_OK;
         HMMB_LAUNCH("bw_forward", k_bw_fwd4<BIDIAG>, (c1 - c0) * FWD4_SPLIT, BW_THREADS, smem_f, stage_work + c0, s.d_blks, (const uint4 *)s.d_obs,
                     s.d_len, h->d_pi, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_flag,
-                    h->d_allfull, FWD4_SPLIT, s.symmask());
+                    h->d_allfull, FWD4_SPLIT, SYM_MASK);
         HMMB_LAUNCH("bw_backward", (k_bw_bwd4<BIDIAG, MT, REP>), c1 - c0, bwd_threads, smem_b, stage_work + c0, s.d_blks, (const uint4 *)s.d_obs,
                     s.d_len, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_bzero,
                     h->d_allfull, h->d_partials + (size_t)c0 * h->pstride, h->pstride, h->d_flag, h->d_newflags);
@@ -1465,9 +1411,8 @@ static int launch_special_estep(hmmb_bw *h) {
         // partials) is private to its blocks; the compute stream joins both side streams afterwards.
         PendingPrepare &p = *s.pend;
         int bdone = 0, cdone = 0;
-        cudaEvent_t tdone[PendingPrepare::MAX_STAGES] = {}, tbeg[PendingPrepare::MAX_STAGES] = {};
         cudaStream_t main_stream = c.stream;
-        const bool side = p.nstage > 2 && !getenv("HMMB_PIPE_ONE_STREAM");
+        const bool side = p.nstage > 2;
         struct Restore { Ctx &c; cudaStream_t s; ~Restore() { c.stream = s; } } restore{c, main_stream};
         if (side) {
             cudaEvent_t fork = event_get();
@@ -1478,10 +1423,8 @@ static int launch_special_estep(hmmb_bw *h) {
         for (int j = 0; j < p.nstage; ++j) {
             if (side) c.stream = c.stage_stream[j & 1];
             HMMB_CUDA(cudaStreamWaitEvent(c.stream, p.up->ev[p.ev_index[j]], 0));
-            if (p.up->t0) { cudaEventCreate(&tbeg[j]); cudaEventRecord(tbeg[j], c.stream); }
             HMMB_TRY(launch_repack_range(s, p.up->d_raw, p.idx_bytes, bdone, p.blk_end[j], s.d_bad));
             HMMB_TRY(launch_range(cdone, p.cta_end[j]));
-            if (p.up->t0) { cudaEventCreate(&tdone[j]); cudaEventRecord(tdone[j], c.stream); }
             bdone = p.blk_end[j];
             cdone = p.cta_end[j];
         }
@@ -1493,24 +1436,6 @@ static int launch_special_estep(hmmb_bw *h) {
                 HMMB_CUDA(cudaStreamWaitEvent(main_stream, join, 0));
                 event_put(join);
             }
-        }
-        if (p.up->t0) {  // HMMB_TIMING: where the upload chunks and the stages sit on one time line
-            cudaStreamSynchronize(c.stream);
-            for (int k = 0; k < p.up->nchunk; ++k) {
-                float ms = 0.f;
-                cudaEventElapsedTime(&ms, p.up->t0, p.up->ev[k]);
-                fprintf(stderr, "[hmmb] upload chunk %d landed at %.2f ms\n", k, ms);
-            }
-            for (int j = 0; j < p.nstage; ++j) {
-                float a = 0.f, b = 0.f;
-                cudaEventElapsedTime(&a, p.up->t0, tbeg[j]);
-                cudaEventElapsedTime(&b, p.up->t0, tdone[j]);
-                fprintf(stderr, "[hmmb] stage %d (blocks < %d, CTAs < %d): %.2f -> %.2f ms\n", j, p.blk_end[j], p.cta_end[j], a, b);
-                cudaEventDestroy(tbeg[j]);
-                cudaEventDestroy(tdone[j]);
-            }
-            cudaEventDestroy(p.up->t0);
-            p.up->t0 = nullptr;
         }
         h->check_bad = true;
         h->pend_release = std::move(s.pend);  // raw buffer + events: released after the next stream sync
@@ -1527,7 +1452,7 @@ static int launch_special_estep(hmmb_bw *h) {
     HMMB_LAUNCH("bw_forward", k_bw_fwd4<BIDIAG>, (s.ncta_fwd ? s.ncta_fwd : s.ncta) * FWD4_SPLIT, BW_THREADS, smem_f,
                 s.ncta_fwd ? s.d_work_fwd : s.d_work, s.d_blks, (const uint4 *)s.d_obs,
                 s.d_len, h->d_pi, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_flag,
-                h->d_allfull, FWD4_SPLIT, s.symmask());
+                h->d_allfull, FWD4_SPLIT, SYM_MASK);
     HMMB_TRY((launch_exact<uint16_t, true>(h)));
     HMMB_LAUNCH("bw_backward", (k_bw_bwd4<BIDIAG, MT, REP>), s.ncta, bwd_threads, smem_b, s.d_work, s.d_blks, (const uint4 *)s.d_obs,
                 s.d_len, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_bzero,
@@ -1541,7 +1466,7 @@ static int launch_ltr_estep(hmmb_bw *h) {
     if (s.ncta == 0) return HMMB_OK;
     const int M = h->M;
     const size_t smem_f = (size_t)M * NS * 8 + (size_t)M * 8 + (size_t)M * 2;
-    const size_t smem_b = (size_t)M * NS * 8 + (size_t)LTR_WARPS * LTR_STAGE_BUFS * 32 * Ltr<NS>::ROWB + (size_t)2 * NS * 8 +
+    const size_t smem_b = (size_t)M * NS * 8 + (size_t)LTR_WARPS * 32 * Ltr<NS>::ROWB + (size_t)2 * NS * 8 +
                           (size_t)LTR_WARPS * 2 * NS * 8;
     HMMB_CUDA(cudaFuncSetAttribute(k_bw_fwdL<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_f));
     HMMB_CUDA(cudaFuncSetAttribute(k_bw_bwdL<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
@@ -1555,7 +1480,7 @@ static int launch_ltr_estep(hmmb_bw *h) {
         PendingPrepare &p = *s.pend;
         int bdone = 0, cdone = 0;
         cudaStream_t main_stream = c.stream;
-        const bool side = p.nstage > 2 && !getenv("HMMB_PIPE_ONE_STREAM");
+        const bool side = p.nstage > 2;
         struct Restore { Ctx &c; cudaStream_t s; ~Restore() { c.stream = s; } } restore{c, main_stream};
         if (side) {
             cudaEvent_t fork = event_get();
@@ -1595,7 +1520,6 @@ static int launch_ltr_estep(hmmb_bw *h) {
                 event_put(join);
             }
         }
-        if (p.up->t0) { cudaEventDestroy(p.up->t0); p.up->t0 = nullptr; }
         h->check_bad = true;
         h->pend_release = std::move(s.pend);
         HMMB_TRY((launch_exact<uint16_t, true>(h)));
@@ -1691,7 +1615,7 @@ static int launch_rescue(hmmb_bw *h) {
 #define RESCUE(SYMT, BLK, BASE)                                                                                       \
     HMMB_LAUNCH("bw_rescue", (k_bw_rescue<SYMT, BLK>), h->exact_grid, BW_THREADS, 0, s.d_obs, BASE, s.d_len, s.d_word, s.R, \
                 h->N, h->M, h->d_pi, h->d_A, h->d_Bt, h->act_cur, h->d_exact_scratch, h->exact_stride, h->d_thinmask, \
-                h->d_slot_of, own, h->rstride, s.symmask())
+                h->d_slot_of, own, h->rstride, SYM_MASK)
     if (s.blocked()) {
         RESCUE(uint16_t, true, s.d_foff);
     } else if (s.sym_bytes == 1) {
@@ -1775,7 +1699,7 @@ static int bw_one_pass(hmmb_bw *h, int32_t *mask, double eps, int max_iter, int 
                 h->d_accum + (size_t)h->W * h->astride, h->world, h->W, h->N, h->M, h->d_pi, h->d_A, h->d_Bt,
                 mask, h->d_active, h->d_iters, h->d_prev, h->d_hist, h->hist_cap, eps, max_iter, h->d_any, h->d_bzero,
                 h->d_thinmask, h->d_thin_new, h->d_redo, skip_new_thin, h->d_slot_of, rescue_base(h), h->slot_cap, h->rstride,
-                getenv("HMMB_NO_THIN_RESCUE") ? 0.0 : THIN_LIMIT);
+                THIN_LIMIT);
     return HMMB_OK;
 }
 
@@ -1928,7 +1852,7 @@ static int launch_score_special(SeqSet &s, int W, const double *d_pi, const doub
     if (b1 < 0) b1 = s.nblk;
     const int nb = b1 - b0;  // blocks [b0, b1) (a stage of the pipelined scorer, or all of them)
     if (nb <= 0) return HMMB_OK;
-    if (s.M <= SCORE4R_MAX_M && !getenv("HMMB_SCORE_NO_REPLICAS")) {
+    if (s.M <= SCORE4R_MAX_M) {
         // replicated-B scorer: 8 warps per CTA, 2 CTAs per SM, about six waves of CTAs
         int bpc = std::max(SCORE4R_WARPS, (int)(((int64_t)nb * W + c.sm_count * 12 - 1) / (c.sm_count * 12)));
         bpc = (bpc + SCORE4R_WARPS - 1) / SCORE4R_WARPS * SCORE4R_WARPS;
@@ -1984,11 +1908,7 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
         ~Guard() { s.release(); for (void *p : ptrs) dev_free(p); }
     } guard{s, {}};
     // left-to-right models at N = 8 / 16 are scored one utterance per thread (k_scoreL)
-    bool ltr = ltr_shape_ok(N, M);
-    for (size_t e = 0; e < (size_t)W * N * N && ltr; ++e) {
-        const int ij = (int)(e % (size_t)(N * N)), i = ij / N, j = ij % N;
-        if (j != i && j != i + 1 && A[e] > 0.0) ltr = false;
-    }
+    const bool ltr = ltr_shape_ok(N, M) && upper_bidiagonal(A, W, N);
     const size_t nB = (size_t)W * N * M, nA = (size_t)W * N * N, nP = (size_t)W * N;
     double *tmp = nullptr, *d_pi = nullptr, *d_A = nullptr, *d_Bt = nullptr, *d_ll = nullptr;
     int32_t *d_arg = nullptr;
@@ -2026,11 +1946,7 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
     if (U == 0) return HMMB_OK;
     if (!models_up) HMMB_TRY(upload_models());
     if (s.pend) {
-        bool bidiag = true;
-        for (size_t e = 0; e < nA && bidiag; ++e) {
-            const int ij = (int)(e % 16), i = ij / 4, j = ij % 4;
-            if (j != i && j != i + 1 && A[e] > 0.0) bidiag = false;
-        }
+        const bool bidiag = upper_bidiagonal(A, W, N);
         PendingPrepare &p = *s.pend;
         int bdone = 0;
         // a pageable result matrix cannot leave stage by stage (its copies would block the host between the
@@ -2080,11 +1996,7 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
     }
     int rc;
     if (s.special4) {
-        bool bidiag = true;
-        for (size_t e = 0; e < nA && bidiag; ++e) {
-            const int ij = (int)(e % 16), i = ij / 4, j = ij % 4;
-            if (j != i && j != i + 1 && A[e] > 0.0) bidiag = false;
-        }
+        const bool bidiag = upper_bidiagonal(A, W, N);
         rc = bidiag ? launch_score_special<true>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan)
                     : launch_score_special<false>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan);
     } else if (s.ltr_ns) {

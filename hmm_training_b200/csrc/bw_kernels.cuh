@@ -11,12 +11,8 @@
 namespace hmmb {
 
 // resident CTAs per SM the generic E-step kernels are compiled for (1 = no register cap)
-#ifndef GEN_FWD_MIN_CTAS
-#define GEN_FWD_MIN_CTAS 1
-#endif
-#ifndef GEN_BWD_MIN_CTAS
-#define GEN_BWD_MIN_CTAS 1
-#endif
+constexpr int GEN_FWD_MIN_CTAS = 1;
+constexpr int GEN_BWD_MIN_CTAS = 1;
 
 // generic path: convert to the canonical symbol width, validate range
 template <typename InT, typename SymT>

@@ -15,13 +15,17 @@
 //               alpha-hat spilled [block][t][chunk][lane] as coalesced 16-byte streaming stores.
 //   k_bw_bwdL   backward pass fused with gamma / xi / emission-count accumulation.  Each lane's
 //               gamma_t row (NS fp64 = 128 B at NS = 16) is staged in shared memory (padded
-//               rows, conflict-free) and added to the word's count row in the global
-//               accumulator by the L2 atomic units, which frees the shared memory a [M][NS]
-//               count table would need for B^T.  Measured on B200 (scripts/microbench2.cu,
-//               clk per row per SM): coalesced RED rows with lanes = states 7.8, one TMA bulk
-//               reduction per lane (cp.reduce.async.bulk .add.f64) 7.6, shared table + row
-//               locks 8.9, shared CAS atomics 11.8, per-element global RED 24.4.  The RED
-//               rows are the default (see HMMB_LTR_TMA below).
+//               rows, conflict-free), re-read with lanes = states and added to the word's count
+//               row in the global accumulator with coalesced fp64 REDs (the L2 atomic units),
+//               which frees the shared memory a [M][NS] count table would need for B^T.
+//               Measured on B200 (scripts/microbench2.cu, clk per row per SM): coalesced RED
+//               rows with lanes = states 7.8, one TMA bulk reduction per lane
+//               (cp.reduce.async.bulk .add.f64) 7.6, shared table + row locks 8.9, shared CAS
+//               atomics 11.8, per-element global RED 24.4.  The TMA instruction takes its
+//               operands from uniform registers, so a warp issues its 32 reductions in a serial
+//               ELECT / R2UR / UBLKRED loop (ncu, profiles/r1i_*: 42 % of the kernel's
+//               instructions): config 4 backward 5.55 ms with it against 4.54 ms with the RED
+//               rows.  That variant was removed; it is in the history at commit 03a55a2.
 //
 // Numerics are those of the N = 4 kernels (bw4_kernels.cuh): exact power-of-two rescale,
 // smallest-denormal FMA addends that keep "value > 0 <=> the reference's log value is
@@ -33,21 +37,7 @@
 
 namespace hmmb {
 
-// Emission-count scatter-add of the backward pass: 0 (default) = coalesced fp64 REDs of the staged
-// gamma rows re-read with lanes = states; 1 = one TMA bulk reduction (cp.reduce.async.bulk
-// .add.f64, SASS UBLKRED) per lane.  Both bottom out at ~7.6-7.8 clk per row per SM in the L2
-// atomic units (scripts/microbench2.cu), but the TMA instruction takes its operands from
-// uniform registers, so a warp issues its 32 reductions in a serial ELECT / R2UR / UBLKRED loop
-// (ncu, profiles/r1i_*: 42 % of the kernel's instructions, each waiting on the previous one):
-// config 4 backward 5.55 ms with TMA vs the RED rows below.
-#ifndef HMMB_LTR_TMA
-#define HMMB_LTR_TMA 0
-#endif
-constexpr int LTR_STAGE_BUFS = HMMB_LTR_TMA ? 2 : 1;
 constexpr int LTR_WARPS = 8;
-#ifndef LTR_SERPENTINE
-#define LTR_SERPENTINE 1
-#endif
 constexpr int LTR_THREADS = LTR_WARPS * 32;
 constexpr int LTR_MAX_SYM = 1 << SYM_BITS;   // codewords share the packed u16 layout of the N = 4 path
 // steps ahead of use for the alpha-hat L2 prefetch (3 / 6 / 12 and an extra L1 prefetch measured
@@ -65,8 +55,6 @@ struct Ltr {
         return (int)row * CPR + (c ^ (int)((row / (8 / CPR)) & (CPR - 1)));
     }
 };
-
-__device__ __forceinline__ unsigned smem_addr(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 
 template <int N>
 __device__ __forceinline__ double tree_sum(const double (&x)[N]) {
@@ -366,7 +354,7 @@ k_bw_fwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
     // gets about the same number of steps (plain striding gave warp 0 the longest block of every round: with four
     // rounds per CTA the last warp idled for a tenth of the kernel at the CTA's final barrier)
     for (int rb = cw.blk_begin, rnd = 0; rb < cw.blk_end; rb += LTR_WARPS, ++rnd) {
-        const int b = rb + (LTR_SERPENTINE && (rnd & 1) ? LTR_WARPS - 1 - warp : warp);
+        const int b = rb + ((rnd & 1) ? LTR_WARPS - 1 - warp : warp);
         if (b >= cw.blk_end) continue;
         const Blk bk = blks[b];
         int T = lane < bk.nseq ? len_sorted[bk.first + lane] : 0;
@@ -527,12 +515,6 @@ __device__ __noinline__ void bwdL_step_slow(BwdLState<NS> &st, const double *__r
     st.vpos = vp;
 }
 
-// TMA bulk reduction: global[dst .. dst+bytes) += shared[src .. src+bytes) element-wise in fp64
-__device__ __forceinline__ void bulk_reduce_add_f64(double *dst_global, unsigned src_smem, int bytes) {
-    asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.f64 [%0], [%1], %2;"
-                 :: "l"(dst_global), "r"(src_smem), "r"(bytes) : "memory");
-}
-
 // Accumulator layout per word: [pi N][xi N*N][cnt M*N] (fp64, L2 atomics), N == NS.
 template <int NS>
 __global__ void __launch_bounds__(LTR_THREADS, NS == 8 ? 2 : 1)
@@ -545,8 +527,8 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
     using S16 = Sym<uint16_t>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double2 *sB = reinterpret_cast<double2 *>(smem_raw);                                  // [M * CPR] swizzled B^T
-    unsigned char *sStage = reinterpret_cast<unsigned char *>(sB + (size_t)M * L::CPR);    // [warps][bufs][32][ROWB]
-    double *sA = reinterpret_cast<double *>(sStage + (size_t)LTR_WARPS * LTR_STAGE_BUFS * 32 * L::ROWB);  // a_ii [NS], a_i,i+1 [NS]
+    unsigned char *sStage = reinterpret_cast<unsigned char *>(sB + (size_t)M * L::CPR);    // [warps][32][ROWB]
+    double *sA = reinterpret_cast<double *>(sStage + (size_t)LTR_WARPS * 32 * L::ROWB);   // a_ii [NS], a_i,i+1 [NS]
     double *sRed = sA + 2 * NS;                                                            // [warps][2 * NS]
     __shared__ unsigned sSeen[2];
 
@@ -570,25 +552,20 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
     const double tiny = tiny_pos();
     double *accw = accum + (size_t)cw.word * astride;
     double *acc_cnt = accw + NS + NS * NS;
-    unsigned char *stage_w = sStage + (size_t)warp * LTR_STAGE_BUFS * 32 * L::ROWB + (size_t)lane * L::ROWB;
-#if !HMMB_LTR_TMA
+    unsigned char *stage = sStage + (size_t)warp * 32 * L::ROWB + (size_t)lane * L::ROWB;
     // count flush with lanes = states: lane (fo, jj) reads state jj of staged rows fo, fo + FPI, ...
     const int flush_jj = lane % NS, flush_fo = lane / NS;
-    const unsigned char *flush_src = sStage + (size_t)warp * LTR_STAGE_BUFS * 32 * L::ROWB + (size_t)flush_fo * L::ROWB + flush_jj * 8;
+    const unsigned char *flush_src = sStage + (size_t)warp * 32 * L::ROWB + (size_t)flush_fo * L::ROWB + flush_jj * 8;
     const int flush_sym_off = NS * 8 - flush_jj * 8;  // from the lane's element to the row's padding word
     double *flush_dst = acc_cnt + flush_jj;
-#endif
 
     double v[NS], Xs[NS], Xn[NS];
 #pragma unroll
     for (int i = 0; i < NS; ++i) Xs[i] = Xn[i] = 0.0;
     unsigned seenS = 0u, seenN = 0u;
-#if HMMB_LTR_TMA
-    int step_parity = 0;
-#endif
 
     for (int rb = cw.blk_begin, rnd = 0; rb < cw.blk_end; rb += LTR_WARPS, ++rnd) {
-        const int b = rb + (LTR_SERPENTINE && (rnd & 1) ? LTR_WARPS - 1 - warp : warp);
+        const int b = rb + ((rnd & 1) ? LTR_WARPS - 1 - warp : warp);
         if (b >= cw.blk_end) continue;
         const Blk bk = blks[b];
         int T = 0;
@@ -607,14 +584,12 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
         const char *sp_line = reinterpret_cast<const char *>(spill + (size_t)bk.spill_base * L::CPR * 32) + (size_t)lane * 128;
         const int nch = (bk.tmax + SPC4 - 1) / SPC4;
         uint4 wnext = __ldg(op + (size_t)(nch - 1) * 32);
-#if !HMMB_LTR_TMA
         if (T < bk.tmax) {  // this lane sits out the block's first steps (or all of them): its staged row reads as zero
-            double2 *sg = reinterpret_cast<double2 *>(stage_w);
+            double2 *sg = reinterpret_cast<double2 *>(stage);
 #pragma unroll
             for (int p = 0; p < L::CPR; ++p) sg[p] = make_double2(0.0, 0.0);
-            *reinterpret_cast<unsigned *>(stage_w + NS * 8) = 0u;
+            *reinterpret_cast<unsigned *>(stage + NS * 8) = 0u;
         }
-#endif
         // alpha-hat of the step to come.  Every step loads its successor's row into these registers right after its
         // own last use of them, so that the load (an L2 hit thanks to the prefetch below) is in flight during the
         // count flush and the next step's q = A v, instead of being waited for at the first product with q (that
@@ -644,14 +619,6 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
                 const int t = c * SPC4 + s;
                 const unsigned sym = S16::pop_back(w) & SYM_MASK;
                 const bool act = t < T;
-#if HMMB_LTR_TMA
-                // the staging buffer used two steps ago must have been read by the TMA unit
-                asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-                unsigned char *stage = stage_w + (size_t)step_parity * 32 * L::ROWB;
-                step_parity ^= 1;
-#else
-                unsigned char *stage = stage_w;
-#endif
                 // pull the spill towards L2 well ahead
                 prefetch_l2_if(sp_line + (size_t)(t - BWDL_L2_PREFETCH) * (NS * 8 * 32), t >= BWDL_L2_PREFETCH && lane * 128 < NS * 8 * 32);
                 if (act) {
@@ -682,7 +649,7 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
                             // lean step: beta_t(i) ~ q_i = a_ii v_i + a_i,i+1 v_{i+1} (:163-199); gamma_t(i) = al_i q_i / norm
                             // (:389-394); xi_t(i,j) = al_i a_ij v_j / norm (:397-410); norm = sum_i al_i q_i.  The denormal
                             // addends keep a finite-but-underflowed log value (barely) positive.  Nothing is committed
-                            // (v, Xs, Xn, the TMA reduction) before the three magnitude tests have passed.
+                            // (v, Xs, Xn, the count REDs) before the three magnitude tests have passed.
                             double q[NS];
 #pragma unroll
                             for (int i = 0; i < NS - 1; ++i) q[i] = fma(sA[NS + i], v[i + 1], fma(sA[i], v[i], tiny));
@@ -743,13 +710,6 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
 #pragma unroll
                         for (int p = 0; p < L::CPR; ++p) sg[p] = make_double2(g[2 * p], g[2 * p + 1]);
                     }
-#if HMMB_LTR_TMA
-                    // emission-count numerators (:460-500) and, at t = 0, the pi sums (:415-426): the lane's
-                    // gamma row is added to the word's accumulator rows by the TMA unit (L2 fp64 atomics)
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    bulk_reduce_add_f64(acc_cnt + (size_t)sym * NS, smem_addr(stage), NS * 8);
-                    if (t == 0) bulk_reduce_add_f64(accw, smem_addr(stage), NS * 8);
-#endif
                 }
                 {  // alpha-hat of step t - 1 (at t = 0: row 0 once more, unused)
                     const int tp = t > 0 ? t - 1 : 0;
@@ -760,9 +720,6 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
                         al[2 * q + 1] = x.y;
                     }
                 }
-#if HMMB_LTR_TMA
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-#else
                 // emission-count numerators (:460-500) and, at t = 0, the pi sums (:415-426): the staged
                 // gamma rows are re-read with lanes = states (NS lanes per row, 32 / NS rows per
                 // instruction) and added to the word's accumulator rows with coalesced fp64 REDs
@@ -803,7 +760,6 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
                     }
                 }
                 __syncwarp();
-#endif
             }
         }
         if (imprecise) {  // sticky hand-over; the host redoes this E-step once (hmmb_bw_iterate)
@@ -811,9 +767,6 @@ k_bw_bwdL(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
             atomicAdd(new_flags, 1);
         }
     }
-#if HMMB_LTR_TMA
-    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-#endif
 
     // ---- CTA flush of the xi sums: warp shuffle tree, then one fp64 RED per entry
     double *red = sRed + (size_t)warp * 2 * NS;

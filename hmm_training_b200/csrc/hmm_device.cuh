@@ -325,7 +325,7 @@ struct LinObs {
 template <typename SymT>
 struct BlkObs {
     const uint4 *p;  // chunk row of this sequence's lane: obs_blk + blk.obs_base + lane
-    unsigned mask = 0x7ffu;  // codeword bits of a packed entry: 11, or 8 in the peer encoding (bw4_kernels.cuh)
+    unsigned mask = 0x7ffu;  // the 11 codeword bits of a packed entry (bw4_kernels.cuh)
     __device__ __forceinline__ unsigned operator[](int t) const {
         // blocked layout: 8 packed u16 per uint4, codeword in the low bits (bw4_kernels.cuh)
         const unsigned short *c = reinterpret_cast<const unsigned short *>(p + (size_t)(t / 8) * 32);

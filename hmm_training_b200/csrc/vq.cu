@@ -23,15 +23,9 @@
 namespace hmmb {
 
 constexpr int VQ_THREADS = 256;
-#ifndef VQ_MIN_CTAS
-#define VQ_MIN_CTAS 3           // resident CTAs per SM the assign kernel is compiled for: 80 registers, no spills; encode call 0.212 (2) / 0.199 (3) / 0.206 ms (4)
-#endif
+constexpr int VQ_MIN_CTAS = 3;  // resident CTAs per SM the assign kernel is compiled for: 80 registers, no spills; encode call 0.212 (2) / 0.199 (3) / 0.206 ms (4)
 constexpr int VQ_TILE = 512;  // centroids per shared-memory tile: 512 * 12 * 8 B = 48 KB
 constexpr int VQ_D = 12;      // dims 1..12 take part in the distance
-#ifndef VQ_ILP
-#define VQ_ILP 4              // centroids in flight per thread (4 / 8 and one-batch-per-CTA grids all measured 0.47 ms:
-                              // the kernel sits at ~78 % of the fp64 issue rate counting the 25 DP instructions per pair)
-#endif
 constexpr int ACC_W = 14;     // per-centroid accumulator row: 13 sums + count
 constexpr int VQ_PRIV_K = 32; // up to this many centroids every warp keeps a private accumulator table
 
@@ -453,7 +447,7 @@ static size_t vq_smem_bytes(int K, int mode, int *smem_accum) {
     size_t tile = tk * VQ_D * sizeof(double) + tk4 * VQ_D * sizeof(float) + tk4 * sizeof(float);
     size_t acc = (size_t)K * ACC_W * sizeof(double);
     *smem_accum = 0;
-    if (mode == 1 && K <= VQ_PRIV_K && !getenv("HMMB_LBG_NO_PRIVATE")) {
+    if (mode == 1 && K <= VQ_PRIV_K) {
         *smem_accum = 2;
         const size_t warps = VQ_THREADS / 32;
         return tile + warps * (acc + 32 * 13 * sizeof(double)) + warps * 32 * sizeof(int);

@@ -1,6 +1,5 @@
 """End-to-end breakdown of one engine.bw_fit-style call (create / set / iterate / get / close), config 3 by default,
-config 4 with C4=1; PINP=1 also pins the initial parameters and the result arrays; HMMB_TIMING=1 adds the library's
-own stage times on stderr."""
+config 4 with C4=1; PINP=1 also pins the initial parameters and the result arrays."""
 import sys, time, os
 sys.path.insert(0, os.getcwd())
 import numpy as np, torch
