@@ -375,7 +375,16 @@ int hmmb_set_stream(void *cuda_stream) {
     HMMB_TRY(require_init());
     Ctx &c = ctx();
     phase_collect();
-    c.stream = cuda_stream ? (cudaStream_t)cuda_stream : c.own_stream;
+    cudaStream_t next = cuda_stream ? (cudaStream_t)cuda_stream : c.own_stream;
+    if (next != c.stream) {
+        // A call may return with kernels still queued on the old stream (hmmb_vq_encode_dev) whose device blocks the
+        // allocator already hands out again: the new stream starts behind everything queued on the old one.
+        cudaEvent_t e = event_get();
+        HMMB_CUDA(cudaEventRecord(e, c.stream));
+        HMMB_CUDA(cudaStreamWaitEvent(next, e, 0));
+        event_put(e);
+    }
+    c.stream = next;
     return HMMB_OK;
 }
 

@@ -44,7 +44,10 @@ int hmmb_shutdown(void);                   /* free workspace, destroy stream    
 const char *hmmb_last_error(void);
 const char *hmmb_version(void);
 int hmmb_device_info(int *sm_count, int *cc_major, int *cc_minor, int64_t *global_mem_bytes);
-int hmmb_set_stream(void *cuda_stream);    /* NULL restores the library's own stream        */
+/* NULL restores the library's own stream.  The stream is used from the next call on and starts behind the work
+ * queued on the previous one; the library's own stream is non-blocking (not ordered with the legacy default
+ * stream), so without hmmb_set_stream a caller synchronises around calls that take device pointers. */
+int hmmb_set_stream(void *cuda_stream);
 void *hmmb_get_stream(void);
 int hmmb_synchronize(void);
 /* pinned host memory for callers that want async H2D/D2H */
@@ -84,7 +87,10 @@ int hmmb_comm_destroy(void);
  * sqrt(sum_{d=1..12} (x_d - c_kd)^2), strict '<' (lowest index wins ties); dimension 0
  * (energy) is ignored (:100,:107).  X [F,13], C [K,13] fp64 -> idx_out [F] int32.        */
 int hmmb_vq_encode(const double *X, int64_t F, const double *C, int K, int32_t *idx_out);
-/* same on device-resident buffers; d_dist (nullable) receives the winning distance       */
+/* same on device-resident buffers; d_dist (nullable) receives the winning distance.  dX / dC are read and
+ * d_idx / d_dist written on hmmb_get_stream(): the inputs must be complete on that stream when the call runs, and
+ * the call returns WITHOUT waiting — the outputs are ready for work queued on that stream afterwards, or after
+ * hmmb_synchronize().                                                                     */
 int hmmb_vq_encode_dev(const double *dX, int64_t F, const double *dC, int K, int32_t *d_idx,
                        double *d_dist);
 /* hmmb_vq_encode + the near-tie report of the parity contract (BASELINE.json north_star: "codeword indices
@@ -104,7 +110,8 @@ int hmmb_vq_encode_ex(const double *X, int64_t F, const double *C, int K, int32_
  *   C_out [Kout,13]; gens_out [(1 + 2 + ... + 2^n_gen), 13] = [C0] + converged centroids of
  *   each generation (:466,:517); assign_out [F] = frame.parent_centroid_id (:502);
  *   iters_per_gen [n_gen]; gdist_out [n_gen] (nullable) last sum of min distances (:503).
- * x_on_device != 0: X is a device pointer (frames already resident in HBM).
+ * x_on_device != 0: X is a device pointer (frames already resident in HBM), read on hmmb_get_stream() (it must be
+ * complete on that stream); the call returns with every output written to the host and X no longer in use.
  * Multi-GPU: every rank passes its shard of frames and the same hook; sums/counts/distance
  * are all-reduced once per Lloyd pass (SURVEY.md §8e).                                      */
 int hmmb_lbg_fit(const double *X, int64_t F, int x_on_device, int K, int max_iter, double eps,
@@ -129,6 +136,10 @@ int hmmb_lbg_fit_ex(const double *X, int64_t F, int x_on_device, int K, int max_
  * word_of_seq[r] in [0, W).  Limits: 1 <= N <= 32, 1 <= M <= 65536, T >= 1.            */
 typedef struct hmmb_bw hmmb_bw_t;
 
+/* obs_on_device != 0: obs is a device pointer (offsets and word_of_seq stay on the host) and sequence r starts at
+ * codeword offsets[r] of it; it is read on hmmb_get_stream() (it must be complete on that stream) and no longer in
+ * use when the create returns: the trainer keeps its own copies.  A codeword >= M fails the create
+ * (HMMB_ERR_RANGE).                                                                      */
 int hmmb_bw_create(hmmb_bw_t **out, const void *obs, int idx_bytes, int obs_on_device,
                    const int64_t *offsets, const int32_t *word_of_seq, int64_t R, int W, int N,
                    int M);
@@ -199,7 +210,8 @@ int hmmb_bw_fit(const void *obs, int idx_bytes, const int64_t *offsets, const in
  * test_hmm, :139-161: ll_out [U,W] = log P(O_u | model_w) from LINEAR pi/A/B (zeros are
  * structural -inf, :67-69); argmax_out [U] = first model with the strictly largest score,
  * -1 ("unknown", :161) if every score is -inf.  ll_out / argmax_out may be NULL.
- * obs_on_device != 0: obs is a device pointer; offsets stay on the host.                  */
+ * obs_on_device != 0: obs is a device pointer; offsets stay on the host.  It is read on hmmb_get_stream() (it must
+ * be complete on that stream); the call returns with ll_out / argmax_out written and obs no longer in use.     */
 int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets, int64_t U,
                int W, int N, int M, const double *pi, const double *A, const double *B,
                double *ll_out, int32_t *argmax_out);
@@ -210,7 +222,9 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
  * librosa.feature.mfcc(y=frame, sr, n_mfcc=13, n_fft=L, hop_length=None, center=False, n_mels=26).
  * 2 <= L <= 1024 (the reference's frames have 320 samples, the tail frame of a recording 13..319).
  * librosa is not available where this was built: the kernel follows its published algorithm as
- * restated in oracle/mfcc_oracle.py; parity with librosa itself is unpinned (DESIGN.md).          */
+ * restated in oracle/mfcc_oracle.py; parity with librosa itself is unpinned (DESIGN.md).
+ * y_on_device != 0: Y is read on hmmb_get_stream() (it must be complete on that stream); the call returns with
+ * mfcc_out written and Y no longer in use.                                                       */
 int hmmb_mfcc_frames(const double *Y, int64_t F, int L, int y_on_device, double sr, double *mfcc_out);
 
 /* ------------------------------------------------------------------ frame-file loader (host only)

@@ -82,21 +82,22 @@ def test_left_to_right_kernels_match_reference_golden(name, monkeypatch):
 
 def test_baum_welch_shuffled_sequence_order(kernel_family):
     """The library sorts sequences by (word, length); interleaved / shuffled input must give
-    the same models (sum order changes only at the 1e-16 level)."""
+    the same models (sum order changes only at the 1e-16 level), whatever the width of the codewords."""
     g = load_golden("bw_uniform_s1_it3")
     N, M = int(g["N"]), int(g["M"])
     corpus = split_corpus(g)
     rng = np.random.default_rng(0)
     seqs = [(w, s) for w, word in enumerate(corpus) for s in word]
     perm = rng.permutation(len(seqs))
-    obs = np.concatenate([seqs[i][1] for i in perm]).astype(np.int64)  # int64 input path
     lens = np.array([len(seqs[i][1]) for i in perm])
     offsets = np.concatenate([[0], np.cumsum(lens)]).astype(np.int64)
     wos = np.array([seqs[i][0] for i in perm], dtype=np.int32)
     W = len(corpus)
     pi0, A0, B0 = _init_for(g, W, N, M)
-    pi, A, B, hist, iters = engine.bw_fit(obs, offsets, wos, W, N, M, pi0, A0, B0, max_iterations=3)
-    _check_bw("shuffled", g, pi, A, B, hist, iters, N, M)
+    for dt in (np.int64, np.uint32):  # 8- and 4-byte codewords
+        obs = np.concatenate([seqs[i][1] for i in perm]).astype(dt)
+        pi, A, B, hist, iters = engine.bw_fit(obs, offsets, wos, W, N, M, pi0, A0, B0, max_iterations=3)
+        _check_bw(f"shuffled {np.dtype(dt).name}", g, pi, A, B, hist, iters, N, M)
 
 
 @pytest.mark.parametrize("N,M,T", [(4, 256, 200), (4, 300, 37), (3, 20, 15), (8, 64, 40), (16, 1024, 50), (32, 128, 12)])
@@ -558,10 +559,29 @@ def test_lbg_degenerate_duplicates_near_tie():
         assert relabel.setdefault(int(a), int(b)) == int(b)
 
 
-@pytest.mark.parametrize("name", ["lbg_600_k32", "lbg_1200_k256_it3", "lbg_k1", "lbg_k24_nonpow2"])
-def test_lbg_matches_reference_golden(name):
+def _with_residence(argname, values):
+    """Parameter sets (value, residence) for the LBG tests: every value with host frames (id: the value) and with
+    frames already in device memory (id: value-device)."""
+    return pytest.mark.parametrize(
+        f"{argname},residence", [(v, "host") for v in values] + [(v, "device") for v in values],
+        ids=list(values) + [f"{v}-device" for v in values])
+
+
+def _lbg_fit_from(residence, X, *args):
+    """engine.lbg_fit on host frames, or on a device copy of them (hmmb_lbg_fit_ex with x_on_device = 1)."""
+    if residence == "host":
+        return engine.lbg_fit(X, *args)
+    import torch
+    dX = torch.from_numpy(np.ascontiguousarray(X, dtype=np.float64)).cuda()
+    torch.cuda.synchronize()
+    return engine.lbg_fit(None, *args, x_dev_ptr=dX.data_ptr(), F=len(X))
+
+
+@_with_residence("name", ["lbg_600_k32", "lbg_1200_k256_it3", "lbg_k1", "lbg_k24_nonpow2"])
+def test_lbg_matches_reference_golden(name, residence):
     g = load_golden(name)
-    C, gens, assign, iters, _ = engine.lbg_fit(g["X"], int(g["K"]), int(g["max_iterations"]), float(g["epsilon"]))
+    C, gens, assign, iters, _ = _lbg_fit_from(residence, g["X"], int(g["K"]), int(g["max_iterations"]),
+                                              float(g["epsilon"]))
     assert C.shape == g["C"].shape
     assert np.array_equal(iters, g["iters"])
     assert_close(C, g["C"], "centroids", rtol=1e-9, atol=1e-12)
@@ -575,13 +595,14 @@ def test_lbg_no_data():
         engine.lbg_fit(np.zeros((0, 13)), 4)
 
 
-@pytest.mark.parametrize("case", ["max_iterations_0", "max_iterations_1", "epsilon_0", "k2", "k3", "k_above_frames", "one_frame",
-                                  "identical_frames", "nan_coordinate"])
-def test_lbg_edge_inputs_match_oracle(case):
+@_with_residence("case", ["max_iterations_0", "max_iterations_1", "epsilon_0", "k2", "k3", "k_above_frames", "one_frame",
+                          "identical_frames", "nan_coordinate"])
+def test_lbg_edge_inputs_match_oracle(case, residence):
     """Edge inputs of createCodeVector (CodeVector/codevector_functions.py:442-531).  The C oracle was compared with the
     reference itself on every one of them (same centroids, assignments and iteration counts: scripts/edge_probe.py has
     the list); here the device path is held to the oracle — a NaN coordinate included, which the reference carries
-    through its distances and means without complaint."""
+    through its distances and means without complaint — with the frames passed from host memory and from device
+    memory."""
     from oracle import vq_oracle as V
     X = synthetic.mfcc_mixture(3, 200, K=8)
     K, mi, eps = 8, 20, 1e-3
@@ -595,7 +616,7 @@ def test_lbg_edge_inputs_match_oracle(case):
     elif case == "identical_frames": X = np.tile(X[:1], (30, 1))
     elif case == "nan_coordinate":
         X = X.copy(); X[3, 4] = np.nan; K, mi = 4, 5
-    C, gens, assign, iters, gdist = engine.lbg_fit(X, K, mi, eps)
+    C, gens, assign, iters, gdist = _lbg_fit_from(residence, X, K, mi, eps)
     Co, genso, assigno, iterso, gdisto = V.lbg(X, K, mi, eps)
     assert C.shape == Co.shape and np.array_equal(iters, iterso)
     assert np.allclose(C, Co, rtol=1e-9, atol=0, equal_nan=True)
