@@ -76,6 +76,8 @@ SYMBOLS = [
     ("hmmb_frames_json_scan", _c.c_int64, [_c.c_char_p, _c.c_int64, _c.c_void_p, _c.c_int64]),
     ("hmmb_score", _c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int, _c.c_int,
                               _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p]),
+    ("hmmb_viterbi", _c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_void_p, _c.c_int, _c.c_int,
+                                _c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p]),
 ]
 
 

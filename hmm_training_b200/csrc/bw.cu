@@ -1,4 +1,4 @@
-// Host side of the Baum-Welch trainer and the forward scorer: sequence sorting/blocking,
+// Host side of the Baum-Welch trainer, the forward scorer and the Viterbi decoder: sequence sorting/blocking,
 // device layout, the EM loop, and the C ABI declared in include/hmmb200.h.
 #include <algorithm>
 #include <cstdlib>
@@ -8,6 +8,7 @@
 
 #include "bw_kernels.cuh"
 #include "bwltr_kernels.cuh"
+#include "viterbi_kernels.cuh"
 
 namespace hmmb {
 
@@ -2034,3 +2035,118 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
     return HMMB_OK;
 }
 
+// ---------------------------------------------------------------- Viterbi decoding
+template <int NS, bool BIDIAG>
+static int launch_viterbi_blocked(SeqSet &s, const double *d_lpi, const double *d_lA, const double *d_lBt, double *d_score,
+                                  int8_t *d_last, void *d_bp) {
+    if (s.ncta == 0) return HMMB_OK;
+    const size_t smem = (size_t)s.M * NS * sizeof(double);
+    HMMB_CUDA(cudaFuncSetAttribute((k_viterbiB<NS, BIDIAG>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // The work items are sized for the trainer's CTAs (about two per SM at N = 4, each for one 16-warp backward CTA);
+    // one 8-warp Viterbi CTA per item would leave the SMs with a few warps each for a latency-bound per-thread
+    // recursion, so every item is shared by enough CTAs for about eight per SM.
+    const int split = std::max(1, std::min(BWD4_MAX_WARPS, (ctx().sm_count * 8 + s.ncta - 1) / s.ncta));
+    dim3 g((unsigned)s.ncta, (unsigned)split);
+    HMMB_LAUNCH("viterbi", (k_viterbiB<NS, BIDIAG>), g, VIT_THREADS, smem, s.d_work, s.d_blks, (const uint4 *)s.d_obs, s.d_len,
+                s.d_order, d_lpi, d_lA, d_lBt, s.M, d_score, d_last, (VitRow<NS> *)d_bp);
+    return HMMB_OK;
+}
+
+template <int NS>
+static int launch_vit_backtrace_blocked(SeqSet &s, const int8_t *d_last, const void *d_bp, int8_t *d_path) {
+    if (s.nblk == 0) return HMMB_OK;
+    constexpr int WPB = VIT_THREADS / 32;
+    HMMB_LAUNCH("viterbi_backtrace", k_vit_backtraceB<NS>, (s.nblk + WPB - 1) / WPB, VIT_THREADS, 0, s.d_blks, s.nblk, s.d_len,
+                s.d_off, d_last, (const VitRow<NS> *)d_bp, d_path);
+    return HMMB_OK;
+}
+
+template <int NP, typename SymT>
+static int launch_viterbi_generic(SeqSet &s, const double *d_lpi, const double *d_lA, const double *d_lBt, double *d_score,
+                                  int8_t *d_last, uint8_t *d_bp) {
+    Ctx &c = ctx();
+    constexpr int GPW = 32 / NP;
+    int64_t grid = (std::max<int64_t>(s.R, 1) + BW_WARPS * GPW - 1) / (BW_WARPS * GPW);
+    grid = std::min<int64_t>(grid, (int64_t)c.sm_count * 16);
+    const int64_t total_groups = grid * BW_WARPS * GPW;
+    const int64_t per_group = (s.R + total_groups - 1) / total_groups;
+    HMMB_LAUNCH("viterbi", (k_viterbiG<NP, SymT>), (unsigned)grid, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len, s.d_word,
+                s.d_order, s.d_foff, s.R, per_group, s.N, s.M, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp);
+    return HMMB_OK;
+}
+
+int hmmb_viterbi(const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets, int64_t U,
+                 const int32_t *model_of_utt, int W, int N, int M, const double *pi, const double *A, const double *B,
+                 double *score_out, int8_t *path_out) {
+    HMMB_TRY(require_init());
+    if (!pi || !A || !B || W <= 0 || W > 65535 || (U > 0 && !model_of_utt)) {
+        set_error("hmmb_viterbi: bad arguments (W=%d)", W);
+        return HMMB_ERR_ARG;
+    }
+    Ctx &c = ctx();
+    SeqSet s;
+    struct Guard {
+        SeqSet &s; std::vector<void *> ptrs;
+        ~Guard() { s.release(); for (void *p : ptrs) dev_free(p); }
+    } guard{s, {}};
+    // the layouts and kernel families of hmmb_score: left-to-right models at N = 8 / 16 one utterance per thread
+    const bool ltr = ltr_shape_ok(N, M) && upper_bidiagonal(A, W, N);
+    HMMB_TRY(seqset_build(s, obs, idx_bytes, obs_on_device, offsets, model_of_utt, U, W, N, M, ltr ? LAYOUT_LTR : LAYOUT_AUTO));
+    if (U == 0) return HMMB_OK;
+    const size_t nB = (size_t)W * N * M, nA = (size_t)W * N * N, nP = (size_t)W * N;
+    double *tmp = nullptr, *d_lBt = nullptr, *d_lA = nullptr, *d_lpi = nullptr, *d_score = nullptr;
+    HMMB_TRY(dev_alloc_t(&tmp, nB + nA + nP)); guard.ptrs.push_back(tmp);
+    HMMB_TRY(dev_alloc_t(&d_lBt, nB + nA + nP)); guard.ptrs.push_back(d_lBt);
+    d_lA = d_lBt + nB;
+    d_lpi = d_lA + nA;
+    HMMB_TRY(dev_alloc_t(&d_score, (size_t)U)); guard.ptrs.push_back(d_score);
+    HMMB_CUDA(cudaMemcpyAsync(tmp, B, nB * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    HMMB_CUDA(cudaMemcpyAsync(tmp + nB, A, nA * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    HMMB_CUDA(cudaMemcpyAsync(tmp + nB + nA, pi, nP * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    HMMB_LAUNCH("viterbi_load", k_vit_logs, (unsigned)std::min<size_t>((nB + nA + nP + 255) / 256, (size_t)c.sm_count * 8), 256, 0,
+                tmp + 0, tmp + nB, tmp + nB + nA, W, N, M, d_lBt, d_lA, d_lpi);
+    // backpointers: blocked layouts one packed row per step and lane (1 byte per frame at N = 4 / 8, 2 at N = 16);
+    // generic layout one byte per state per frame
+    const bool want_path = path_out != nullptr;
+    int8_t *d_last = nullptr, *d_path = nullptr;
+    void *d_bp = nullptr;
+    if (want_path) {
+        const size_t row_bytes = s.ltr_ns == 16 ? 2 : 1;
+        const size_t bp_bytes = s.blocked() ? (size_t)s.spill_steps * 32 * row_bytes : (size_t)s.frames * N;
+        HMMB_TRY(dev_alloc(&d_bp, bp_bytes)); guard.ptrs.push_back(d_bp);
+        HMMB_TRY(dev_alloc_t(&d_last, (size_t)U)); guard.ptrs.push_back(d_last);
+        HMMB_TRY(dev_alloc_t(&d_path, (size_t)s.frames)); guard.ptrs.push_back(d_path);
+    }
+    int rc = HMMB_OK;
+    if (s.special4) {
+        rc = upper_bidiagonal(A, W, N) ? launch_viterbi_blocked<4, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)
+                                       : launch_viterbi_blocked<4, false>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp);
+        if (rc == HMMB_OK && want_path) rc = launch_vit_backtrace_blocked<4>(s, d_last, d_bp, d_path);
+    } else if (s.ltr_ns) {
+        rc = s.ltr_ns == 16 ? launch_viterbi_blocked<16, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)
+                            : launch_viterbi_blocked<8, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp);
+        if (rc == HMMB_OK && want_path)
+            rc = s.ltr_ns == 16 ? launch_vit_backtrace_blocked<16>(s, d_last, d_bp, d_path)
+                                : launch_vit_backtrace_blocked<8>(s, d_last, d_bp, d_path);
+    } else {
+        uint8_t *bp8 = (uint8_t *)d_bp;
+#define GEN(NPV)                                                                                                        \
+    case NPV:                                                                                                           \
+        rc = s.sym_bytes == 1 ? launch_viterbi_generic<NPV, uint8_t>(s, d_lpi, d_lA, d_lBt, d_score, d_last, bp8)       \
+                              : launch_viterbi_generic<NPV, uint16_t>(s, d_lpi, d_lA, d_lBt, d_score, d_last, bp8);     \
+        break;
+        switch (s.NP) {
+            GEN(4) GEN(8) GEN(16) GEN(32)
+            default: rc = HMMB_ERR_UNSUPPORTED;
+        }
+#undef GEN
+        if (rc == HMMB_OK && want_path)
+            HMMB_LAUNCH("viterbi_backtrace", k_vit_backtraceG, (unsigned)((U + VIT_THREADS - 1) / VIT_THREADS), VIT_THREADS, 0, U, N,
+                        s.d_len, s.d_off, s.d_foff, d_last, bp8, d_path);
+    }
+    HMMB_TRY(rc);
+    if (score_out) HMMB_TRY(d2h_big(score_out, d_score, (size_t)U * sizeof(double), c.stream));
+    if (want_path) HMMB_TRY(d2h_big(path_out, d_path, (size_t)s.frames, c.stream));
+    HMMB_CUDA(cudaStreamSynchronize(c.stream));
+    return HMMB_OK;
+}

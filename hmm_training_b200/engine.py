@@ -300,3 +300,38 @@ def score(obs, offsets, N: int, M: int, pi, A, B, obs_dev_ptr: Optional[int] = N
     arg = np.empty(max(U, 1), dtype=np.int32)
     check(lib.hmmb_score(op, ib, on_dev, ptr(offsets), U, W, N, M, ptr(pi), ptr(A), ptr(B), ptr(ll), ptr(arg)))
     return ll, arg[:U]
+
+
+def viterbi(obs, offsets, model_of_utt, N: int, M: int, pi, A, B, want_path: bool = True,
+            obs_dev_ptr: Optional[int] = None, idx_bytes: Optional[int] = None):
+    """Most likely state path of every utterance under its own model (hmmb_viterbi; an extension, the reference
+    has no Viterbi).  Utterance u is decoded against model model_of_utt[u]; pi [W,N], A [W,N,N], B [W,N,M] linear.
+
+    Returns (score float64 [U], path int8 [frames] or None): score[u] is the log-probability of the best path
+    (-inf if the utterance is impossible under its model), and frame t of utterance u is path[offsets[u] -
+    offsets[0] + t] (-1 on every frame of an impossible utterance).  want_path=False decodes the scores only."""
+    lib = _lib.load()
+    pi, A, B = c_f64(pi), c_f64(A), c_f64(B)
+    W = pi.shape[0]
+    if pi.shape != (W, N) or A.shape != (W, N, N) or B.shape != (W, N, M):
+        raise ValueError("model parameter shapes do not match (W, N, M)")
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+    U = len(offsets) - 1
+    model_of_utt = np.ascontiguousarray(model_of_utt, dtype=np.int32)
+    if model_of_utt.shape != (U,):
+        raise ValueError(f"model_of_utt must hold one model index per utterance ({U})")
+    if obs_dev_ptr is None:
+        obs = np.ascontiguousarray(obs)
+        if obs.dtype.kind == "i":
+            if obs.size and int(obs.min()) < 0:
+                raise IndexError("negative codeword index")
+            obs = obs.view({1: np.uint8, 2: np.uint16, 4: np.uint32, 8: np.uint64}[obs.dtype.itemsize])
+        op, on_dev, ib = ptr(obs), 0, obs.dtype.itemsize
+    else:
+        op, on_dev, ib = ctypes.c_void_p(obs_dev_ptr), 1, int(idx_bytes)
+    frames = int(offsets[-1] - offsets[0]) if U > 0 else 0
+    score = np.empty(max(U, 1))
+    path = np.empty(max(frames, 1), dtype=np.int8) if want_path else None
+    check(lib.hmmb_viterbi(op, ib, on_dev, ptr(offsets), U, ptr(model_of_utt), W, N, M, ptr(pi), ptr(A), ptr(B),
+                           ptr(score), ptr(path)))
+    return score[:U], (path[:frames] if want_path else None)

@@ -3,7 +3,8 @@
     calculate_log_likelihood   HMM/hmm_testing.py:49-104
     test_hmm                   HMM/hmm_testing.py:107-163
     create_confusion_matrix    HMM/hmm_testing.py:166-218
-plus ``score_all`` (every utterance against every model in one launch).
+plus ``score_all`` (every utterance against every model in one launch) and ``viterbi_align`` (the most
+likely state path of every utterance under a chosen model; an extension, the reference has no Viterbi).
 """
 from __future__ import annotations
 
@@ -54,6 +55,41 @@ def score_all(observations: Sequence[np.ndarray], all_hmm: Sequence[HMMTrained])
         arg[better] = w
         best[better] = ll[better, w]
     return ll, arg
+
+
+def viterbi_align(observations: Sequence[np.ndarray], all_hmm: Sequence[HMMTrained], model_index):
+    """Viterbi alignment of every utterance against the model all_hmm[model_index[u]] (for example score_all's
+    argmax, or the index of the utterance's known word for forced alignment).
+
+    Returns (scores float64 [U], paths: one int8 array of states per utterance): the log-probability of the best
+    state path and that path.  Index -1 ("unknown") and utterances impossible under their model give -inf and a
+    path of -1.  Models of different (states, symbols) are grouped as in score_all, one launch per group."""
+    seqs = [np.asarray(o) for o in observations]
+    idx = np.asarray(model_index, dtype=np.int64).reshape(-1)
+    if len(idx) != len(seqs):
+        raise ValueError(f"model_index has {len(idx)} entries for {len(seqs)} utterances")
+    if any(len(o) == 0 for o in seqs):
+        raise IndexError("index 0 is out of bounds for axis 0 with size 0")  # as score_all (hmm_testing.py:75)
+    if len(idx) and (int(idx.min()) < -1 or int(idx.max()) >= len(all_hmm)):
+        raise IndexError(f"model index outside [-1, {len(all_hmm)})")
+    scores = np.full(len(seqs), -np.inf)
+    paths = [np.full(len(o), -1, dtype=np.int8) for o in seqs]
+    groups: Dict[Tuple[int, int], List[int]] = {}
+    for w, h in enumerate(all_hmm):
+        groups.setdefault((int(h.states), int(h.symbols)), []).append(w)
+    for (N, M), cols in groups.items():
+        local = np.full(len(all_hmm) + 1, -1, dtype=np.int64)  # (slot -1 stays -1: "unknown")
+        local[cols] = np.arange(len(cols))
+        utts = np.nonzero(local[idx] >= 0)[0]
+        if len(utts) == 0:
+            continue
+        _, _, pi, A, B = _stack_models([all_hmm[w] for w in cols])
+        obs, offsets = _lib.pack_sequences([seqs[u] for u in utts], M)
+        sc, path = engine.viterbi(obs, offsets, local[idx[utts]], N, M, pi, A, B)
+        scores[utts] = sc
+        for k, u in enumerate(utts):
+            paths[u] = path[offsets[k]:offsets[k + 1]].copy()
+    return scores, paths
 
 
 def calculate_log_likelihood(recording_observations: np.ndarray, hmm: HMMTrained) -> float:

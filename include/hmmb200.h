@@ -216,6 +216,26 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
                int W, int N, int M, const double *pi, const double *A, const double *B,
                double *ll_out, int32_t *argmax_out);
 
+/* ------------------------------------------------------------------ Viterbi decoding
+ * An extension: the reference has no Viterbi.  The most likely state path of every utterance under its own model
+ * (utterance u against model model_of_utt[u], host array, values in [0, W)) and that path's log-probability, from
+ * LINEAR pi [W,N], A [W,N,N], B [W,N,M] (entries <= 0 or NaN are structural zeros, log = -inf):
+ *     delta_0(j) = log pi_j + log b_j(o_0)
+ *     delta_t(j) = (max_i (delta_t-1(i) + log a_ij)) + log b_j(o_t)
+ *     psi_t(j)   = the smallest i that reaches the max;  the last state is the smallest j that reaches
+ *                  max_j delta_T-1(j), and score_out[u] is that max.
+ * An utterance that is impossible under its model (score -inf) gets -1 for every frame.
+ * path_out [offsets[U] - offsets[0]] int8, input frame order: frame t of utterance u is at
+ * path_out[offsets[u] - offsets[0] + t].  path_out == NULL decodes the scores only (no backpointers are stored);
+ * score_out is then bit-identical to the call with a path.  score_out may be NULL.
+ * obs / idx_bytes / obs_on_device / offsets as for hmmb_score.  1 <= N <= 32, 1 <= M <= 65536, W <= 65535.
+ * Errors: HMMB_ERR_RANGE (codeword >= M), HMMB_ERR_EMPTY (empty utterance), HMMB_ERR_ARG (model index outside
+ * [0, W)), HMMB_ERR_UNSUPPORTED (N or M out of range), HMMB_ERR_OOM (the backpointers do not fit: 1 byte per frame
+ * at N = 4 and left-to-right N = 8, 2 at left-to-right N = 16, N bytes otherwise).                                */
+int hmmb_viterbi(const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets, int64_t U,
+                 const int32_t *model_of_utt, int W, int N, int M, const double *pi, const double *A,
+                 const double *B, double *score_out, int8_t *path_out);
+
 /* ------------------------------------------------------------------ MFCC front-end
  * Replaces RawDataMFCC.calculate_mfcc, CodeVector/codevector_classes.py:226-250, batched: F frames
  * of L samples each (Y [F,L] fp64, host or device) -> mfcc_out [F,13] (host), the coefficients of
