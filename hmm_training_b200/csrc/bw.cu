@@ -5,6 +5,7 @@
 #include <functional>
 #include <memory>
 #include <numeric>
+#include <type_traits>
 
 #include "bw_kernels.cuh"
 #include "bwltr_kernels.cuh"
@@ -312,12 +313,15 @@ static int score_stages(bool want_ll) {
 }
 
 // ---------------------------------------------------------------- sequence set (shared by BW and scoring)
+// Device layout of a sequence set: blocks of 32 same-word sequences for the N = 4 kernels or for the left-to-right
+// kernels (N = 8 / 16), or one codeword stream for the lanes-per-state kernels (any N)
+enum Layout { LAYOUT_LANES, LAYOUT_N4, LAYOUT_LTR };
+
 struct SeqSet {
     int64_t R = 0, frames = 0;
     int N = 0, M = 0, NP = 0, sym_bytes = 1;
-    bool special4 = false;            // blocked layout (32 same-word sequences per block), N = 4 kernels
-    int ltr_ns = 0;                   // blocked layout for the left-to-right kernels with NS = ltr_ns states
-    bool blocked() const { return special4 || ltr_ns != 0; }
+    Layout layout = LAYOUT_LANES;
+    bool blocked() const { return layout != LAYOUT_LANES; }
     std::vector<int32_t> order;       // sorted -> original
     std::vector<int64_t> seq_begin;   // per word [W+1] (sorted order)
     std::vector<int32_t> cta_begin;   // per word [W+1]
@@ -377,8 +381,7 @@ static int h2d_join() {
 static int pick_np(int N) { return N <= 4 ? 4 : (N <= 8 ? 8 : (N <= 16 ? 16 : 32)); }
 
 // Is every one of the W row-major N x N matrices A upper-bidiagonal (a_ij > 0 only for j = i or j = i + 1, the
-// reference's left-to-right topology)?  Zeros of A stay zeros under re-estimation, so the answer holds for a whole fit;
-// it selects the kernel family.
+// reference's left-to-right topology)?  Zeros of A stay zeros under re-estimation, so the answer holds for a whole fit.
 static bool upper_bidiagonal(const double *A, int W, int N) {
     const size_t nA = (size_t)W * N * N;
     for (size_t e = 0; e < nA; ++e) {
@@ -386,6 +389,65 @@ static bool upper_bidiagonal(const double *A, int W, int N) {
         if (j != i && j != i + 1 && A[e] > 0.0) return false;
     }
     return true;
+}
+
+// Kernel family of W models with N states, M codewords and the transition matrices A (nullptr: not known yet).
+struct Family {
+    Layout blocked;  // the blocked layout whose kernels hold this (N, M), LAYOUT_LANES if none does
+    bool bidiag;     // every A is upper-bidiagonal: the 7-term N = 4 kernels; LAYOUT_LTR requires it
+    Layout layout() const { return blocked == LAYOUT_LTR && !bidiag ? LAYOUT_LANES : blocked; }
+};
+
+// The one place that reads the switches routing models to the other kernel family: HMMB_FORCE_GENERIC (every shape to
+// the lanes-per-state kernels), HMMB_NO_LTR (N = 8 / 16 to them) and HMMB_FORCE_DENSE_A (A treated as dense).
+static Family pick_family(int N, int M, const double *A, int W) {
+    Family f{LAYOUT_LANES, A && !getenv("HMMB_FORCE_DENSE_A") && upper_bidiagonal(A, W, N)};
+    if (getenv("HMMB_FORCE_GENERIC")) return f;
+    if (N == 4 && M <= BW4_MAX_M) {
+        f.blocked = LAYOUT_N4;
+    } else if ((N == 8 || N == 16) && M <= LTR_MAX_SYM && !getenv("HMMB_NO_LTR")) {
+        // can the left-to-right kernels (bwltr_kernels.cuh) hold this model shape?
+        const size_t stage = (size_t)LTR_WARPS * 32 * (N * 8 + 16);
+        const size_t smem_b = (size_t)M * N * 8 + stage + (size_t)2 * N * 8 + (size_t)LTR_WARPS * 2 * N * 8 + 64;
+        if (smem_b <= ctx().smem_optin) f.blocked = LAYOUT_LTR;
+    }
+    return f;
+}
+
+// Calls f(std::integral_constant<int, NP>{}, SymT{}) with the lanes per state and the codeword type of the
+// lanes-per-state layout s, that is with the template arguments of its kernels.
+template <typename F>
+static int with_lanes(const SeqSet &s, F &&f) {
+    auto sym = [&](auto np) { return s.sym_bytes == 1 ? f(np, uint8_t{}) : f(np, uint16_t{}); };
+    switch (s.NP) {
+        case 4: return sym(std::integral_constant<int, 4>{});
+        case 8: return sym(std::integral_constant<int, 8>{});
+        case 16: return sym(std::integral_constant<int, 16>{});
+        case 32: return sym(std::integral_constant<int, 32>{});
+    }
+    return HMMB_ERR_UNSUPPORTED;
+}
+
+// Calls f(SymT{}, std::bool_constant<BLOCKED>{}) with how the codewords of s are stored: packed u16 entries in the
+// blocked layouts, 1 or 2 bytes each in the lanes-per-state layout (the exact and rescue kernels read either).
+template <typename F>
+static int with_codewords(const SeqSet &s, F &&f) {
+    if (s.blocked()) return f(uint16_t{}, std::true_type{});
+    return s.sym_bytes == 1 ? f(uint8_t{}, std::false_type{}) : f(uint16_t{}, std::false_type{});
+}
+
+// Grid of the lanes-per-state kernels over R sequences: NP lanes per group of one sequence at a time, at most 16 CTAs
+// per SM, each group taking per_group consecutive sequences.
+struct LanesGrid {
+    unsigned grid;
+    int64_t per_group;
+};
+static LanesGrid lanes_grid(int64_t R, int NP) {
+    const int64_t groups_per_cta = BW_WARPS * (32 / NP);
+    const int64_t grid = std::min<int64_t>((std::max<int64_t>(R, 1) + groups_per_cta - 1) / groups_per_cta,
+                                           (int64_t)ctx().sm_count * 16);
+    const int64_t total_groups = grid * groups_per_cta;
+    return {(unsigned)grid, (R + total_groups - 1) / total_groups};
 }
 
 // repack blocks [b0, b1) of the blocked layouts from the raw codewords (any input width)
@@ -448,21 +510,10 @@ static int launch_prepare(SeqSet &s, const InT *d_in, int64_t nsym, int *d_bad, 
 }
 
 // Sort sequences by (word, length desc), build blocks / CTA work items, move the codewords
-// to the device in the layout the kernels read.  word_of_seq == nullptr: a single "word"
+// to the device in `layout`.  word_of_seq == nullptr: a single "word"
 // (scoring: every utterance is scored against every model).
-enum SeqLayout { LAYOUT_GENERIC = 0, LAYOUT_AUTO = 1, LAYOUT_LTR = 2 };
-
-// can the left-to-right kernels (bwltr_kernels.cuh) hold this model shape?
-static bool ltr_shape_ok(int N, int M) {
-    if (N != 8 && N != 16) return false;
-    if (M > LTR_MAX_SYM) return false;
-    const size_t stage = (size_t)LTR_WARPS * 32 * (N * 8 + 16);
-    const size_t smem_b = (size_t)M * N * 8 + stage + (size_t)2 * N * 8 + (size_t)LTR_WARPS * 2 * N * 8 + 64;
-    return smem_b <= ctx().smem_optin && !getenv("HMMB_FORCE_GENERIC") && !getenv("HMMB_NO_LTR");
-}
-
 static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets,
-                        const int32_t *word_of_seq, int64_t R, int W, int N, int M, int layout, bool defer = false,
+                        const int32_t *word_of_seq, int64_t R, int W, int N, int M, Layout layout, bool defer = false,
                         const std::function<int()> *mid_hook = nullptr, int max_stages = 2) {
     Ctx &c = ctx();
     if (R < 0 || W <= 0 || !offsets || (R > 0 && !obs)) { set_error("bad sequence arguments"); return HMMB_ERR_ARG; }
@@ -471,8 +522,7 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
     if (idx_bytes != 1 && idx_bytes != 2 && idx_bytes != 4 && idx_bytes != 8) { set_error("idx_bytes must be 1, 2, 4 or 8"); return HMMB_ERR_ARG; }
     s.R = R; s.N = N; s.M = M; s.NP = pick_np(N);
     s.sym_bytes = M <= 256 ? 1 : 2;
-    s.special4 = layout == LAYOUT_AUTO && N == 4 && M <= BW4_MAX_M && !getenv("HMMB_FORCE_GENERIC");
-    s.ltr_ns = (layout == LAYOUT_LTR) ? N : 0;
+    s.layout = layout;
 
     std::unique_ptr<EarlyUpload> up_owner(new EarlyUpload());
     EarlyUpload &up = *up_owner;
@@ -620,7 +670,7 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
     int64_t obs_rows = 0;
     if (s.blocked()) {
         const int SPC = SPC4;  // packed u16 entries (codeword | conflict rank) per uint4
-        const int cta_warps = s.special4 ? BWD4_MAX_WARPS : LTR_WARPS;
+        const int cta_warps = s.layout == LAYOUT_N4 ? BWD4_MAX_WARPS : LTR_WARPS;
         std::vector<int> word_blk_begin(nwords + 1, 0);
         for (int w = 0; w < nwords; ++w) {
             word_blk_begin[w] = (int)blks.size();
@@ -642,9 +692,9 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         // CTA work items: ~2 per SM (N = 4) / ~4 per SM (left-to-right kernels, one 8-warp CTA per SM), at least one
         // warp-round each
         // (N = 4: one fat backward CTA per SM, about two waves; the forward kernel splits every item over FWD4_SPLIT CTAs)
-        const int target = s.special4 ? c.sm_count * 2 : c.sm_count * 4;
+        const int target = s.layout == LAYOUT_N4 ? c.sm_count * 2 : c.sm_count * 4;
         int bpc = std::max(1, (s.nblk + target - 1) / target);
-        if (bpc > 1 || !s.special4) bpc = (bpc + cta_warps - 1) / cta_warps * cta_warps;
+        if (bpc > 1 || s.layout != LAYOUT_N4) bpc = (bpc + cta_warps - 1) / cta_warps * cta_warps;
         s.cta_begin.assign(nwords + 1, 0);
         // N = 4, large inputs: EXACTLY `target` items of (almost) equal size, apportioned to the words by their block counts
         // (largest remainder).  The fat backward CTA works in rounds of 16 blocks and one CTA occupies an SM, so the kernel
@@ -652,7 +702,7 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         // CTA slots — 14 rounds per SM for 13.2 rounds of work, 16 SMs idle in the second wave.  296 items of 105.6 blocks
         // are 6 full rounds and one with 10 of the 16 warps busy, which is shorter than a full one.
         std::vector<int> items_of_word;
-        if (s.special4 && (int64_t)s.nblk >= (int64_t)target * cta_warps * 2) {
+        if (s.layout == LAYOUT_N4 && (int64_t)s.nblk >= (int64_t)target * cta_warps * 2) {
             items_of_word.assign(nwords, 0);
             std::vector<std::pair<double, int>> rem;
             int64_t assigned = 0;
@@ -704,7 +754,7 @@ static int seqset_build(SeqSet &s, const void *obs, int idx_bytes, int obs_on_de
         s.cta_begin[nwords] = (int)work.size();
         s.ncta = (int)work.size();
         s.ncta_fwd = (int)work_fwd.size();
-        if (s.special4 && defer) {
+        if (s.layout == LAYOUT_N4 && defer) {
             const int fine_items = c.sm_count * 8;  // about eight per SM (SeqSet::cta_begin_fine)
             int bpf = std::max(1, (s.nblk + fine_items - 1) / fine_items);
             if (bpf > 1) bpf = (bpf + cta_warps - 1) / cta_warps * cta_warps;
@@ -980,7 +1030,7 @@ static int bw_finish_create(hmmb_bw *h, int64_t R) {
     TRYF(dev_alloc_t(&h->d_seq_begin, (size_t)W + 1));
     TRYF(h2d_small(h->d_seq_begin, s.seq_begin.data(), (W + 1) * sizeof(int64_t)));
     size_t spill_bytes;
-    if (s.special4) {
+    if (s.layout == LAYOUT_N4) {
         // + BWD4_SPILL_PAD rows in front: k_bw_bwd4 loads row t - 2 unconditionally (for t < 2 that is the tail of
         // the previous block, or this padding for the first block; the values are never used)
         spill_bytes = (size_t)(std::max<int64_t>(s.spill_steps, 1) + BWD4_SPILL_PAD) * 64 * sizeof(double2);
@@ -1030,13 +1080,17 @@ int hmmb_bw_create_ex(hmmb_bw_t **out, const void *obs, int idx_bytes, int obs_o
     h->W = W; h->N = N; h->M = M;
     auto fail = [&](int code) { bw_release(h); delete h; return code; };
     int rc;
-    h->has_ltr = ltr_shape_ok(N, M);
     const bool have_params = pi0 && A0 && B0;
+    // N = 8 / 16: the generic layout in `s` and, if the left-to-right kernels hold the shape, the blocked one in `sl`
+    // (set_params picks between them)
+    const Family fam = pick_family(N, M, have_params ? A0 : nullptr, W);
+    const Layout s_layout = fam.blocked == LAYOUT_N4 ? LAYOUT_N4 : LAYOUT_LANES;
+    h->has_ltr = fam.blocked == LAYOUT_LTR;
     // Pipelined create for the left-to-right kernels (N = 8 / 16): pinned host codewords, initial parameters given
     // and every A upper-bidiagonal.  Only the blocked layout is built, and its repack is left to the first E-step.
-    const bool ltr_pipe = h->has_ltr && (flags & HMMB_BW_PIPELINE_UPLOAD) && have_params && !obs_on_device && R > 0 &&
-                          offsets && obs && offsets[R] > offsets[0] && !getenv("HMMB_FORCE_DENSE_A") &&
-                          host_is_pinned((const char *)obs + (size_t)offsets[0] * idx_bytes) && upper_bidiagonal(A0, W, N);
+    const bool ltr_pipe = fam.layout() == LAYOUT_LTR && (flags & HMMB_BW_PIPELINE_UPLOAD) && !obs_on_device && R > 0 &&
+                          offsets && obs && offsets[R] > offsets[0] &&
+                          host_is_pinned((const char *)obs + (size_t)offsets[0] * idx_bytes);
     if (h->has_ltr && !ltr_pipe && !obs_on_device && R > 0 && offsets && obs && offsets[R] > offsets[0]) {
         // both layouts are built from the codewords: upload them once
         const size_t in_bytes = (size_t)(offsets[R] - offsets[0]) * idx_bytes;
@@ -1080,7 +1134,7 @@ int hmmb_bw_create_ex(hmmb_bw_t **out, const void *obs, int idx_bytes, int obs_o
             // input not in (word, length descending) order: the build did the repack itself and its raw buffer is
             // gone, so the generic layout is built now, from the host codewords, as in a plain create
             h->ltr_only = false;
-            rc = seqset_build(h->s, obs, idx_bytes, 0, offsets, word_of_seq, R, W, N, M, LAYOUT_AUTO);
+            rc = seqset_build(h->s, obs, idx_bytes, 0, offsets, word_of_seq, R, W, N, M, s_layout);
             if (rc != HMMB_OK) return fail(rc);
         } else {
             h->keep_offsets.assign(offsets, offsets + R + 1);
@@ -1088,7 +1142,7 @@ int hmmb_bw_create_ex(hmmb_bw_t **out, const void *obs, int idx_bytes, int obs_o
         }
     } else {
         const bool pipeline = (flags & HMMB_BW_PIPELINE_UPLOAD) != 0 && !h->has_ltr;
-        rc = seqset_build(h->s, obs, idx_bytes, obs_on_device, offsets, word_of_seq, R, W, N, M, LAYOUT_AUTO, pipeline,
+        rc = seqset_build(h->s, obs, idx_bytes, obs_on_device, offsets, word_of_seq, R, W, N, M, s_layout, pipeline,
                           pipeline ? &finish : nullptr, PIPE_STAGES);
         if (rc != HMMB_OK) return fail(rc);
         if (h->has_ltr) {
@@ -1124,7 +1178,7 @@ int64_t hmmb_bw_total_frames(hmmb_bw_t *h) { return h ? h->s.frames : 0; }
 const char *hmmb_bw_kernel_family(hmmb_bw_t *h) {
     if (!h) return "";
     if (h->use_ltr) return "left_to_right";
-    if (h->s.special4) return h->bidiag ? "n4_left_to_right" : "n4_dense";
+    if (h->s.layout == LAYOUT_N4) return h->bidiag ? "n4_left_to_right" : "n4_dense";
     return "generic";
 }
 
@@ -1148,7 +1202,7 @@ static int bw_build_generic_lazily(hmmb_bw *h) {
     if (!h->d_raw) { set_error("dense transition matrices: the trainer no longer holds the raw codewords"); return HMMB_ERR_UNSUPPORTED; }
     const int64_t R = h->sl.R;
     HMMB_TRY(seqset_build(h->s, (const char *)h->d_raw - (size_t)h->keep_offsets[0] * h->raw_idx_bytes, h->raw_idx_bytes, 1,
-                          h->keep_offsets.data(), h->keep_words.data(), R, h->W, h->N, h->M, LAYOUT_AUTO));
+                          h->keep_offsets.data(), h->keep_words.data(), R, h->W, h->N, h->M, LAYOUT_LANES));
     // (bw_finish_create sized the alpha spill for both layouts already)
     h->ltr_only = false;
     dev_free(h->d_raw);
@@ -1269,8 +1323,8 @@ static int bw_set_params_impl(hmmb_bw *h, const double *pi0, const double *A0, c
     }
     // upper-bidiagonal A (the reference's left-to-right default) selects the 7-term N = 4 kernels and the
     // left-to-right kernels for N = 8 / 16
-    h->bidiag = N == 4 && upper_bidiagonal(A0, W, N) && !getenv("HMMB_FORCE_DENSE_A");
-    h->use_ltr = h->has_ltr && upper_bidiagonal(A0, W, N) && !getenv("HMMB_FORCE_DENSE_A");
+    h->bidiag = pick_family(N, M, A0, W).bidiag;
+    h->use_ltr = h->has_ltr && h->bidiag;
     if (h->ltr_only && !h->use_ltr) HMMB_TRY(bw_build_generic_lazily(h));
     HMMB_LAUNCH("bw_load", k_load_clamped, (unsigned)std::min<size_t>((nA + 255) / 256, 1024), 256, 0, tmp + nB, (int64_t)nA, h->d_A);
     HMMB_LAUNCH("bw_load", k_load_clamped, (unsigned)std::min<size_t>((nP + 255) / 256, 1024), 256, 0, tmp + nB + nA, (int64_t)nP, h->d_pi);
@@ -1352,21 +1406,60 @@ static int launch_exact(hmmb_bw *h) {
 
 template <int NP, typename SymT>
 static int launch_generic_estep(hmmb_bw *h) {
-    Ctx &c = ctx();
     SeqSet &s = h->s;
-    constexpr int GPW = 32 / NP;
-    const int64_t groups_needed = std::max<int64_t>(s.R, 1);
-    int64_t grid = (groups_needed + BW_WARPS * GPW - 1) / (BW_WARPS * GPW);
-    grid = std::min<int64_t>(grid, (int64_t)c.sm_count * 16);
-    const int64_t total_groups = grid * BW_WARPS * GPW;
-    const int64_t per_group = (s.R + total_groups - 1) / total_groups;
-    HMMB_LAUNCH("bw_forward", (k_bw_fwdG<NP, SymT>), (unsigned)grid, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len,
-                s.d_word, s.d_foff, s.R, per_group, h->N, h->M, h->d_pi, h->d_A, h->d_Bt, h->d_spill, h->d_llseq,
+    const LanesGrid g = lanes_grid(s.R, NP);
+    HMMB_LAUNCH("bw_forward", (k_bw_fwdG<NP, SymT>), g.grid, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len,
+                s.d_word, s.d_foff, s.R, g.per_group, h->N, h->M, h->d_pi, h->d_A, h->d_Bt, h->d_spill, h->d_llseq,
                 h->act_cur, h->d_flag);
     HMMB_TRY((launch_exact<SymT, false>(h)));
-    HMMB_LAUNCH("bw_backward", (k_bw_bwdG<NP, SymT>), (unsigned)grid, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len,
-                s.d_word, s.d_foff, s.R, per_group, h->N, h->M, h->d_A, h->d_Bt, h->d_spill, h->d_llseq, h->act_cur,
+    HMMB_LAUNCH("bw_backward", (k_bw_bwdG<NP, SymT>), g.grid, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len,
+                s.d_word, s.d_foff, s.R, g.per_group, h->N, h->M, h->d_A, h->d_Bt, h->d_spill, h->d_llseq, h->act_cur,
                 h->d_accum, h->astride, h->d_flag, h->d_newflags);
+    return HMMB_OK;
+}
+
+// First E-step of a pipelined fit on the blocked layout s (N = 4 or left-to-right): stage j = the blocks whose codewords
+// have landed (copy-stream event), repacked and pushed through forward + backward while the next chunks are still on
+// PCIe.  A stage is a fraction of a wave of CTAs, so consecutive stages go to two alternating side streams: the next
+// stage's repack and forward pass fill the SMs that the tail of this stage's backward pass leaves idle.  Everything a
+// stage writes (blocked codewords, spill, per-sequence results, per-CTA partials or fp64 atomics into the accumulators)
+// is private to its blocks; the compute stream joins both side streams afterwards.  stage(c0, c1) launches the work
+// items [c0, c1) on the context's stream.  Sequences the forward passes handed over are redone by the exact kernel after
+// the stages (their accumulator contributions are independent of the backward pass).
+template <typename StageFn>
+static int run_staged_estep(hmmb_bw *h, SeqSet &s, StageFn &&stage) {
+    Ctx &c = ctx();
+    PendingPrepare &p = *s.pend;
+    int bdone = 0, cdone = 0;
+    cudaStream_t main_stream = c.stream;
+    const bool side = p.nstage > 2;
+    struct Restore { Ctx &c; cudaStream_t s; ~Restore() { c.stream = s; } } restore{c, main_stream};
+    if (side) {
+        cudaEvent_t fork = event_get();
+        HMMB_CUDA(cudaEventRecord(fork, main_stream));
+        for (auto st : c.stage_stream) HMMB_CUDA(cudaStreamWaitEvent(st, fork, 0));
+        event_put(fork);
+    }
+    for (int j = 0; j < p.nstage; ++j) {
+        if (side) c.stream = c.stage_stream[j & 1];
+        HMMB_CUDA(cudaStreamWaitEvent(c.stream, p.up->ev[p.ev_index[j]], 0));
+        HMMB_TRY(launch_repack_range(s, p.up->d_raw, p.idx_bytes, bdone, p.blk_end[j], s.d_bad));
+        if (p.cta_end[j] > cdone) HMMB_TRY(stage(cdone, p.cta_end[j]));
+        bdone = p.blk_end[j];
+        cdone = p.cta_end[j];
+    }
+    c.stream = main_stream;
+    if (side) {
+        for (auto st : c.stage_stream) {
+            cudaEvent_t join = event_get();
+            HMMB_CUDA(cudaEventRecord(join, st));
+            HMMB_CUDA(cudaStreamWaitEvent(main_stream, join, 0));
+            event_put(join);
+        }
+    }
+    h->check_bad = true;
+    h->pend_release = std::move(s.pend);  // raw buffer + events: released after the next stream sync
+    HMMB_TRY((launch_exact<uint16_t, true>(h)));
     return HMMB_OK;
 }
 
@@ -1390,75 +1483,38 @@ static int launch_special_estep(hmmb_bw *h) {
     size_t smem_b = 0;
     const int bwd_threads = 32 * bwd4_warps(h->M, REP, BIDIAG, c.smem_optin, &smem_b);
     HMMB_CUDA(cudaFuncSetAttribute((k_bw_bwd4<BIDIAG, MT, REP>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-    // forward + backward of the CTA work items [c0, c1) of the staged E-step's list (the finer one where it exists)
-    const CtaWork *stage_work = s.ncta_fine > 0 ? s.d_work_fine : s.d_work;
-    const int stage_ncta = s.ncta_fine > 0 ? s.ncta_fine : s.ncta;
-    auto launch_range = [&](int c0, int c1) -> int {
-        if (c1 <= c0) return HMMB_OK;
-        HMMB_LAUNCH("bw_forward", k_bw_fwd4<BIDIAG>, (c1 - c0) * FWD4_SPLIT, BW_THREADS, smem_f, stage_work + c0, s.d_blks, (const uint4 *)s.d_obs,
-                    s.d_len, h->d_pi, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_flag,
-                    h->d_allfull, FWD4_SPLIT, SYM_MASK);
-        HMMB_LAUNCH("bw_backward", (k_bw_bwd4<BIDIAG, MT, REP>), c1 - c0, bwd_threads, smem_b, stage_work + c0, s.d_blks, (const uint4 *)s.d_obs,
-                    s.d_len, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_bzero,
+    // forward / backward pass over the CTA work items [c0, c1) of `list`
+    auto fwd = [&](const CtaWork *list, int c0, int c1) -> int {
+        HMMB_LAUNCH("bw_forward", k_bw_fwd4<BIDIAG>, (c1 - c0) * FWD4_SPLIT, BW_THREADS, smem_f, list + c0, s.d_blks,
+                    (const uint4 *)s.d_obs, s.d_len, h->d_pi, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur,
+                    h->d_flag, h->d_allfull, FWD4_SPLIT, SYM_MASK);
+        return HMMB_OK;
+    };
+    auto bwd = [&](const CtaWork *list, int c0, int c1) -> int {
+        HMMB_LAUNCH("bw_backward", (k_bw_bwd4<BIDIAG, MT, REP>), c1 - c0, bwd_threads, smem_b, list + c0, s.d_blks,
+                    (const uint4 *)s.d_obs, s.d_len, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_bzero,
                     h->d_allfull, h->d_partials + (size_t)c0 * h->pstride, h->pstride, h->d_flag, h->d_newflags);
         return HMMB_OK;
     };
     if (s.pend) {
-        // first E-step of a pipelined fit: stage j = the blocks whose codewords have landed (copy-stream event),
-        // repacked and pushed through forward + backward while the next chunks are still on PCIe
-        // A stage is a fraction of a wave of CTAs, so consecutive stages go to two alternating side streams:
-        // the next stage's repack and forward pass fill the SMs that the tail of this stage's backward pass
-        // leaves idle.  Everything a stage writes (blocked codewords, spill, per-sequence results, per-CTA
-        // partials) is private to its blocks; the compute stream joins both side streams afterwards.
-        PendingPrepare &p = *s.pend;
-        int bdone = 0, cdone = 0;
-        cudaStream_t main_stream = c.stream;
-        const bool side = p.nstage > 2;
-        struct Restore { Ctx &c; cudaStream_t s; ~Restore() { c.stream = s; } } restore{c, main_stream};
-        if (side) {
-            cudaEvent_t fork = event_get();
-            HMMB_CUDA(cudaEventRecord(fork, main_stream));
-            for (auto st : c.stage_stream) HMMB_CUDA(cudaStreamWaitEvent(st, fork, 0));
-            event_put(fork);
-        }
-        for (int j = 0; j < p.nstage; ++j) {
-            if (side) c.stream = c.stage_stream[j & 1];
-            HMMB_CUDA(cudaStreamWaitEvent(c.stream, p.up->ev[p.ev_index[j]], 0));
-            HMMB_TRY(launch_repack_range(s, p.up->d_raw, p.idx_bytes, bdone, p.blk_end[j], s.d_bad));
-            HMMB_TRY(launch_range(cdone, p.cta_end[j]));
-            bdone = p.blk_end[j];
-            cdone = p.cta_end[j];
-        }
-        c.stream = main_stream;
-        if (side) {
-            for (auto st : c.stage_stream) {
-                cudaEvent_t join = event_get();
-                HMMB_CUDA(cudaEventRecord(join, st));
-                HMMB_CUDA(cudaStreamWaitEvent(main_stream, join, 0));
-                event_put(join);
-            }
-        }
-        h->check_bad = true;
-        h->pend_release = std::move(s.pend);  // raw buffer + events: released after the next stream sync
-        // sequences this forward pass handed over are redone by the exact kernel after the stages (their
-        // accumulator contributions are independent of the backward pass); the per-CTA statistic, taken inside
-        // k_bw_bwd4 while those sequences still carried their NaN mark, is then retaken
-        HMMB_TRY((launch_exact<uint16_t, true>(h)));
+        // the staged E-step launches from the finer work list where it exists
+        const CtaWork *stage_work = s.ncta_fine > 0 ? s.d_work_fine : s.d_work;
+        const int stage_ncta = s.ncta_fine > 0 ? s.ncta_fine : s.ncta;
+        HMMB_TRY(run_staged_estep(h, s, [&](int c0, int c1) -> int {
+            HMMB_TRY(fwd(stage_work, c0, c1));
+            return bwd(stage_work, c0, c1);
+        }));
+        // the per-CTA statistic, taken inside k_bw_bwd4 while the sequences the exact kernel redid still carried their
+        // NaN mark, is retaken
         HMMB_LAUNCH("bw_exact", k_bw_llstat_fix, stage_ncta, BW_THREADS, 0, stage_work, s.d_blks, h->d_llseq, h->act_cur,
                     h->d_flag, h->d_partials, h->pstride, h->M);
         h->estep_fine = s.ncta_fine > 0;  // k_bw_reduce sums this E-step's partials over the finer list's per-word ranges
         return HMMB_OK;
     }
     h->estep_fine = false;
-    HMMB_LAUNCH("bw_forward", k_bw_fwd4<BIDIAG>, (s.ncta_fwd ? s.ncta_fwd : s.ncta) * FWD4_SPLIT, BW_THREADS, smem_f,
-                s.ncta_fwd ? s.d_work_fwd : s.d_work, s.d_blks, (const uint4 *)s.d_obs,
-                s.d_len, h->d_pi, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_flag,
-                h->d_allfull, FWD4_SPLIT, SYM_MASK);
+    HMMB_TRY(s.ncta_fwd ? fwd(s.d_work_fwd, 0, s.ncta_fwd) : fwd(s.d_work, 0, s.ncta));
     HMMB_TRY((launch_exact<uint16_t, true>(h)));
-    HMMB_LAUNCH("bw_backward", (k_bw_bwd4<BIDIAG, MT, REP>), s.ncta, bwd_threads, smem_b, s.d_work, s.d_blks, (const uint4 *)s.d_obs,
-                s.d_len, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_bzero,
-                h->d_allfull, h->d_partials, h->pstride, h->d_flag, h->d_newflags);
-    return HMMB_OK;
+    return bwd(s.d_work, 0, s.ncta);
 }
 
 template <int NS>
@@ -1471,71 +1527,38 @@ static int launch_ltr_estep(hmmb_bw *h) {
                           (size_t)LTR_WARPS * 2 * NS * 8;
     HMMB_CUDA(cudaFuncSetAttribute(k_bw_fwdL<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_f));
     HMMB_CUDA(cudaFuncSetAttribute(k_bw_bwdL<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+    // forward / backward pass over the CTA work items [c0, c1)
+    auto fwd = [&](int c0, int c1) -> int {
+        HMMB_LAUNCH("bw_forward", k_bw_fwdL<NS>, c1 - c0, LTR_THREADS, smem_f, s.d_work + c0, s.d_blks, (const uint4 *)s.d_obs,
+                    s.d_len, h->d_pi, h->d_A, h->d_Bt, M, (double2 *)h->d_spill, h->d_llseq, h->act_cur, h->d_flag,
+                    h->d_allfull);
+        return HMMB_OK;
+    };
+    auto bwd = [&](int c0, int c1) -> int {
+        HMMB_LAUNCH("bw_backward", k_bw_bwdL<NS>, c1 - c0, LTR_THREADS, smem_b, s.d_work + c0, s.d_blks, (const uint4 *)s.d_obs,
+                    s.d_len, h->d_A, h->d_Bt, M, (const double2 *)h->d_spill, h->d_llseq, h->act_cur, h->d_bzero,
+                    h->d_allfull, h->d_accum, h->astride, h->d_flag, h->d_newflags);
+        return HMMB_OK;
+    };
     if (s.pend) {
-        // First E-step of a pipelined create (see launch_special_estep): stage j = the blocks whose codewords have
-        // landed, repacked and pushed through forward + backward on two alternating side streams while the later
-        // chunks are still on PCIe.  The accumulators take fp64 atomics from every stage, the exact kernel runs
-        // after the stages (its contributions do not depend on the backward pass), and the convergence statistic
-        // is taken from the per-sequence values by k_bw_reduce afterwards, so nothing has to be retaken.
-        Ctx &c = ctx();
-        PendingPrepare &p = *s.pend;
-        int bdone = 0, cdone = 0;
-        cudaStream_t main_stream = c.stream;
-        const bool side = p.nstage > 2;
-        struct Restore { Ctx &c; cudaStream_t s; ~Restore() { c.stream = s; } } restore{c, main_stream};
-        if (side) {
-            cudaEvent_t fork = event_get();
-            HMMB_CUDA(cudaEventRecord(fork, main_stream));
-            for (auto st : c.stage_stream) HMMB_CUDA(cudaStreamWaitEvent(st, fork, 0));
-            event_put(fork);
-        }
-        for (int j = 0; j < p.nstage; ++j) {
-            if (side) c.stream = c.stage_stream[j & 1];
-            HMMB_CUDA(cudaStreamWaitEvent(c.stream, p.up->ev[p.ev_index[j]], 0));
-            HMMB_TRY(launch_repack_range(s, p.up->d_raw, p.idx_bytes, bdone, p.blk_end[j], s.d_bad));
-            const int c0 = cdone, c1 = p.cta_end[j];
-            if (c1 > c0 && h->bpieces_issued > 0) {
+        // the accumulators take fp64 atomics from every stage and the convergence statistic is taken from the
+        // per-sequence values by k_bw_reduce afterwards, so nothing has to be retaken after the exact kernel
+        return run_staged_estep(h, s, [&](int c0, int c1) -> int {
+            if (h->bpieces_issued > 0) {
                 // B^T of this stage's words (pieces are word ranges [W p / P, W (p + 1) / P), ready in order)
                 const int w_last = (int)(std::upper_bound(s.cta_begin.begin(), s.cta_begin.end(), c1 - 1) - s.cta_begin.begin()) - 1;
                 int need = 0;
                 while (need < h->bpieces - 1 && (int64_t)h->W * (need + 1) / h->bpieces <= w_last) ++need;
-                HMMB_CUDA(cudaStreamWaitEvent(c.stream, h->bt_ready[need], 0));
+                HMMB_CUDA(cudaStreamWaitEvent(ctx().stream, h->bt_ready[need], 0));
             }
-            if (c1 > c0) {
-                HMMB_LAUNCH("bw_forward", k_bw_fwdL<NS>, c1 - c0, LTR_THREADS, smem_f, s.d_work + c0, s.d_blks, (const uint4 *)s.d_obs,
-                            s.d_len, h->d_pi, h->d_A, h->d_Bt, M, (double2 *)h->d_spill, h->d_llseq, h->act_cur, h->d_flag,
-                            h->d_allfull);
-                HMMB_LAUNCH("bw_backward", k_bw_bwdL<NS>, c1 - c0, LTR_THREADS, smem_b, s.d_work + c0, s.d_blks, (const uint4 *)s.d_obs,
-                            s.d_len, h->d_A, h->d_Bt, M, (const double2 *)h->d_spill, h->d_llseq, h->act_cur, h->d_bzero,
-                            h->d_allfull, h->d_accum, h->astride, h->d_flag, h->d_newflags);
-            }
-            bdone = p.blk_end[j];
-            cdone = p.cta_end[j];
-        }
-        c.stream = main_stream;
-        if (side) {
-            for (auto st : c.stage_stream) {
-                cudaEvent_t join = event_get();
-                HMMB_CUDA(cudaEventRecord(join, st));
-                HMMB_CUDA(cudaStreamWaitEvent(main_stream, join, 0));
-                event_put(join);
-            }
-        }
-        h->check_bad = true;
-        h->pend_release = std::move(s.pend);
-        HMMB_TRY((launch_exact<uint16_t, true>(h)));
-        return HMMB_OK;
+            HMMB_TRY(fwd(c0, c1));
+            return bwd(c0, c1);
+        });
     }
-    HMMB_LAUNCH("bw_forward", k_bw_fwdL<NS>, s.ncta, LTR_THREADS, smem_f, s.d_work, s.d_blks, (const uint4 *)s.d_obs, s.d_len,
-                h->d_pi, h->d_A, h->d_Bt, M, (double2 *)h->d_spill, h->d_llseq, h->act_cur, h->d_flag, h->d_allfull);
+    HMMB_TRY(fwd(0, s.ncta));
     HMMB_TRY((launch_exact<uint16_t, true>(h)));
     const int groups = (h->allreduce && h->world > 1) ? std::min(h->overlap_groups, h->W) : 1;
-    if (groups <= 1) {
-        HMMB_LAUNCH("bw_backward", k_bw_bwdL<NS>, s.ncta, LTR_THREADS, smem_b, s.d_work, s.d_blks, (const uint4 *)s.d_obs, s.d_len,
-                    h->d_A, h->d_Bt, M, (const double2 *)h->d_spill, h->d_llseq, h->act_cur, h->d_bzero, h->d_allfull,
-                    h->d_accum, h->astride, h->d_flag, h->d_newflags);
-        return HMMB_OK;
-    }
+    if (groups <= 1) return bwd(0, s.ncta);
     // Communication / compute overlap (config 4: 133 MB of accumulators per iteration).  The convergence
     // statistic and the sequence counts only need the forward pass, so k_bw_reduce runs first; the backward
     // pass then goes word group by word group, and each group's slice of the accumulator buffer is handed to the
@@ -1547,10 +1570,7 @@ static int launch_ltr_estep(hmmb_bw *h) {
     for (int g = 0; g < groups; ++g) {
         const int w0 = (int)((int64_t)h->W * g / groups), w1 = (int)((int64_t)h->W * (g + 1) / groups);
         const int c0 = s.cta_begin[w0], c1 = s.cta_begin[w1];
-        if (c1 > c0)
-            HMMB_LAUNCH("bw_backward", k_bw_bwdL<NS>, c1 - c0, LTR_THREADS, smem_b, s.d_work + c0, s.d_blks, (const uint4 *)s.d_obs,
-                        s.d_len, h->d_A, h->d_Bt, M, (const double2 *)h->d_spill, h->d_llseq, h->act_cur, h->d_bzero,
-                        h->d_allfull, h->d_accum, h->astride, h->d_flag, h->d_newflags);
+        if (c1 > c0) HMMB_TRY(bwd(c0, c1));
         int rc = h->allreduce(h->d_accum + (size_t)w0 * h->astride, (int64_t)(w1 - w0) * h->astride, h->user);
         if (rc != 0) { set_error("allreduce hook failed (%d)", rc); return HMMB_ERR_CUDA; }
     }
@@ -1564,19 +1584,12 @@ static int launch_ltr_estep(hmmb_bw *h) {
 static int bw_estep(hmmb_bw *h) {
     if (h->use_ltr) return h->N == 16 ? launch_ltr_estep<16>(h) : launch_ltr_estep<8>(h);
     SeqSet &s = h->s;
-    if (s.special4) {
+    if (s.layout == LAYOUT_N4) {
         if (h->M == 256) return h->bidiag ? launch_special_estep<true, 256, BWD4_REP>(h) : launch_special_estep<false, 256, BWD4_REP>(h);
         if (h->M < 256) return h->bidiag ? launch_special_estep<true, 0, BWD4_REP>(h) : launch_special_estep<false, 0, BWD4_REP>(h);
         return h->bidiag ? launch_special_estep<true, 0, 1>(h) : launch_special_estep<false, 0, 1>(h);
     }
-#define GEN(NPV)                                                                               \
-    case NPV:                                                                                  \
-        return s.sym_bytes == 1 ? launch_generic_estep<NPV, uint8_t>(h) : launch_generic_estep<NPV, uint16_t>(h);
-    switch (s.NP) {
-        GEN(4) GEN(8) GEN(16) GEN(32)
-    }
-#undef GEN
-    return HMMB_ERR_UNSUPPORTED;
+    return with_lanes(s, [&](auto np, auto sym) { return launch_generic_estep<decltype(np)::value, decltype(sym)>(h); });
 }
 
 // Called right after a cudaStreamSynchronize of the compute stream: the pipelined prepare's upload
@@ -1613,19 +1626,12 @@ static int launch_rescue(hmmb_bw *h) {
     double *own = rescue_base(h) + (size_t)h->rank * h->slot_cap * h->rstride;
     const int64_t n = h->slot_cap * h->rstride;
     HMMB_LAUNCH("bw_rescue", k_bw_rescue_init, (unsigned)std::min<int64_t>((n + 255) / 256, 1024), 256, 0, own, n);
-#define RESCUE(SYMT, BLK, BASE)                                                                                       \
-    HMMB_LAUNCH("bw_rescue", (k_bw_rescue<SYMT, BLK>), h->exact_grid, BW_THREADS, 0, s.d_obs, BASE, s.d_len, s.d_word, s.R, \
-                h->N, h->M, h->d_pi, h->d_A, h->d_Bt, h->act_cur, h->d_exact_scratch, h->exact_stride, h->d_thinmask, \
-                h->d_slot_of, own, h->rstride, SYM_MASK)
-    if (s.blocked()) {
-        RESCUE(uint16_t, true, s.d_foff);
-    } else if (s.sym_bytes == 1) {
-        RESCUE(uint8_t, false, s.d_off);
-    } else {
-        RESCUE(uint16_t, false, s.d_off);
-    }
-#undef RESCUE
-    return HMMB_OK;
+    return with_codewords(s, [&](auto sym, auto blocked) -> int {
+        HMMB_LAUNCH("bw_rescue", (k_bw_rescue<decltype(sym), decltype(blocked)::value>), h->exact_grid, BW_THREADS, 0, s.d_obs,
+                    blocked() ? s.d_foff : s.d_off, s.d_len, s.d_word, s.R, h->N, h->M, h->d_pi, h->d_A, h->d_Bt, h->act_cur,
+                    h->d_exact_scratch, h->exact_stride, h->d_thinmask, h->d_slot_of, own, h->rstride, SYM_MASK);
+        return HMMB_OK;
+    });
 }
 
 // Called after a stream synchronisation with the number of states the M-step has newly flagged: gives every flagged
@@ -1677,9 +1683,10 @@ static int bw_one_pass(hmmb_bw *h, int32_t *mask, double eps, int max_iter, int 
     }
     HMMB_TRY(launch_rescue(h));
     if (!h->estep_reduced) {
-        const dim3 rgrid((unsigned)h->W, h->s.special4 ? (unsigned)((h->nacc + RED_EX - 1) / RED_EX) : 1u);
-        HMMB_LAUNCH("bw_reduce", k_bw_reduce, rgrid, RED_THREADS, 0, h->s.special4 ? h->d_partials : nullptr, h->pstride,
-                    (h->s.special4 && h->estep_fine) ? h->d_cta_begin_fine : h->d_cta_begin, h->d_llseq, h->d_seq_begin, h->d_accum, h->astride, h->nacc,
+        const bool n4 = h->s.layout == LAYOUT_N4;  // the N = 4 E-step leaves per-CTA partials
+        const dim3 rgrid((unsigned)h->W, n4 ? (unsigned)((h->nacc + RED_EX - 1) / RED_EX) : 1u);
+        HMMB_LAUNCH("bw_reduce", k_bw_reduce, rgrid, RED_THREADS, 0, n4 ? h->d_partials : nullptr, h->pstride,
+                    (n4 && h->estep_fine) ? h->d_cta_begin_fine : h->d_cta_begin, h->d_llseq, h->d_seq_begin, h->d_accum, h->astride, h->nacc,
                     h->d_accum + (size_t)h->W * h->astride, h->rank, h->W, mask);
         if (h->allreduce && h->world > 1) {
             static int pid_ar = -1;
@@ -1832,58 +1839,54 @@ int hmmb_bw_fit(const void *obs, int idx_bytes, const int64_t *offsets, const in
 }
 
 // ---------------------------------------------------------------- recognition
+// The sequence set and device buffers of one hmmb_score / hmmb_viterbi call, released however the call returns.
+struct CallGuard {
+    SeqSet &s;
+    std::vector<void *> ptrs;
+    ~CallGuard() { s.release(); for (void *p : ptrs) dev_free(p); }
+};
+
 template <int NP, typename SymT>
 static int launch_score_generic(SeqSet &s, int W, const double *d_pi, const double *d_A, const double *d_Bt, double *d_ll, int32_t *d_nan) {
-    Ctx &c = ctx();
-    constexpr int GPW = 32 / NP;
-    int64_t grid = (std::max<int64_t>(s.R, 1) + BW_WARPS * GPW - 1) / (BW_WARPS * GPW);
-    grid = std::min<int64_t>(grid, (int64_t)c.sm_count * 16);
-    const int64_t total_groups = grid * BW_WARPS * GPW;
-    const int64_t per_group = (s.R + total_groups - 1) / total_groups;
-    dim3 g((unsigned)grid, (unsigned)W);
+    const LanesGrid lg = lanes_grid(s.R, NP);
+    dim3 g(lg.grid, (unsigned)W);
     HMMB_LAUNCH("score", (k_scoreG<NP, SymT>), g, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len, s.d_order, s.R,
-                per_group, s.N, s.M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
+                lg.per_group, s.N, s.M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
     return HMMB_OK;
 }
 
-template <bool BIDIAG>
-static int launch_score_special(SeqSet &s, int W, const double *d_pi, const double *d_A, const double *d_Bt, double *d_ll, int32_t *d_nan,
-                                int b0 = 0, int b1 = -1) {
+// N = 4 scorers over the blocks [b0, b1) (a stage of the pipelined scorer, or all of them); bidiag: every A is
+// upper-bidiagonal
+static int launch_score_special(SeqSet &s, bool bidiag, int W, const double *d_pi, const double *d_A, const double *d_Bt,
+                                double *d_ll, int32_t *d_nan, int b0, int b1) {
     Ctx &c = ctx();
-    if (b1 < 0) b1 = s.nblk;
-    const int nb = b1 - b0;  // blocks [b0, b1) (a stage of the pipelined scorer, or all of them)
+    const int nb = b1 - b0;
     if (nb <= 0) return HMMB_OK;
+    // both scorers have one signature; [BIDIAG][VECB] picks the instance
+    using Score4 = decltype(&k_score4<false, false>);
+    const bool vecb = s.tmax_all > SCORE4_SCALAR_BOUND_MAX_T;
     if (s.M <= SCORE4R_MAX_M) {
+        const Score4 k[2][2] = {{k_score4r<false, false>, k_score4r<false, true>}, {k_score4r<true, false>, k_score4r<true, true>}};
         // replicated-B scorer: 8 warps per CTA, 2 CTAs per SM, about six waves of CTAs
         int bpc = std::max(SCORE4R_WARPS, (int)(((int64_t)nb * W + c.sm_count * 12 - 1) / (c.sm_count * 12)));
         bpc = (bpc + SCORE4R_WARPS - 1) / SCORE4R_WARPS * SCORE4R_WARPS;
         bpc = std::min(bpc, 128);
         dim3 g((unsigned)((nb + bpc - 1) / bpc), (unsigned)W);
         const size_t smem = (size_t)SCORE4R_MAX_M * SCORE4R_REP * 2 * sizeof(double2) + (size_t)s.M * sizeof(double) + (size_t)((s.M + 15) & ~15);
-        if (s.tmax_all > SCORE4_SCALAR_BOUND_MAX_T) {
-            HMMB_CUDA(cudaFuncSetAttribute((k_score4r<BIDIAG, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            HMMB_LAUNCH("score", (k_score4r<BIDIAG, true>), g, SCORE4R_WARPS * 32, smem, s.d_blks + b0, nb, bpc, (const uint4 *)s.d_obs,
-                        s.d_len, s.d_order, d_pi, d_A, d_Bt, s.M, W, d_ll, d_nan);
-        } else {
-            HMMB_CUDA(cudaFuncSetAttribute((k_score4r<BIDIAG, false>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            HMMB_LAUNCH("score", (k_score4r<BIDIAG, false>), g, SCORE4R_WARPS * 32, smem, s.d_blks + b0, nb, bpc, (const uint4 *)s.d_obs,
-                        s.d_len, s.d_order, d_pi, d_A, d_Bt, s.M, W, d_ll, d_nan);
-        }
+        HMMB_CUDA(cudaFuncSetAttribute(k[bidiag][vecb], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        HMMB_LAUNCH("score", k[bidiag][vecb], g, SCORE4R_WARPS * 32, smem, s.d_blks + b0, nb, bpc, (const uint4 *)s.d_obs,
+                    s.d_len, s.d_order, d_pi, d_A, d_Bt, s.M, W, d_ll, d_nan);
         return HMMB_OK;
     }
+    const Score4 k[2][2] = {{k_score4<false, false>, k_score4<false, true>}, {k_score4<true, false>, k_score4<true, true>}};
     // each CTA re-uses one model's B for several 32-utterance blocks
     int bpc = std::max(BW_WARPS, (s.nblk * W + c.sm_count * 16 - 1) / (c.sm_count * 16));
     bpc = (bpc + BW_WARPS - 1) / BW_WARPS * BW_WARPS;
     bpc = std::min(bpc, 64);
     dim3 g((unsigned)((nb + bpc - 1) / bpc), (unsigned)W);
     const size_t smem = (size_t)s.M * 5 * sizeof(double) + (size_t)((s.M + 15) & ~15);
-    if (s.tmax_all > SCORE4_SCALAR_BOUND_MAX_T) {
-        HMMB_LAUNCH("score", (k_score4<BIDIAG, true>), g, BW_THREADS, smem, s.d_blks + b0, nb, bpc, (const uint4 *)s.d_obs, s.d_len,
-                    s.d_order, d_pi, d_A, d_Bt, s.M, W, d_ll, d_nan);
-    } else {
-        HMMB_LAUNCH("score", (k_score4<BIDIAG, false>), g, BW_THREADS, smem, s.d_blks + b0, nb, bpc, (const uint4 *)s.d_obs, s.d_len,
-                    s.d_order, d_pi, d_A, d_Bt, s.M, W, d_ll, d_nan);
-    }
+    HMMB_LAUNCH("score", k[bidiag][vecb], g, BW_THREADS, smem, s.d_blks + b0, nb, bpc, (const uint4 *)s.d_obs, s.d_len,
+                s.d_order, d_pi, d_A, d_Bt, s.M, W, d_ll, d_nan);
     return HMMB_OK;
 }
 
@@ -1904,12 +1907,8 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
     if (!pi || !A || !B || W <= 0 || W > 65535) { set_error("hmmb_score: bad arguments (W=%d)", W); return HMMB_ERR_ARG; }
     Ctx &c = ctx();
     SeqSet s;
-    struct Guard {
-        SeqSet &s; std::vector<void *> ptrs;
-        ~Guard() { s.release(); for (void *p : ptrs) dev_free(p); }
-    } guard{s, {}};
-    // left-to-right models at N = 8 / 16 are scored one utterance per thread (k_scoreL)
-    const bool ltr = ltr_shape_ok(N, M) && upper_bidiagonal(A, W, N);
+    CallGuard guard{s, {}};
+    const Family fam = pick_family(N, M, A, W);
     const size_t nB = (size_t)W * N * M, nA = (size_t)W * N * N, nP = (size_t)W * N;
     double *tmp = nullptr, *d_pi = nullptr, *d_A = nullptr, *d_Bt = nullptr, *d_ll = nullptr;
     int32_t *d_arg = nullptr;
@@ -1941,97 +1940,74 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
     // Pipelined scorer (N = 4, pinned codewords in length-descending order, small models): the stages of the
     // upload are repacked and scored as they land, and each stage's rows of the [U, W] matrix start their way back
     // to the host while the next stage is being scored.
-    const bool pipeline = !ltr && nB * sizeof(double) <= (size_t(4) << 20) && !getenv("HMMB_SCORE_NO_PIPELINE");
-    HMMB_TRY(seqset_build(s, obs, idx_bytes, obs_on_device, offsets, nullptr, U, 1, N, M, ltr ? LAYOUT_LTR : LAYOUT_AUTO,
-                          pipeline, pipeline ? &upload_models : nullptr, score_stages(ll_out != nullptr)));
+    const bool pipeline = fam.layout() != LAYOUT_LTR && nB * sizeof(double) <= (size_t(4) << 20) && !getenv("HMMB_SCORE_NO_PIPELINE");
+    HMMB_TRY(seqset_build(s, obs, idx_bytes, obs_on_device, offsets, nullptr, U, 1, N, M, fam.layout(), pipeline,
+                          pipeline ? &upload_models : nullptr, score_stages(ll_out != nullptr)));
     if (U == 0) return HMMB_OK;
     if (!models_up) HMMB_TRY(upload_models());
-    if (s.pend) {
-        const bool bidiag = upper_bidiagonal(A, W, N);
-        PendingPrepare &p = *s.pend;
-        int bdone = 0;
-        // a pageable result matrix cannot leave stage by stage (its copies would block the host between the
-        // stages): it goes through the bounce buffers after the last stage
-        const bool ll_pinned = ll_out && host_is_pinned(ll_out);
-        cudaEvent_t scored = event_get();
-        for (int j = 0; j < p.nstage; ++j) {
-            HMMB_CUDA(cudaStreamWaitEvent(c.stream, p.up->ev[p.ev_index[j]], 0));
-            HMMB_TRY(launch_repack_range(s, p.up->d_raw, p.idx_bytes, bdone, p.blk_end[j], s.d_bad));
-            HMMB_TRY(bidiag ? launch_score_special<true>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan, bdone, p.blk_end[j])
-                            : launch_score_special<false>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan, bdone, p.blk_end[j]));
-            if (ll_out && ll_pinned) {
-                // scoring has a single "word", so block b holds utterances [32 b, 32 b + 32) of the (identity) order
-                const int64_t u0 = (int64_t)bdone * 32, u1 = std::min<int64_t>(U, (int64_t)p.blk_end[j] * 32);
-                HMMB_CUDA(cudaEventRecord(scored, c.stream));
-                HMMB_CUDA(cudaStreamWaitEvent(c.d2h_stream, scored, 0));
-                HMMB_CUDA(cudaMemcpyAsync(ll_out + u0 * W, d_ll + u0 * W, (size_t)(u1 - u0) * W * sizeof(double),
-                                          cudaMemcpyDeviceToHost, c.d2h_stream));
-            }
-            bdone = p.blk_end[j];
-        }
-        event_put(scored);
-        HMMB_LAUNCH("score_argmax", k_argmax_first, (unsigned)((U + 255) / 256), 256, 0, d_ll, U, W, d_arg);
-        int32_t flags[2] = {0, 0};
-        HMMB_CUDA(cudaMemcpyAsync(&flags[0], d_nan, sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
-        HMMB_CUDA(cudaMemcpyAsync(&flags[1], s.d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
-        if (argmax_out) HMMB_CUDA(cudaMemcpyAsync(argmax_out, d_arg, (size_t)U * sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
-        if (ll_out && !ll_pinned) HMMB_TRY(d2h_big(ll_out, d_ll, (size_t)U * W * sizeof(double), c.stream));
-        HMMB_CUDA(cudaStreamSynchronize(c.stream));
-        HMMB_CUDA(cudaStreamSynchronize(c.d2h_stream));
-        s.pend.reset();
-        if (flags[1]) {
-            set_error("codeword out of range: some observation is >= M=%d (reference: IndexError)", M);
-            return HMMB_ERR_RANGE;
-        }
-        if (flags[0]) {
-            // rare: the precision guard marked pairs; recompute them in log space and send everything again
+    // [exact recompute of the pairs the precision guard marked,] argmax, results to the host
+    auto finish = [&](bool recompute, bool send_ll) -> int {
+        if (recompute) {
             const int64_t warps = std::min<int64_t>((int64_t)c.sm_count * 16, U);
             const int eg = (int)std::max<int64_t>(1, (warps + BW_WARPS - 1) / BW_WARPS);
-            HMMB_LAUNCH("score_exact", (k_score_exact<uint16_t, true>), eg, BW_THREADS, 0, s.d_obs, s.d_foff, s.d_len, s.d_order, U, N, M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
-            HMMB_LAUNCH("score_argmax", k_argmax_first, (unsigned)((U + 255) / 256), 256, 0, d_ll, U, W, d_arg);
-            if (argmax_out) HMMB_CUDA(cudaMemcpyAsync(argmax_out, d_arg, (size_t)U * sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
-            if (ll_out) HMMB_TRY(d2h_big(ll_out, d_ll, (size_t)U * W * sizeof(double), c.stream));
-            HMMB_CUDA(cudaStreamSynchronize(c.stream));
+            HMMB_TRY(with_codewords(s, [&](auto sym, auto blocked) -> int {
+                HMMB_LAUNCH("score_exact", (k_score_exact<decltype(sym), decltype(blocked)::value>), eg, BW_THREADS, 0, s.d_obs,
+                            blocked() ? s.d_foff : s.d_off, s.d_len, s.d_order, U, N, M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
+                return HMMB_OK;
+            }));
         }
+        HMMB_LAUNCH("score_argmax", k_argmax_first, (unsigned)((U + 255) / 256), 256, 0, d_ll, U, W, d_arg);
+        if (argmax_out) HMMB_CUDA(cudaMemcpyAsync(argmax_out, d_arg, (size_t)U * sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
+        if (send_ll) HMMB_TRY(d2h_big(ll_out, d_ll, (size_t)U * W * sizeof(double), c.stream));
+        HMMB_CUDA(cudaStreamSynchronize(c.stream));
         return HMMB_OK;
-    }
-    int rc;
-    if (s.special4) {
-        const bool bidiag = upper_bidiagonal(A, W, N);
-        rc = bidiag ? launch_score_special<true>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan)
-                    : launch_score_special<false>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan);
-    } else if (s.ltr_ns) {
-        rc = s.ltr_ns == 16 ? launch_score_ltr<16>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan) : launch_score_ltr<8>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan);
-    } else {
-#define GEN(NPV)                                                                                         \
-    case NPV:                                                                                            \
-        rc = s.sym_bytes == 1 ? launch_score_generic<NPV, uint8_t>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan)         \
-                              : launch_score_generic<NPV, uint16_t>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan);       \
-        break;
-        switch (s.NP) {
-            GEN(4) GEN(8) GEN(16) GEN(32)
-            default: rc = HMMB_ERR_UNSUPPORTED;
-        }
-#undef GEN
-    }
-    HMMB_TRY(rc);
-    {
-        // precision guard: pairs marked NaN are recomputed in log space
-        int64_t warps = std::min<int64_t>((int64_t)c.sm_count * 16, U);
-        const int eg = (int)std::max<int64_t>(1, (warps + BW_WARPS - 1) / BW_WARPS);
-        if (s.blocked()) {
-            HMMB_LAUNCH("score_exact", (k_score_exact<uint16_t, true>), eg, BW_THREADS, 0, s.d_obs, s.d_foff, s.d_len, s.d_order, U, N, M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
+    };
+    if (!s.pend) {
+        if (s.layout == LAYOUT_N4) {
+            HMMB_TRY(launch_score_special(s, fam.bidiag, W, d_pi, d_A, d_Bt, d_ll, d_nan, 0, s.nblk));
+        } else if (s.layout == LAYOUT_LTR) {
+            HMMB_TRY(N == 16 ? launch_score_ltr<16>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan) : launch_score_ltr<8>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan));
         } else {
-            if (s.sym_bytes == 1)
-                HMMB_LAUNCH("score_exact", (k_score_exact<uint8_t, false>), eg, BW_THREADS, 0, s.d_obs, s.d_off, s.d_len, s.d_order, U, N, M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
-            else
-                HMMB_LAUNCH("score_exact", (k_score_exact<uint16_t, false>), eg, BW_THREADS, 0, s.d_obs, s.d_off, s.d_len, s.d_order, U, N, M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
+            HMMB_TRY(with_lanes(s, [&](auto np, auto sym) {
+                return launch_score_generic<decltype(np)::value, decltype(sym)>(s, W, d_pi, d_A, d_Bt, d_ll, d_nan);
+            }));
         }
+        // (k_score_exact returns at once when no pair was marked)
+        return finish(true, ll_out != nullptr);
     }
-    HMMB_LAUNCH("score_argmax", k_argmax_first, (unsigned)((U + 255) / 256), 256, 0, d_ll, U, W, d_arg);
-    if (argmax_out) HMMB_CUDA(cudaMemcpyAsync(argmax_out, d_arg, (size_t)U * sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
-    if (ll_out) HMMB_TRY(d2h_big(ll_out, d_ll, (size_t)U * W * sizeof(double), c.stream));
-    HMMB_CUDA(cudaStreamSynchronize(c.stream));
+    PendingPrepare &p = *s.pend;
+    int bdone = 0;
+    // a pageable result matrix cannot leave stage by stage (its copies would block the host between the
+    // stages): it goes through the bounce buffers after the last stage
+    const bool ll_pinned = ll_out && host_is_pinned(ll_out);
+    cudaEvent_t scored = event_get();
+    for (int j = 0; j < p.nstage; ++j) {
+        HMMB_CUDA(cudaStreamWaitEvent(c.stream, p.up->ev[p.ev_index[j]], 0));
+        HMMB_TRY(launch_repack_range(s, p.up->d_raw, p.idx_bytes, bdone, p.blk_end[j], s.d_bad));
+        HMMB_TRY(launch_score_special(s, fam.bidiag, W, d_pi, d_A, d_Bt, d_ll, d_nan, bdone, p.blk_end[j]));
+        if (ll_pinned) {
+            // scoring has a single "word", so block b holds utterances [32 b, 32 b + 32) of the (identity) order
+            const int64_t u0 = (int64_t)bdone * 32, u1 = std::min<int64_t>(U, (int64_t)p.blk_end[j] * 32);
+            HMMB_CUDA(cudaEventRecord(scored, c.stream));
+            HMMB_CUDA(cudaStreamWaitEvent(c.d2h_stream, scored, 0));
+            HMMB_CUDA(cudaMemcpyAsync(ll_out + u0 * W, d_ll + u0 * W, (size_t)(u1 - u0) * W * sizeof(double),
+                                      cudaMemcpyDeviceToHost, c.d2h_stream));
+        }
+        bdone = p.blk_end[j];
+    }
+    event_put(scored);
+    int32_t flags[2] = {0, 0};  // a pair marked by the precision guard, a codeword out of range
+    HMMB_CUDA(cudaMemcpyAsync(&flags[0], d_nan, sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
+    HMMB_CUDA(cudaMemcpyAsync(&flags[1], s.d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, c.stream));
+    HMMB_TRY(finish(false, ll_out && !ll_pinned));
+    HMMB_CUDA(cudaStreamSynchronize(c.d2h_stream));
+    s.pend.reset();
+    if (flags[1]) {
+        set_error("codeword out of range: some observation is >= M=%d (reference: IndexError)", M);
+        return HMMB_ERR_RANGE;
+    }
+    // rare: the precision guard marked pairs; recompute them in log space and send everything again
+    if (flags[0]) return finish(true, ll_out != nullptr);
     return HMMB_OK;
 }
 
@@ -2064,14 +2040,9 @@ static int launch_vit_backtrace_blocked(SeqSet &s, const int8_t *d_last, const v
 template <int NP, typename SymT>
 static int launch_viterbi_generic(SeqSet &s, const double *d_lpi, const double *d_lA, const double *d_lBt, double *d_score,
                                   int8_t *d_last, uint8_t *d_bp) {
-    Ctx &c = ctx();
-    constexpr int GPW = 32 / NP;
-    int64_t grid = (std::max<int64_t>(s.R, 1) + BW_WARPS * GPW - 1) / (BW_WARPS * GPW);
-    grid = std::min<int64_t>(grid, (int64_t)c.sm_count * 16);
-    const int64_t total_groups = grid * BW_WARPS * GPW;
-    const int64_t per_group = (s.R + total_groups - 1) / total_groups;
-    HMMB_LAUNCH("viterbi", (k_viterbiG<NP, SymT>), (unsigned)grid, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len, s.d_word,
-                s.d_order, s.d_foff, s.R, per_group, s.N, s.M, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp);
+    const LanesGrid g = lanes_grid(s.R, NP);
+    HMMB_LAUNCH("viterbi", (k_viterbiG<NP, SymT>), g.grid, BW_THREADS, 0, (const SymT *)s.d_obs, s.d_off, s.d_len, s.d_word,
+                s.d_order, s.d_foff, s.R, g.per_group, s.N, s.M, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp);
     return HMMB_OK;
 }
 
@@ -2085,13 +2056,10 @@ int hmmb_viterbi(const void *obs, int idx_bytes, int obs_on_device, const int64_
     }
     Ctx &c = ctx();
     SeqSet s;
-    struct Guard {
-        SeqSet &s; std::vector<void *> ptrs;
-        ~Guard() { s.release(); for (void *p : ptrs) dev_free(p); }
-    } guard{s, {}};
-    // the layouts and kernel families of hmmb_score: left-to-right models at N = 8 / 16 one utterance per thread
-    const bool ltr = ltr_shape_ok(N, M) && upper_bidiagonal(A, W, N);
-    HMMB_TRY(seqset_build(s, obs, idx_bytes, obs_on_device, offsets, model_of_utt, U, W, N, M, ltr ? LAYOUT_LTR : LAYOUT_AUTO));
+    CallGuard guard{s, {}};
+    // the layouts and kernel families of hmmb_score
+    const Family fam = pick_family(N, M, A, W);
+    HMMB_TRY(seqset_build(s, obs, idx_bytes, obs_on_device, offsets, model_of_utt, U, W, N, M, fam.layout()));
     if (U == 0) return HMMB_OK;
     const size_t nB = (size_t)W * N * M, nA = (size_t)W * N * N, nP = (size_t)W * N;
     double *tmp = nullptr, *d_lBt = nullptr, *d_lA = nullptr, *d_lpi = nullptr, *d_score = nullptr;
@@ -2111,40 +2079,31 @@ int hmmb_viterbi(const void *obs, int idx_bytes, int obs_on_device, const int64_
     int8_t *d_last = nullptr, *d_path = nullptr;
     void *d_bp = nullptr;
     if (want_path) {
-        const size_t row_bytes = s.ltr_ns == 16 ? 2 : 1;
+        const size_t row_bytes = s.layout == LAYOUT_LTR && N == 16 ? 2 : 1;
         const size_t bp_bytes = s.blocked() ? (size_t)s.spill_steps * 32 * row_bytes : (size_t)s.frames * N;
         HMMB_TRY(dev_alloc(&d_bp, bp_bytes)); guard.ptrs.push_back(d_bp);
         HMMB_TRY(dev_alloc_t(&d_last, (size_t)U)); guard.ptrs.push_back(d_last);
         HMMB_TRY(dev_alloc_t(&d_path, (size_t)s.frames)); guard.ptrs.push_back(d_path);
     }
-    int rc = HMMB_OK;
-    if (s.special4) {
-        rc = upper_bidiagonal(A, W, N) ? launch_viterbi_blocked<4, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)
-                                       : launch_viterbi_blocked<4, false>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp);
-        if (rc == HMMB_OK && want_path) rc = launch_vit_backtrace_blocked<4>(s, d_last, d_bp, d_path);
-    } else if (s.ltr_ns) {
-        rc = s.ltr_ns == 16 ? launch_viterbi_blocked<16, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)
-                            : launch_viterbi_blocked<8, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp);
-        if (rc == HMMB_OK && want_path)
-            rc = s.ltr_ns == 16 ? launch_vit_backtrace_blocked<16>(s, d_last, d_bp, d_path)
-                                : launch_vit_backtrace_blocked<8>(s, d_last, d_bp, d_path);
+    if (s.layout == LAYOUT_N4) {
+        HMMB_TRY((fam.bidiag ? launch_viterbi_blocked<4, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)
+                             : launch_viterbi_blocked<4, false>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)));
+        if (want_path) HMMB_TRY(launch_vit_backtrace_blocked<4>(s, d_last, d_bp, d_path));
+    } else if (s.layout == LAYOUT_LTR) {
+        HMMB_TRY((N == 16 ? launch_viterbi_blocked<16, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)
+                          : launch_viterbi_blocked<8, true>(s, d_lpi, d_lA, d_lBt, d_score, d_last, d_bp)));
+        if (want_path)
+            HMMB_TRY(N == 16 ? launch_vit_backtrace_blocked<16>(s, d_last, d_bp, d_path)
+                             : launch_vit_backtrace_blocked<8>(s, d_last, d_bp, d_path));
     } else {
         uint8_t *bp8 = (uint8_t *)d_bp;
-#define GEN(NPV)                                                                                                        \
-    case NPV:                                                                                                           \
-        rc = s.sym_bytes == 1 ? launch_viterbi_generic<NPV, uint8_t>(s, d_lpi, d_lA, d_lBt, d_score, d_last, bp8)       \
-                              : launch_viterbi_generic<NPV, uint16_t>(s, d_lpi, d_lA, d_lBt, d_score, d_last, bp8);     \
-        break;
-        switch (s.NP) {
-            GEN(4) GEN(8) GEN(16) GEN(32)
-            default: rc = HMMB_ERR_UNSUPPORTED;
-        }
-#undef GEN
-        if (rc == HMMB_OK && want_path)
+        HMMB_TRY(with_lanes(s, [&](auto np, auto sym) {
+            return launch_viterbi_generic<decltype(np)::value, decltype(sym)>(s, d_lpi, d_lA, d_lBt, d_score, d_last, bp8);
+        }));
+        if (want_path)
             HMMB_LAUNCH("viterbi_backtrace", k_vit_backtraceG, (unsigned)((U + VIT_THREADS - 1) / VIT_THREADS), VIT_THREADS, 0, U, N,
                         s.d_len, s.d_off, s.d_foff, d_last, bp8, d_path);
     }
-    HMMB_TRY(rc);
     if (score_out) HMMB_TRY(d2h_big(score_out, d_score, (size_t)U * sizeof(double), c.stream));
     if (want_path) HMMB_TRY(d2h_big(path_out, d_path, (size_t)s.frames, c.stream));
     HMMB_CUDA(cudaStreamSynchronize(c.stream));

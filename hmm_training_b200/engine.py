@@ -136,6 +136,21 @@ def lbg_fit(X, K: int = 256, max_iterations: int = 100, epsilon: float = 0.001,
 
 
 # ------------------------------------------------------------------------------- Baum-Welch
+def _codewords(obs, obs_dev_ptr: Optional[int], idx_bytes: Optional[int]):
+    """(pointer, on_device, idx_bytes, keepalive) of the codewords: an integer host array (signed arrays go as their
+    unsigned view once no entry is negative), or obs_dev_ptr to idx_bytes-wide codewords already in HBM."""
+    if obs_dev_ptr is not None:
+        return ctypes.c_void_p(obs_dev_ptr), 1, int(idx_bytes), None
+    obs = np.ascontiguousarray(obs)
+    if obs.dtype.kind not in "iu":
+        raise TypeError("codewords must be integers")
+    if obs.dtype.kind == "i":
+        if obs.size and int(obs.min()) < 0:
+            raise IndexError("negative codeword index")
+        obs = obs.view({1: np.uint8, 2: np.uint16, 4: np.uint32, 8: np.uint64}[obs.dtype.itemsize])
+    return ptr(obs), 0, obs.dtype.itemsize, obs
+
+
 class BaumWelch:
     """Device-resident batched Baum-Welch trainer (wraps hmmb_bw_*).
 
@@ -150,17 +165,7 @@ class BaumWelch:
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         word_of_seq = np.ascontiguousarray(word_of_seq, dtype=np.int32)
         self.R = len(offsets) - 1
-        if obs_dev_ptr is None:
-            obs = np.ascontiguousarray(obs)
-            if obs.dtype.kind not in "iu":
-                raise TypeError("codewords must be integers")
-            if obs.dtype.kind == "i":
-                if obs.size and int(obs.min()) < 0:
-                    raise IndexError("negative codeword index")
-                obs = obs.view({1: np.uint8, 2: np.uint16, 4: np.uint32, 8: np.uint64}[obs.dtype.itemsize])
-            op, on_dev, ib = ptr(obs), 0, obs.dtype.itemsize
-        else:
-            op, on_dev, ib = ctypes.c_void_p(obs_dev_ptr), 1, int(idx_bytes)
+        op, on_dev, ib, obs = _codewords(obs, obs_dev_ptr, idx_bytes)
         h = ctypes.c_void_p()
         # pipeline_upload: hmmb_bw_create_ex may return while pinned codewords are still crossing PCIe;
         # the first iterate() runs behind the upload, so the buffer is kept alive until close()
@@ -282,15 +287,7 @@ def score(obs, offsets, N: int, M: int, pi, A, B, obs_dev_ptr: Optional[int] = N
         raise ValueError("model parameter shapes do not match (W, N, M)")
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
     U = len(offsets) - 1
-    if obs_dev_ptr is None:
-        obs = np.ascontiguousarray(obs)
-        if obs.dtype.kind == "i":
-            if obs.size and int(obs.min()) < 0:
-                raise IndexError("negative codeword index")
-            obs = obs.view({1: np.uint8, 2: np.uint16, 4: np.uint32, 8: np.uint64}[obs.dtype.itemsize])
-        op, on_dev, ib = ptr(obs), 0, obs.dtype.itemsize
-    else:
-        op, on_dev, ib = ctypes.c_void_p(obs_dev_ptr), 1, int(idx_bytes)
+    op, on_dev, ib, obs = _codewords(obs, obs_dev_ptr, idx_bytes)
     if out_ll is not None:  # caller-provided [U, W] fp64 buffer (e.g. pinned memory: the D2H copy is then direct)
         if out_ll.shape != (U, W) or out_ll.dtype != np.float64 or not out_ll.flags.c_contiguous:
             raise ValueError(f"out_ll must be a C-contiguous float64 array of shape ({U}, {W})")
@@ -320,15 +317,7 @@ def viterbi(obs, offsets, model_of_utt, N: int, M: int, pi, A, B, want_path: boo
     model_of_utt = np.ascontiguousarray(model_of_utt, dtype=np.int32)
     if model_of_utt.shape != (U,):
         raise ValueError(f"model_of_utt must hold one model index per utterance ({U})")
-    if obs_dev_ptr is None:
-        obs = np.ascontiguousarray(obs)
-        if obs.dtype.kind == "i":
-            if obs.size and int(obs.min()) < 0:
-                raise IndexError("negative codeword index")
-            obs = obs.view({1: np.uint8, 2: np.uint16, 4: np.uint32, 8: np.uint64}[obs.dtype.itemsize])
-        op, on_dev, ib = ptr(obs), 0, obs.dtype.itemsize
-    else:
-        op, on_dev, ib = ctypes.c_void_p(obs_dev_ptr), 1, int(idx_bytes)
+    op, on_dev, ib, obs = _codewords(obs, obs_dev_ptr, idx_bytes)
     frames = int(offsets[-1] - offsets[0]) if U > 0 else 0
     score = np.empty(max(U, 1))
     path = np.empty(max(frames, 1), dtype=np.int8) if want_path else None

@@ -39,6 +39,22 @@ def test_no_cpu_fallback_without_gpu():
     assert "no CPU fallback" in str(ei.value)
 
 
+def test_non_integer_codewords_are_rejected_before_the_library():
+    """Host codewords must be integers in every entry point: the bits of a float array are not codewords (an all-zero
+    float64 array would otherwise be read as codeword 0).  The check runs before any device work."""
+    from hmm_training_b200 import engine
+    N, M, W = 4, 8, 2
+    pi, A, B = (np.tile(x, (W,) + (1,) * x.ndim) for x in engine.default_init(N, M))
+    offsets = np.array([0, 3, 5], np.int64)
+    for obs in (np.zeros(5), np.zeros(5, np.float32), np.zeros(5, bool)):
+        with pytest.raises(TypeError):
+            engine.score(obs, offsets, N, M, pi, A, B)
+        with pytest.raises(TypeError):
+            engine.viterbi(obs, offsets, np.zeros(2, np.int32), N, M, pi, A, B)
+        with pytest.raises(TypeError):
+            engine.BaumWelch(obs, offsets, np.zeros(2, np.int32), W, N, M)
+
+
 def test_product_package_never_imports_oracle():
     pkg = os.path.join(ROOT, "hmm_training_b200")
     for dirpath, _, files in os.walk(pkg):

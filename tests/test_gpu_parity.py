@@ -426,6 +426,63 @@ def test_scoring_left_to_right_kernels(N, M, kind, monkeypatch):
     assert np.array_equal(arg[clear], argg[clear])
 
 
+@pytest.mark.parametrize("N,M,dense_family", [(4, 64, "n4_dense"), (8, 40, "generic")])
+def test_dense_a_switch_in_trainer_scorer_and_decoder(N, M, dense_family, monkeypatch):
+    """HMMB_FORCE_DENSE_A=1 treats an upper-bidiagonal A as dense in all three entry points: N = 4 then trains, scores
+    and decodes on the dense N = 4 kernels, N = 8 on the lanes-per-state kernels.  Both runs must match the oracle.
+    At N = 4 Viterbi only adds and compares, and the terms the bidiagonal kernel skips are -inf, so its results must
+    equal the default run's bit for bit.  Scores and trained models come out of different floating-point code in the two
+    kernel families and differ in the last bits, so they are held to each other at the parity tolerance."""
+    from test_gpu_viterbi import check_against_oracle
+
+    rng = np.random.default_rng(N * 31 + M)
+    W = 3
+    corpus = [synthetic.clustered_sequences(rng, 40, N=N, M=M, tmin=1, tmax=70, shift=5 * w, spread=max(2, M // (2 * N)))
+              for w in range(W)]
+    obs, offsets, wos = synthetic.pack_corpus(corpus, M)
+    seqs = [s for word in corpus for s in word]
+    pi0, A0, B0 = _ltr_init(rng, W, N, M, "random")
+    iters_max = 4
+    runs = {}
+    for dense in (False, True):
+        if dense:
+            monkeypatch.setenv("HMMB_FORCE_DENSE_A", "1")
+        else:
+            monkeypatch.delenv("HMMB_FORCE_DENSE_A", raising=False)
+        with engine.BaumWelch(obs, offsets, wos, W, N, M) as bw:
+            bw.set_params(pi0, A0, B0)
+            family = bw.kernel_family()
+            bw.iterate(iters_max, 1e-6, iters_max)
+            trained = bw.params() + bw.history(iters_max)
+        runs[dense] = (family, trained, engine.score(obs, offsets, N, M, pi0, A0, B0),
+                       engine.viterbi(obs, offsets, wos, N, M, pi0, A0, B0))
+    assert runs[False][0] == ("n4_left_to_right" if N == 4 else "left_to_right")
+    family, (pi, A, B, hist, iters), (ll, arg), (vscore, vpath) = runs[True]
+    assert family == dense_family
+    for w in range(W):
+        Ao, Bo, pio, h, it = O.hmm_training(corpus[w], N=N, M=M, max_iterations=iters_max,
+                                            init=(pi0[w], A0[w], B0[w]), return_history=True)
+        assert it == iters[w]
+        assert_close(hist[w, :it], h, f"dense N{N} w{w} ll")
+        assert_close(A[w], Ao, f"dense N{N} w{w} A")
+        assert_close(B[w], Bo, f"dense N{N} w{w} B")
+        assert_close(pi[w], pio, f"dense N{N} w{w} pi")
+        assert_same_support(A[w], Ao); assert_same_support(pi[w], pio)
+        assert np.array_equal(floored_set(B[w], M), floored_set(Bo, M))
+    ref = O.score_batch(seqs, [(A0[w], B0[w], pi0[w]) for w in range(W)])
+    assert_close(ll, ref, f"dense N{N} score")
+    assert np.array_equal(np.isneginf(ll), np.isneginf(ref))
+    assert np.array_equal(arg, O.argmax_first(ll))
+    check_against_oracle(seqs, wos, pi0, A0, B0, vscore, vpath, offsets, f"dense N{N} viterbi")
+    if N == 4:
+        (_, (ll_b, _), (vscore_b, vpath_b)) = runs[False][1:]
+        assert np.array_equal(vscore, vscore_b) and np.array_equal(vpath, vpath_b)
+        assert_close(ll, ll_b, "dense vs bidiagonal N = 4 scores")
+        for x, y, what in zip(runs[True][1], runs[False][1], ("pi", "A", "B", "ll history")):
+            assert_close(x[np.isfinite(y)], y[np.isfinite(y)], f"dense vs bidiagonal N = 4 kernels: trained {what}")
+        assert np.array_equal(runs[True][1][4], runs[False][1][4])
+
+
 def _tiny_models(rng, W, N, M):
     """Left-to-right models whose emission rows hold denormal / 1e-300-range / zero entries:
     what saved reference models look like after safe_exp underflow (hmm_training.py:524-526)."""
