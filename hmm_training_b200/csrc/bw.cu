@@ -213,13 +213,13 @@ __global__ void k_argmax_first(const double *__restrict__ ll, int64_t U, int W, 
     out[u] = bi;
 }
 
-// Exact recomputation of the (utterance, model) pairs the precision guard marked with NaN.
+// Exact recomputation of the (utterance, model) pairs the precision guard marked with NaN; n_pairs counts them.
 template <typename SymT, bool BLOCKED>
 __global__ void __launch_bounds__(BW_THREADS)
 k_score_exact(const void *__restrict__ obs, const int64_t *__restrict__ base_sorted, const int32_t *__restrict__ len_sorted,
               const int32_t *__restrict__ order, int64_t U, int N, int M, int W, const double *__restrict__ pi,
               const double *__restrict__ A, const double *__restrict__ Bt, double *__restrict__ ll_out,
-              const int32_t *__restrict__ any_nan) {
+              const int32_t *__restrict__ any_nan, int64_t *__restrict__ n_pairs) {
     if (*any_nan == 0) return;  // the scorers marked nothing: no scan of the [U, W] matrix
     const int lane = threadIdx.x & 31;
     const int64_t gw = (int64_t)blockIdx.x * BW_WARPS + (threadIdx.x >> 5);
@@ -242,7 +242,10 @@ k_score_exact(const void *__restrict__ obs, const int64_t *__restrict__ base_sor
                     LinObs<SymT> o{reinterpret_cast<const SymT *>(obs) + base_sorted[i]};
                     logP = exact_forward(T, N, lane, o, piw, Aw, Btw, (double *)nullptr);
                 }
-                if (lane == 0) row[w] = logP;
+                if (lane == 0) {
+                    row[w] = logP;
+                    atomicAdd(reinterpret_cast<unsigned long long *>(n_pairs), 1ULL);
+                }
                 __syncwarp();
             }
         }
@@ -1904,15 +1907,21 @@ static int launch_score_ltr(SeqSet &s, int W, const double *d_pi, const double *
 int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets, int64_t U, int W, int N, int M,
                const double *pi, const double *A, const double *B, double *ll_out, int32_t *argmax_out) {
     HMMB_TRY(require_init());
-    if (!pi || !A || !B || W <= 0 || W > 65535) { set_error("hmmb_score: bad arguments (W=%d)", W); return HMMB_ERR_ARG; }
     Ctx &c = ctx();
+    // the flag the scorers set when the precision guard marked a pair, and the count of pairs k_score_exact recomputed
+    // (hmmb_score_diagnostics): one slot of the context, cleared together before anything can fail, so that the count
+    // always describes this call
+    if (!c.score_slot) HMMB_TRY(dev_alloc_t(&c.score_slot, 4));
+    HMMB_CUDA(cudaMemsetAsync(c.score_slot, 0, 4 * sizeof(int32_t), c.stream));
+    if (!pi || !A || !B || W <= 0 || W > 65535) { set_error("hmmb_score: bad arguments (W=%d)", W); return HMMB_ERR_ARG; }
     SeqSet s;
     CallGuard guard{s, {}};
     const Family fam = pick_family(N, M, A, W);
     const size_t nB = (size_t)W * N * M, nA = (size_t)W * N * N, nP = (size_t)W * N;
     double *tmp = nullptr, *d_pi = nullptr, *d_A = nullptr, *d_Bt = nullptr, *d_ll = nullptr;
     int32_t *d_arg = nullptr;
-    int32_t *d_nan = nullptr;  // set by the scorers when the precision guard marked a pair
+    int32_t *d_nan = c.score_slot;
+    int64_t *d_npairs = reinterpret_cast<int64_t *>(c.score_slot + 2);
     bool models_up = false;
     // model parameters -> device.  In the pipelined scorer this runs inside seqset_build, between the first chunks and the rest
     // of the codeword upload and on the same DMA queue (see hmmb_bw_create_ex).
@@ -1925,8 +1934,6 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
         HMMB_TRY(dev_alloc_t(&d_Bt, nB)); guard.ptrs.push_back(d_Bt);
         HMMB_TRY(dev_alloc_t(&d_ll, (size_t)U * W)); guard.ptrs.push_back(d_ll);
         HMMB_TRY(dev_alloc_t(&d_arg, (size_t)U)); guard.ptrs.push_back(d_arg);
-        HMMB_TRY(dev_alloc_t(&d_nan, 1)); guard.ptrs.push_back(d_nan);
-        HMMB_CUDA(cudaMemsetAsync(d_nan, 0, sizeof(int32_t), c.stream));
         HMMB_TRY(h2d_small(tmp, B, nB * sizeof(double)));
         HMMB_TRY(h2d_small(tmp + nB, A, nA * sizeof(double)));
         HMMB_TRY(h2d_small(tmp + nB + nA, pi, nP * sizeof(double)));
@@ -1952,7 +1959,8 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
             const int eg = (int)std::max<int64_t>(1, (warps + BW_WARPS - 1) / BW_WARPS);
             HMMB_TRY(with_codewords(s, [&](auto sym, auto blocked) -> int {
                 HMMB_LAUNCH("score_exact", (k_score_exact<decltype(sym), decltype(blocked)::value>), eg, BW_THREADS, 0, s.d_obs,
-                            blocked() ? s.d_foff : s.d_off, s.d_len, s.d_order, U, N, M, W, d_pi, d_A, d_Bt, d_ll, d_nan);
+                            blocked() ? s.d_foff : s.d_off, s.d_len, s.d_order, U, N, M, W, d_pi, d_A, d_Bt, d_ll, d_nan,
+                            d_npairs);
                 return HMMB_OK;
             }));
         }
@@ -2008,6 +2016,19 @@ int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t 
     }
     // rare: the precision guard marked pairs; recompute them in log space and send everything again
     if (flags[0]) return finish(true, ll_out != nullptr);
+    return HMMB_OK;
+}
+
+int hmmb_score_diagnostics(int64_t *exact_pairs) {
+    HMMB_TRY(require_init());
+    if (!exact_pairs) { set_error("hmmb_score_diagnostics: null argument"); return HMMB_ERR_ARG; }
+    Ctx &c = ctx();
+    int64_t n = 0;
+    if (c.score_slot) {
+        HMMB_CUDA(cudaMemcpyAsync(&n, c.score_slot + 2, sizeof(int64_t), cudaMemcpyDeviceToHost, c.stream));
+        HMMB_CUDA(cudaStreamSynchronize(c.stream));
+    }
+    *exact_pairs = n;
     return HMMB_OK;
 }
 

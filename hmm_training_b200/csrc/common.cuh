@@ -76,6 +76,9 @@ struct Ctx {
     // two pinned bounce buffers for large copies from / to PAGEABLE host memory (h2d_big / d2h_big)
     void *bounce[2] = {nullptr, nullptr};
     cudaEvent_t bounce_ev[2] = {nullptr, nullptr};
+    // device slot of hmmb_score, cleared by one memset per call: the precision guard's flag (int32 at [0]) and the
+    // count of pairs k_score_exact recomputed (int64 at [2]), read only by hmmb_score_diagnostics
+    int32_t *score_slot = nullptr;
 };
 
 Ctx &ctx();

@@ -329,6 +329,7 @@ int hmmb_shutdown(void) {
     dev_release_cache();
     for (auto &kv : c.live_blocks) cudaFree(kv.first);
     c.live_blocks.clear();
+    c.score_slot = nullptr;  // was one of the live blocks
     if (c.stage) cudaFreeHost(c.stage);
     c.stage = nullptr;
     c.stage_bytes = 0;

@@ -299,6 +299,14 @@ def score(obs, offsets, N: int, M: int, pi, A, B, obs_dev_ptr: Optional[int] = N
     return ll, arg[:U]
 
 
+def score_diagnostics() -> int:
+    """(utterance, model) pairs the last score() call recomputed with the exact log-space kernel
+    (hmmb_score_diagnostics)."""
+    n = ctypes.c_int64(0)
+    check(_lib.load().hmmb_score_diagnostics(ctypes.byref(n)))
+    return n.value
+
+
 def viterbi(obs, offsets, model_of_utt, N: int, M: int, pi, A, B, want_path: bool = True,
             obs_dev_ptr: Optional[int] = None, idx_bytes: Optional[int] = None):
     """Most likely state path of every utterance under its own model (hmmb_viterbi; an extension, the reference

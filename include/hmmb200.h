@@ -215,6 +215,12 @@ int hmmb_bw_fit(const void *obs, int idx_bytes, const int64_t *offsets, const in
 int hmmb_score(const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets, int64_t U,
                int W, int N, int M, const double *pi, const double *A, const double *B,
                double *ll_out, int32_t *argmax_out);
+/* precision-guard counter of the last hmmb_score call in the process (0 after a call that failed its argument
+ * checks): the (utterance, model) pairs whose score was
+ * recomputed by the exact log-space kernel because the linear forward pass could not hold it to the reference's
+ * precision (denormal or zero emissions on the only live path).  Zero on ordinary data; the scores meet the reference
+ * at 1e-9 either way.  hmmb_score itself does not wait for this count: it is read only here.                    */
+int hmmb_score_diagnostics(int64_t *exact_pairs);
 
 /* ------------------------------------------------------------------ Viterbi decoding
  * An extension: the reference has no Viterbi.  The most likely state path of every utterance under its own model

@@ -50,3 +50,49 @@ def floored_set(B, M):
     ~[1/(1+M*1e-20), 1] of 1e-20 — anything in [0.5e-20, 1.5e-20] qualifies."""
     B = np.asarray(B)
     return (B > 0.5e-20) & (B < 1.5e-20)
+
+
+def run_virtual_ranks(shards, pack, wos, W, N, M, init, iters):
+    """G "virtual ranks" on one device in lock step: rank r trains on the sequences shards[r] (pack(indices) ->
+    (obs, offsets)) with an all-reduce hook that the emulation serves.  Pass k runs every rank and records each rank's
+    buffer of hook call k; the hook calls before it are served the sums recorded so far, so that each rank sees the
+    reduced buffers up to that call and produces its next one from correct parameters.  A pass whose hook calls were all
+    served is the G-rank run.  Returns (pi, A, B, history, iterations, thin states) of that run, every rank's
+    diagnostics() in it, and the number of hook calls per rank."""
+    import ctypes
+
+    from hmm_training_b200 import engine
+    rt = ctypes.CDLL("libcudart.so.12")
+    rt.cudaMemcpy.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int]
+    rt.cudaDeviceSynchronize.argtypes = []
+    G = len(shards)
+    sums = []
+    for _ in range(64):
+        recorded, diags = [], []
+        for r in range(G):
+            mine, k = [], [0]
+
+            def hook(ptr, n, mine=mine, k=k):
+                assert rt.cudaDeviceSynchronize() == 0
+                if k[0] < len(sums):
+                    assert n == len(sums[k[0]])
+                    assert rt.cudaMemcpy(ptr, sums[k[0]].ctypes.data, n * 8, 1) == 0
+                else:
+                    buf = np.empty(n)
+                    assert rt.cudaMemcpy(buf.ctypes.data, ptr, n * 8, 2) == 0
+                    mine.append(buf)
+                k[0] += 1
+
+            obs, off = pack(shards[r])
+            with engine.BaumWelch(obs, off, wos[shards[r]], W, N, M) as bw:
+                bw.set_params(*init)
+                bw.set_dist(r, G, hook)
+                bw.iterate(iters, -1.0, iters)
+                got = bw.params() + bw.history(iters) + (bw.thin_states(),)
+                diags.append(bw.diagnostics())
+            recorded.append(mine)
+        if not recorded[0]:
+            return got, diags, len(sums)
+        assert all(len(m) >= 1 for m in recorded)
+        sums.append(np.sum([m[0] for m in recorded], axis=0))
+    raise AssertionError("the hook calls did not settle")

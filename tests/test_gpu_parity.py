@@ -812,3 +812,4 @@ def test_backward_mass_recovering_through_tiny_state(kernel_family):
     assert_same_support(A[0], Ao); assert_same_support(pi[0], pio)
     assert np.array_equal(floored_set(B[0], M), floored_set(Bo, M))
     print(f"exact passes, backward hand-overs = {diag}")
+    assert diag[1] > 0  # both kernel families hand these sequences over from the backward pass

@@ -8,12 +8,10 @@ with the more ordinary way to get there: tail states of a left-to-right model th
 posterior decays super-exponentially from one EM iteration to the next.  The M-step flags such a state
 (denominator below 2^-200), and from then on its rows come from log-space sums (hmm_device.cuh, "thin-state rescue").
 """
-import ctypes
-
 import numpy as np
 import pytest
 
-from helpers import assert_close, assert_same_support, floored_set
+from helpers import assert_close, assert_same_support, floored_set, run_virtual_ranks
 from oracle import hmm_oracle as O
 from test_properties import _pack, _random_corpus, _random_model
 
@@ -119,42 +117,9 @@ def test_thin_states_over_virtual_ranks():
     wos = np.array(wos, dtype=np.int32)
     want = _fit(engine, seqs, wos, W, N, M, init, iters)
     _check(want, seqs, wos, W, N, M, init, iters)
-    rt = ctypes.CDLL("libcudart.so.12")
-    rt.cudaMemcpy.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int]
-    rt.cudaDeviceSynchronize.argtypes = []
     shards = [dist.shard_sequences_round_robin(wos, r, G) for r in range(G)]
-    # Lock-step emulation: both ranks advance hook call by hook call.  Pass 1 of a call index records every rank's
-    # buffer; pass 2 replays the run and injects the sums recorded so far, so that each rank sees the reduced
-    # buffers up to that call and produces its next one from correct parameters.
-    sums = []
-    for upto in range(1, 64):
-        recorded = []
-        for r in range(G):
-            mine, k = [], [0]
-
-            def hook(ptr, n, mine=mine, k=k):
-                assert rt.cudaDeviceSynchronize() == 0
-                if k[0] < len(sums):
-                    assert n == len(sums[k[0]])
-                    assert rt.cudaMemcpy(ptr, sums[k[0]].ctypes.data, n * 8, 1) == 0
-                else:
-                    buf = np.empty(n)
-                    assert rt.cudaMemcpy(buf.ctypes.data, ptr, n * 8, 2) == 0
-                    mine.append(buf)
-                k[0] += 1
-
-            obs, off = _pack([seqs[i] for i in shards[r]])
-            with engine.BaumWelch(obs, off, wos[shards[r]], W, N, M) as bw:
-                bw.set_params(*init)
-                bw.set_dist(r, G, hook)
-                bw.iterate(iters, -1.0, iters)
-                got = bw.params() + bw.history(iters) + (bw.thin_states(),)
-            recorded.append(mine)
-        if not recorded[0]:
-            break  # every hook call of the run was served from `sums`: `got` is the G-rank result
-        assert all(len(m) >= 1 for m in recorded)
-        sums.append(np.sum([m[0] for m in recorded], axis=0))
-    assert len(sums) > iters  # at least one iteration was repeated
+    got, _, calls = run_virtual_ranks(shards, lambda idx: _pack([seqs[i] for i in idx]), wos, W, N, M, init, iters)
+    assert calls > iters  # at least one iteration was repeated
     for x, y, name in zip(got[:5], want[:5], ("pi", "A", "B", "statistic", "iterations")):
         assert_close(x, y, f"{G} virtual ranks: {name}", rtol=1e-9, atol=1e-12)
     assert got[5] == want[5] >= 1
