@@ -398,13 +398,15 @@ static bool upper_bidiagonal(const double *A, int W, int N) {
 struct Family {
     Layout blocked;  // the blocked layout whose kernels hold this (N, M), LAYOUT_LANES if none does
     bool bidiag;     // every A is upper-bidiagonal: the 7-term N = 4 kernels; LAYOUT_LTR requires it
+    bool full_spill; // N = 4 E-step: spill every alpha-hat row instead of rebuilding the plain odd ones (reference arm)
     Layout layout() const { return blocked == LAYOUT_LTR && !bidiag ? LAYOUT_LANES : blocked; }
 };
 
 // The one place that reads the switches routing models to the other kernel family: HMMB_FORCE_GENERIC (every shape to
-// the lanes-per-state kernels), HMMB_NO_LTR (N = 8 / 16 to them) and HMMB_FORCE_DENSE_A (A treated as dense).
+// the lanes-per-state kernels), HMMB_NO_LTR (N = 8 / 16 to them) and HMMB_FORCE_DENSE_A (A treated as dense); also
+// HMMB_FULL_SPILL (the N = 4 E-step writes and reads every alpha-hat row).
 static Family pick_family(int N, int M, const double *A, int W) {
-    Family f{LAYOUT_LANES, A && !getenv("HMMB_FORCE_DENSE_A") && upper_bidiagonal(A, W, N)};
+    Family f{LAYOUT_LANES, A && !getenv("HMMB_FORCE_DENSE_A") && upper_bidiagonal(A, W, N), getenv("HMMB_FULL_SPILL") != nullptr};
     if (getenv("HMMB_FORCE_GENERIC")) return f;
     if (N == 4 && M <= BW4_MAX_M) {
         f.blocked = LAYOUT_N4;
@@ -896,6 +898,8 @@ struct hmmb_bw {
     bool has_ltr = false;         // sl was built
     bool use_ltr = false;         // every word's A is upper-bidiagonal (checked in set_params): run the sl kernels
     uint8_t *d_allfull = nullptr; // per sequence: every spilled alpha-hat > 0 (written by the forward kernels)
+    uint32_t *d_oddmask = nullptr; // N = 4: per (block, odd step) the lanes that wrote that alpha-hat row (k_bw_fwd4)
+    bool full_spill = false;      // N = 4: every alpha-hat row written and read (HMMB_FULL_SPILL, see pick_family)
     bool check_bad = false;       // pipelined prepare: the codeword-range flag has not been read back yet
     std::unique_ptr<PendingPrepare> pend_release;  // consumed by the E-step; freed after the next stream sync
     void *d_raw = nullptr;        // raw codewords uploaded once when both layouts are built
@@ -953,6 +957,8 @@ struct hmmb_bw {
 
 // alpha-hat spill of the N = 4 kernels (behind its front padding, see bw_finish_create)
 static double2 *spill4(hmmb_bw *h) { return reinterpret_cast<double2 *>(h->d_spill) + (size_t)BWD4_SPILL_PAD * 64; }
+// odd-row lane masks of the N = 4 kernels, one word per spill row (even rows unused), with the same front padding
+static unsigned *oddmask4(hmmb_bw *h) { return h->d_oddmask + BWD4_SPILL_PAD; }
 
 static void bw_drop_pieces(hmmb_bw *h) {
     for (auto &e : h->bt_ready) {
@@ -971,6 +977,7 @@ static void bw_release(hmmb_bw *h) {
     h->s.release();
     h->sl.release();
     dev_free(h->d_allfull);
+    dev_free(h->d_oddmask);
     dev_free(h->d_raw);
     dev_free(h->d_pi); dev_free(h->d_A); dev_free(h->d_Bt); dev_free(h->d_spill); dev_free(h->d_llseq);
     dev_free(h->d_accum); dev_free(h->d_partials); dev_free(h->d_prev); dev_free(h->d_hist); dev_free(h->d_active);
@@ -1044,6 +1051,7 @@ static int bw_finish_create(hmmb_bw *h, int64_t R) {
             TRYF(h2d_small(h->d_cta_begin_fine, s.cta_begin_fine.data(), (W + 1) * sizeof(int32_t)));
         }
         TRYF(dev_alloc_t(&h->d_allfull, (size_t)std::max<int64_t>(R, 1)));
+        TRYF(dev_alloc_t(&h->d_oddmask, (size_t)(std::max<int64_t>(s.spill_steps, 1) + BWD4_SPILL_PAD)));
         TRYF(h2d_small(h->d_cta_begin, s.cta_begin.data(), (W + 1) * sizeof(int32_t)));
     } else {
         spill_bytes = (size_t)std::max<int64_t>(s.frames, 1) * N * sizeof(double);
@@ -1326,7 +1334,9 @@ static int bw_set_params_impl(hmmb_bw *h, const double *pi0, const double *A0, c
     }
     // upper-bidiagonal A (the reference's left-to-right default) selects the 7-term N = 4 kernels and the
     // left-to-right kernels for N = 8 / 16
-    h->bidiag = pick_family(N, M, A0, W).bidiag;
+    const Family fam = pick_family(N, M, A0, W);
+    h->bidiag = fam.bidiag;
+    h->full_spill = fam.full_spill;
     h->use_ltr = h->has_ltr && h->bidiag;
     if (h->ltr_only && !h->use_ltr) HMMB_TRY(bw_build_generic_lazily(h));
     HMMB_LAUNCH("bw_load", k_load_clamped, (unsigned)std::min<size_t>((nA + 255) / 256, 1024), 256, 0, tmp + nB, (int64_t)nA, h->d_A);
@@ -1490,13 +1500,14 @@ static int launch_special_estep(hmmb_bw *h) {
     auto fwd = [&](const CtaWork *list, int c0, int c1) -> int {
         HMMB_LAUNCH("bw_forward", k_bw_fwd4<BIDIAG>, (c1 - c0) * FWD4_SPLIT, BW_THREADS, smem_f, list + c0, s.d_blks,
                     (const uint4 *)s.d_obs, s.d_len, h->d_pi, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur,
-                    h->d_flag, h->d_allfull, FWD4_SPLIT, SYM_MASK);
+                    h->d_flag, h->d_allfull, FWD4_SPLIT, SYM_MASK, oddmask4(h), h->full_spill);
         return HMMB_OK;
     };
     auto bwd = [&](const CtaWork *list, int c0, int c1) -> int {
         HMMB_LAUNCH("bw_backward", (k_bw_bwd4<BIDIAG, MT, REP>), c1 - c0, bwd_threads, smem_b, list + c0, s.d_blks,
                     (const uint4 *)s.d_obs, s.d_len, h->d_A, h->d_Bt, h->M, spill4(h), h->d_llseq, h->act_cur, h->d_bzero,
-                    h->d_allfull, h->d_partials + (size_t)c0 * h->pstride, h->pstride, h->d_flag, h->d_newflags);
+                    h->d_allfull, h->d_partials + (size_t)c0 * h->pstride, h->pstride, h->d_flag, h->d_newflags,
+                    oddmask4(h), h->full_spill);
         return HMMB_OK;
     };
     if (s.pend) {

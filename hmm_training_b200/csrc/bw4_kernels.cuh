@@ -9,9 +9,11 @@
 //                     the emission-count update is computed once here instead of with
 //                     MATCH.ANY every step (measured 1 MATCH per ~55 cycles per SM on B200).
 //   k_bw_fwd4         scaled forward pass, alpha-hat spilled to HBM [block][t][half][lane] as
-//                     coalesced 16-byte streaming stores, B^T of the CTA's word in shared memory.
+//                     coalesced 16-byte streaming stores (even steps, and odd steps that were not
+//                     plain: see fwd4_plain), B^T of the CTA's word in shared memory.
 //   k_bw_bwd4         backward pass fused with the gamma / xi / emission-count accumulation
-//                     (beta never leaves registers); counts go to warp-private shared-memory
+//                     (beta never leaves registers; the plain odd-step alpha-hat rows rebuilt from
+//                     the even ones); counts go to warp-private shared-memory
 //                     copies with plain read-modify-writes in precomputed rank order (no
 //                     atomics, deterministic); one partial per CTA.
 //
@@ -183,6 +185,41 @@ __device__ __forceinline__ Masks4 make_masks4(const double *__restrict__ Aw, con
 // smallest denormal if bit `j` of `m` is set, else +0.0 (integer pipe)
 __device__ __forceinline__ double tiny_if(unsigned m, int j) { return __hiloint2double(0, (int)((m >> j) & 1u)); }
 
+// One PLAIN forward step: every state alive and t > 0, the common case of fwd4_run.  The smallest denormal is the
+// addend of every chain, n = A^T al + tiny and at = b(o_t) .* n + tiny.  k_bw_bwd4 rebuilds the odd-step alpha-hat of
+// such steps from the even-step row with this same function (fwd4_rebuild), so it is written with explicit fma() only:
+// both kernels must get the same bits, not the same value to rounding.
+template <bool BIDIAG>
+__device__ __forceinline__ void fwd4_plain(const double *a, double al0, double al1, double al2, double al3, double2 b01,
+                                           double2 b23, double tiny, double &n0, double &n1, double &n2, double &n3,
+                                           double &at0, double &at1, double &at2, double &at3) {
+    if (BIDIAG) {
+        n0 = fma(al0, a[0], tiny);
+        n1 = fma(al1, a[1], fma(al0, a[4], tiny));
+        n2 = fma(al2, a[2], fma(al1, a[5], tiny));
+        n3 = fma(al3, a[3], fma(al2, a[6], tiny));
+    } else {
+        n0 = fma(al3, a[12], fma(al2, a[8], fma(al1, a[4], fma(al0, a[0], tiny))));
+        n1 = fma(al3, a[13], fma(al2, a[9], fma(al1, a[5], fma(al0, a[1], tiny))));
+        n2 = fma(al3, a[14], fma(al2, a[10], fma(al1, a[6], fma(al0, a[2], tiny))));
+        n3 = fma(al3, a[15], fma(al2, a[11], fma(al1, a[7], fma(al0, a[3], tiny))));
+    }
+    at0 = fma(n0, b01.x, tiny); at1 = fma(n1, b01.y, tiny);
+    at2 = fma(n2, b23.x, tiny); at3 = fma(n3, b23.y, tiny);
+}
+// alpha-hat_t of a plain step from alpha-hat_{t-1} (in place): fwd4_plain, then the rescale of fwd4_run, which is
+// the step's sum, pow2_rescale of it and at * sc.  Each product is rounded on its own (__dmul_rn), as the value
+// fwd4_run spills is, so that no later sum can take it into an FMA.
+template <bool BIDIAG>
+__device__ __forceinline__ void fwd4_rebuild(const double *a, double2 &x01, double2 &x23, double2 b01, double2 b23,
+                                             double tiny) {
+    double n0, n1, n2, n3, at0, at1, at2, at3;
+    fwd4_plain<BIDIAG>(a, x01.x, x01.y, x23.x, x23.y, b01, b23, tiny, n0, n1, n2, n3, at0, at1, at2, at3);
+    const double sc = pow2_rescale_noacc((at0 + at1) + (at2 + at3));
+    x01 = make_double2(__dmul_rn(at0, sc), __dmul_rn(at1, sc));
+    x23 = make_double2(__dmul_rn(at2, sc), __dmul_rn(at3, sc));
+}
+
 // One sequence per lane.  p[j] = pi[j]; B^T of the word in shared memory as two arrays of
 // double2, sB01[sym] = (b_0, b_1)(sym) and sB23[sym] = (b_2, b_3)(sym) — 16-byte rows give a
 // random gather 8 distinct bank slots instead of 4 with 32-byte rows; sBmax[sym] =
@@ -208,6 +245,10 @@ __device__ __forceinline__ double tiny_if(unsigned m, int j) { return __hiloint2
 //     issue-bound scorer when no utterance exceeds SCORE4_SCALAR_BOUND_MAX_T), trips after a few thousand
 //     frames with peaked emissions.
 //
+// SPILL: alpha-hat_t goes to sp[t * 64] for every even t, and for an odd t only if the step was not plain (see
+// fwd4_plain: an alive set still growing or cut by a zero of B, or the exponent-split branch), or if `full` asks for
+// every row.  k_bw_bwd4 rebuilds the other odd rows; oddmask[t] (odd t < tmax) records which lanes wrote row t.
+//
 // REP = 8: B^T is stored eight times, entry (sym, r) at index sym * 8 + r, and a lane reads replica r = lane & 7:
 // the eight lanes of a quarter-warp then always hit eight different 16-byte bank slots, so the gather is free of
 // bank conflicts whatever the codewords are (used by the scorer, whose only shared-memory traffic it is).
@@ -218,7 +259,8 @@ __device__ __forceinline__ double fwd4_run(int T, int tmax, const uint4 *__restr
                                            const unsigned char *__restrict__ sBmask, const double *a,
                                            const double (&p)[4], double rmax, const Masks4 &mk,
                                            double2 *__restrict__ sp, bool &allfull, int slot = 0,
-                                           unsigned symmask = SYM_MASK) {
+                                           unsigned symmask = SYM_MASK, unsigned *__restrict__ oddmask = nullptr,
+                                           bool full = false) {
     using S16 = Sym<uint16_t>;
     double al0 = 0.0, al1 = 0.0, al2 = 0.0, al3 = 0.0;
     double e0 = 0.0, e1 = 0.0, e2 = 0.0, e3 = 0.0;  // error bounds, units of 2^-1000: per state (VECB) or e0 = their sum
@@ -237,26 +279,16 @@ __device__ __forceinline__ double fwd4_run(int T, int tmax, const uint4 *__restr
         for (int s = 0; s < SPC4; ++s) {
             const int t = c * SPC4 + s;
             const unsigned sym = S16::pop_front(w) & symmask;
+            bool plain = false, wrote = false;
             if (t < T && !stop) {
                 const double2 b01 = sB01[sym * REP + slot], b23 = sB23[sym * REP + slot];
                 const unsigned r = (t == 0) ? mk.pmask : lut4(mk.lutF, m);  // reachable before emission
                 m = r & (unsigned)sBmask[sym];
                 double n0, n1, n2, n3, at0, at1, at2, at3;
-                if (m == 0xFu && t > 0) {
+                plain = m == 0xFu && t > 0;
+                if (plain) {
                     // ---- every state alive (the usual case; the first step takes the masked branch)
-                    if (BIDIAG) {
-                        n0 = fma(al0, a[0], tiny);
-                        n1 = fma(al1, a[1], fma(al0, a[4], tiny));
-                        n2 = fma(al2, a[2], fma(al1, a[5], tiny));
-                        n3 = fma(al3, a[3], fma(al2, a[6], tiny));
-                    } else {
-                        n0 = fma(al3, a[12], fma(al2, a[8], fma(al1, a[4], fma(al0, a[0], tiny))));
-                        n1 = fma(al3, a[13], fma(al2, a[9], fma(al1, a[5], fma(al0, a[1], tiny))));
-                        n2 = fma(al3, a[14], fma(al2, a[10], fma(al1, a[6], fma(al0, a[2], tiny))));
-                        n3 = fma(al3, a[15], fma(al2, a[11], fma(al1, a[7], fma(al0, a[3], tiny))));
-                    }
-                    at0 = fma(n0, b01.x, tiny); at1 = fma(n1, b01.y, tiny);
-                    at2 = fma(n2, b23.x, tiny); at3 = fma(n3, b23.y, tiny);
+                    fwd4_plain<BIDIAG>(a, al0, al1, al2, al3, b01, b23, tiny, n0, n1, n2, n3, at0, at1, at2, at3);
                 } else if (m == 0u) {
                     stop = true;  // no state can emit o_t: log P = -inf (:155-160)
                     n0 = n1 = n2 = n3 = at0 = at1 = at2 = at3 = 0.0;
@@ -292,6 +324,7 @@ __device__ __forceinline__ double fwd4_run(int T, int tmax, const uint4 *__restr
                         ssum = (at0 + at1) + (at2 + at3);
                     }
                     allf = false;
+                    plain = false;
                 }
                 if (!stop) {
                     const double sc = pow2_rescale(ssum, esum);
@@ -328,11 +361,18 @@ __device__ __forceinline__ double fwd4_run(int T, int tmax, const uint4 *__restr
                     if (t == T - 1 && !stop) ll = log((al0 + al1) + (al2 + al3)) + (double)esum * LN2;
                 }
                 // a stopped sequence (impossible, or handed to the exact kernel) is skipped by the backward
-                // pass, so nothing of it needs to be spilled from here on
-                if (SPILL && !stop) {
+                // pass, so nothing of it needs to be spilled from here on; the row of a plain odd step is rebuilt
+                // there from the even row before it (fwd4_rebuild)
+                if (SPILL && !stop && (!(t & 1) || !plain || full)) {
                     __stcs(sp + (size_t)t * 64, make_double2(al0, al1));
                     __stcs(sp + (size_t)t * 64 + 32, make_double2(al2, al3));
+                    wrote = true;
                 }
+            }
+            if (SPILL && (t & 1)) {
+                // which lanes wrote this odd row: one word per (block, odd step), all zeros on data without zeros
+                const unsigned wm = __ballot_sync(0xffffffffu, wrote);
+                if ((threadIdx.x & 31) == 0 && t < tmax) oddmask[t] = wm;
             }
         }
     }
@@ -485,7 +525,7 @@ k_bw_fwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
           const int32_t *__restrict__ len_sorted, const double *__restrict__ pi, const double *__restrict__ A,
           const double *__restrict__ Bt, int M, double2 *__restrict__ spill, double *__restrict__ ll_seq,
           const int32_t *__restrict__ active, uint8_t *__restrict__ flag, uint8_t *__restrict__ allfull, int split,
-          unsigned symmask) {
+          unsigned symmask, unsigned *__restrict__ oddmask, bool full_spill) {
     extern __shared__ double sB[];  // [M][4] B^T, [M] per-codeword max, [M] support masks (u8)
     double *sBmax = sB + (size_t)M * 4;
     unsigned char *sBmask = reinterpret_cast<unsigned char *>(sBmax + M);
@@ -510,7 +550,8 @@ k_bw_fwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
         bool af = false;
         const double ll = fwd4_run<BIDIAG, true>(T, bk.tmax, obs_blk + bk.obs_base + lane, reinterpret_cast<const double2 *>(sB),
                                                  reinterpret_cast<const double2 *>(sB) + M, sBmax, sBmask, a, p, rmax,
-                                                 mk, spill + bk.spill_base * 64 + lane, af, 0, symmask);
+                                                 mk, spill + bk.spill_base * 64 + lane, af, 0, symmask,
+                                                 oddmask + bk.spill_base, full_spill);
         if (T > 0) {
             ll_seq[bk.first + lane] = ll;
             allfull[bk.first + lane] = af ? 1 : 0;
@@ -602,7 +643,7 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc) {
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-constexpr int BWD4_SPILL_PAD = 2;    // rows of padding in front of the alpha spill (see the step macro)
+constexpr int BWD4_SPILL_PAD = 2;    // rows of padding in front of the alpha spill and its odd-row masks (see the step macro)
 constexpr int BWD_L2_PREFETCH = 12;  // steps ahead of use for prefetch.global.L2 of the alpha spill (even)
 __device__ __forceinline__ void prefetch_l2(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 // the same under a predicate instead of a branch (ptxas drains the load scoreboards at the first branch of a loop body
@@ -821,8 +862,10 @@ k_bw_llstat_fix(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, 
 
 // Partial layout per CTA (and accumulator layout per word): [pi N][xi N*N][cnt M*N].
 //
-// The time loop is unrolled by two with fixed roles per parity of t, so that the two-deep
-// alpha-hat prefetch (P0 / P1) needs no register-to-register copies.
+// alpha-hat comes from the spill at even steps; at odd steps it is rebuilt from the even row before it (fwd4_rebuild),
+// except for the lanes the forward pass's mask word of that step names (rows it had to write).  The time loop runs
+// four steps (two pairs) per iteration with fixed roles for the two sets of even-row registers (E0 / E1), so that
+// loading the next pair's row needs no register-to-register copies.
 // MT = 256 (the reference's codebook size, CodeVector/main.py) makes every shared-memory offset a literal;
 // MT = 0 takes M at run time.
 //
@@ -839,9 +882,11 @@ k_bw_bwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
           const int32_t *__restrict__ len_sorted, const double *__restrict__ A, const double *__restrict__ Bt, int M_rt,
           const double2 *__restrict__ spill, const double *__restrict__ ll_seq, const int32_t *__restrict__ active,
           const int32_t *__restrict__ b_has_zero, const uint8_t *__restrict__ allfull, double *__restrict__ partials,
-          int64_t pstride, uint8_t *__restrict__ flag, int32_t *__restrict__ new_flags) {
+          int64_t pstride, uint8_t *__restrict__ flag, int32_t *__restrict__ new_flags,
+          const unsigned *__restrict__ oddmask, bool full_spill) {
     using S16 = Sym<uint16_t>;
     const int M = MT ? MT : M_rt;
+    const int pf_lanes = full_spill ? 16 : 8;  // 128-byte lines of each pair prefetched towards L2
     const int nthreads = blockDim.x, nwarps = nthreads >> 5;
     extern __shared__ double smem[];
     double *sB = smem;                                    // B^T replicated: [M * REP] (b0,b1) then [M * REP] (b2,b3)
@@ -904,28 +949,34 @@ k_bw_bwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
         st.rref = 1.0;
         const uint4 *op = obs_blk + bk.obs_base + lane;
         const double2 *sp = spill + bk.spill_base * 64 + lane;
+        // the block's first row as a 32-bit index (the spill, 1 KB a row, fits in device memory): the mask words are
+        // then addressed from the kernel argument, without a 64-bit pointer held through the time loop
+        const int mrow = (int)bk.spill_base;
         const int nch = (bk.tmax + SPC4 - 1) / SPC4;
-        // alpha-hat registers: P0 holds an even time step, P1 an odd one; every step loads its successor's row
-        double2 P0_01 = make_double2(0.0, 0.0), P0_23 = P0_01, P1_01 = P0_01, P1_23 = P0_01;
+        // Even-step alpha-hat rows and the odd-row lane masks of their pairs (odd 2k + 1, even 2k): pair k is held in
+        // set 0 if k is odd, in set 1 if k is even.  The even step of a pair loads the next pair's row into the other set.
+        double2 E0_01 = make_double2(0.0, 0.0), E0_23 = E0_01, E1_01 = E0_01, E1_23 = E0_01;
+        unsigned M0 = 0u, M1 = 0u;
         {
             // the rows of the block's first BWD_L2_PREFETCH steps are not covered by the prefetch inside the loop
+            // (even rows only, unless every row was written)
             const int r1 = nch * SPC4, r0 = max(r1 - BWD_L2_PREFETCH, 0);
             const char *base = reinterpret_cast<const char *>(sp - lane) + (size_t)r0 * 1024;
-            for (int l = lane; l < (r1 - r0) * 8; l += 32) prefetch_l2(base + (size_t)l * 128);
-            const int ta = bk.tmax - 1;  // the first step of the block
-            if (ta < T) {
-                const double2 x01 = __ldcs(sp + (size_t)ta * 64), x23 = __ldcs(sp + (size_t)ta * 64 + 32);
-                if (ta & 1) { P1_01 = x01; P1_23 = x23; }
-                else        { P0_01 = x01; P0_23 = x23; }
-            }
+            for (int l = lane; l < (r1 - r0) * 8; l += 32)
+                if (full_spill || !((l >> 3) & 1)) prefetch_l2(base + (size_t)l * 128);
+            const int ta = bk.tmax - 1;  // the first step of the block, in pair k = ta / 2
+            const double2 x01 = __ldcs(sp + (size_t)(ta & ~1) * 64), x23 = __ldcs(sp + (size_t)(ta & ~1) * 64 + 32);
+            const unsigned mw = (ta & 1) ? __ldg(oddmask + mrow + ta) : 0u;
+            if ((ta >> 1) & 1) { E0_01 = x01; E0_23 = x23; M0 = mw; }
+            else               { E1_01 = x01; E1_23 = x23; M1 = mw; }
         }
         int wbuf = 0;
         cp_async16(&sW[0][tid], op + (size_t)(nch - 1) * 32);
         cp_async_commit();
 
-// One backward step at time T_ (parity C_ = T_ & 1 is a literal; O_ = the other parity).  PACKED_ = the step's
-// codeword | rank << SYM_BITS.
-#define HMMB_BWD_STEP(T_, C_, O_, SP_, PACKED_)                                                                     \
+// One backward step at time T_ (ODD_ = T_ & 1 is a literal) of the pair held in set X_ (Y_ = the other set).
+// PACKED_ = the step's codeword | rank << SYM_BITS.
+#define HMMB_BWD_STEP(T_, ODD_, X_, Y_, SP_, PACKED_)                                                               \
     {                                                                                                               \
         const int t = (T_);                                                                                         \
         const double2 *spt = (SP_); /* = sp + t * 64: every address below is an immediate offset from it */         \
@@ -933,15 +984,31 @@ k_bw_bwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
         if (t < bk.tmax) { /* warp-uniform */                                                                       \
             const unsigned sym = packed & SYM_MASK;                                                                 \
             const bool act = t < T;                                                                                 \
-            const double al0 = P##C_##_01.x, al1 = P##C_##_01.y, al2 = P##C_##_23.x, al3 = P##C_##_23.y;            \
-            /* alpha-hat of step t - 1 goes straight into the other parity's registers (free since the previous  */ \
-            /* step: no copies).  One step ahead is enough because the rows were pulled into L2 BWD_L2_PREFETCH   */ \
-            /* steps ago.  Unconditional: a row at or beyond a lane's own T is never used, and for t = 0 the     */ \
-            /* load lands in the previous block's tail / the front padding of the spill (BWD4_SPILL_PAD).        */ \
-            P##O_##_01 = __ldcs(spt - 64);                                                                          \
-            P##O_##_23 = __ldcs(spt - 64 + 32);                                                                     \
             const unsigned brow = bbase + sym * (unsigned)(REP * 16);                                               \
             const unsigned crow = cbase + sym * 16u;                                                                \
+            double2 bc01, bc23; /* b(o_t): gathered at the top of an odd step, in the lean path of an even one */   \
+            double al0, al1, al2, al3;                                                                              \
+            if (ODD_) {                                                                                             \
+                /* alpha-hat_t of a plain forward step, rebuilt from the even row t - 1 (fwd4_rebuild); the      */ \
+                /* lanes whose step was not plain wrote their row, and the pair's mask word says which (rare)   */ \
+                bc01 = lds128_ro(brow); bc23 = lds128_ro(brow + B23_OFF);                                           \
+                double2 x01 = E##X_##_01, x23 = E##X_##_23;                                                         \
+                fwd4_rebuild<BIDIAG>(a, x01, x23, bc01, bc23, tiny);                                                \
+                if (M##X_) { /* warp-uniform */                                                                     \
+                    if ((M##X_ >> lane) & 1u) { x01 = __ldcs(spt); x23 = __ldcs(spt + 32); }                        \
+                }                                                                                                   \
+                al0 = x01.x; al1 = x01.y; al2 = x23.x; al3 = x23.y;                                                 \
+            } else {                                                                                                \
+                al0 = E##X_##_01.x; al1 = E##X_##_01.y; al2 = E##X_##_23.x; al3 = E##X_##_23.y;                     \
+                /* the next pair's even row (t - 2) and mask word go straight into the other set (free since the */ \
+                /* odd step of this pair: no copies).  One step ahead of its first use is enough because the rows */\
+                /* were pulled into L2 BWD_L2_PREFETCH steps ago.  Unconditional: a row at or beyond a lane's own */\
+                /* T is never used, and for t = 0 the loads land in the previous block's tail / the front padding */\
+                /* of the spill and of the masks (BWD4_SPILL_PAD).                                               */ \
+                E##Y_##_01 = __ldcs(spt - 128);                                                                     \
+                E##Y_##_23 = __ldcs(spt - 128 + 32);                                                                \
+                M##Y_ = __ldg(oddmask + (mrow + t - 1));                                                            \
+            }                                                                                                       \
             const int rank = (int)(packed >> SYM_BITS);                                                             \
             double g0 = undef_f64(), g1 = undef_f64(), g2 = undef_f64(), g3 = undef_f64();                          \
             if (act) {                                                                                              \
@@ -990,15 +1057,15 @@ k_bw_bwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
                         st.seenX = 0xffffu; /* every alpha_i > 0 and every v_j > 0 */                               \
                         const double sc = pow2_rescale_noacc(qs);                                                   \
                         const double h0 = q0 * sc, h1 = q1 * sc, h2 = q2 * sc, h3 = q3 * sc; /* beta-hat_t */       \
-                        const double2 b01 = lds128_ro(brow), b23 = lds128_ro(brow + B23_OFF);                       \
-                        st.v0 = fma(b01.x, h0, tiny); st.v1 = fma(b01.y, h1, tiny);                                 \
-                        st.v2 = fma(b23.x, h2, tiny); st.v3 = fma(b23.y, h3, tiny);                                 \
+                        if (!(ODD_)) { bc01 = lds128_ro(brow); bc23 = lds128_ro(brow + B23_OFF); }                  \
+                        st.v0 = fma(bc01.x, h0, tiny); st.v1 = fma(bc01.y, h1, tiny);                               \
+                        st.v2 = fma(bc23.x, h2, tiny); st.v3 = fma(bc23.y, h3, tiny);                               \
                         const double vs = (st.v0 + st.v1) + (st.v2 + st.v3);                                        \
                         if ((unsigned)__double2hiint(vs) < LEAN_MIN_HI) { /* tiny emission column: careful v */     \
                             double vv[4];                                                                           \
                             /* (q > 0 on this path: a beta-hat the rescale flushed is still a finite log value) */ \
-                            if (bwd4_v_slow(zero_to_tiny(h0), zero_to_tiny(h1), zero_to_tiny(h2), zero_to_tiny(h3), b01.x, b01.y,       \
-                                            b23.x, b23.y, vv)) st.imprecise = true;   \
+                            if (bwd4_v_slow(zero_to_tiny(h0), zero_to_tiny(h1), zero_to_tiny(h2), zero_to_tiny(h3), bc01.x, bc01.y,     \
+                                            bc23.x, bc23.y, vv)) st.imprecise = true; \
                             st.v0 = vv[0]; st.v1 = vv[1]; st.v2 = vv[2]; st.v3 = vv[3];                             \
                             st.vpos = all_pos4(vv[0], vv[1], vv[2], vv[3]);                                         \
                         }                                                                                           \
@@ -1015,9 +1082,9 @@ k_bw_bwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
                         st.rref = r0;                                                                               \
                         g0 = fma(al0, r0, pos_to_tiny(al0)); g1 = fma(al1, r0, pos_to_tiny(al1));                   \
                         g2 = fma(al2, r0, pos_to_tiny(al2)); g3 = fma(al3, r0, pos_to_tiny(al3));                   \
-                        const double2 b01 = lds128_ro(brow), b23 = lds128_ro(brow + B23_OFF);                       \
-                        st.v0 = b01.x; st.v1 = b01.y; st.v2 = b23.x; st.v3 = b23.y;                                 \
-                        st.vpos = all_pos4(b01.x, b01.y, b23.x, b23.y);                                             \
+                        if (!(ODD_)) { bc01 = lds128_ro(brow); bc23 = lds128_ro(brow + B23_OFF); }                  \
+                        st.v0 = bc01.x; st.v1 = bc01.y; st.v2 = bc23.x; st.v3 = bc23.y;                             \
+                        st.vpos = all_pos4(bc01.x, bc01.y, bc23.x, bc23.y);                                         \
                     } else {                                                                                        \
                         /* the careful step works on a stack copy so that `st` itself never has its address */      \
                         /* taken and stays in registers on the lean path                                     */     \
@@ -1055,16 +1122,24 @@ k_bw_bwd4(const CtaWork *__restrict__ work, const Blk *__restrict__ blks, const 
                 cp_async16(&sW[wbuf][tid], op + (size_t)(c - 1) * 32);
                 cp_async_commit();
             }
+            // two pairs per iteration, so that the two register sets keep fixed roles (pair 2 qq + 1 in set 0)
 #pragma unroll 1
-            for (int pr = SPC4 / 2 - 1; pr >= 0; --pr) {
-                // pull the two alpha-hat rows that will be needed BWD_L2_PREFETCH steps from now (2 KB, contiguous)
-                // towards L2: lanes 0..15 take one 128-byte line each
-                if (c * SPC4 + 2 * pr >= BWD_L2_PREFETCH && lane < 16)
+            for (int qq = SPC4 / 4 - 1; qq >= 0; --qq) {
+                // pull the even alpha-hat row that will be needed BWD_L2_PREFETCH steps from now (1 KB) towards L2:
+                // lanes 0..7 take one 128-byte line each (lanes 8..15 the odd row after it, if every row was written)
+                if (c * SPC4 + 4 * qq + 2 >= BWD_L2_PREFETCH && lane < pf_lanes)
                     prefetch_l2(reinterpret_cast<const char *>(spp) - BWD_L2_PREFETCH * 1024 + lane * (128 - 16));
-                const unsigned p1 = S16::pop_back(w);
-                HMMB_BWD_STEP(c * SPC4 + 2 * pr + 1, 1, 0, spp + 64, p1)
-                const unsigned p0 = S16::pop_back(w);
-                HMMB_BWD_STEP(c * SPC4 + 2 * pr, 0, 1, spp, p0)
+                unsigned p = S16::pop_back(w);
+                HMMB_BWD_STEP(c * SPC4 + 4 * qq + 3, 1, 0, 1, spp + 64, p)
+                p = S16::pop_back(w);
+                HMMB_BWD_STEP(c * SPC4 + 4 * qq + 2, 0, 0, 1, spp, p)
+                spp -= 2 * 64;
+                if (c * SPC4 + 4 * qq >= BWD_L2_PREFETCH && lane < pf_lanes)
+                    prefetch_l2(reinterpret_cast<const char *>(spp) - BWD_L2_PREFETCH * 1024 + lane * (128 - 16));
+                p = S16::pop_back(w);
+                HMMB_BWD_STEP(c * SPC4 + 4 * qq + 1, 1, 1, 0, spp + 64, p)
+                p = S16::pop_back(w);
+                HMMB_BWD_STEP(c * SPC4 + 4 * qq, 0, 1, 0, spp, p)
                 spp -= 2 * 64;
             }
         }
