@@ -79,6 +79,9 @@ SYMBOLS = [
     ("hmmb_score_diagnostics", _c.c_int, [_lp]),
     ("hmmb_viterbi", _c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_void_p, _c.c_int, _c.c_int,
                                 _c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p]),
+    ("hmmb_decode_words", _c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_void_p, _c.c_int64, _c.c_int, _c.c_int,
+                                     _c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_double, _c.c_void_p,
+                                     _c.c_void_p, _c.c_void_p, _c.c_void_p]),
 ]
 
 

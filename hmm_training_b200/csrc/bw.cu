@@ -10,6 +10,7 @@
 #include "bw_kernels.cuh"
 #include "bwltr_kernels.cuh"
 #include "viterbi_kernels.cuh"
+#include "words_kernels.cuh"
 
 namespace hmmb {
 
@@ -2138,6 +2139,140 @@ int hmmb_viterbi(const void *obs, int idx_bytes, int obs_on_device, const int64_
     }
     if (score_out) HMMB_TRY(d2h_big(score_out, d_score, (size_t)U * sizeof(double), c.stream));
     if (want_path) HMMB_TRY(d2h_big(path_out, d_path, (size_t)s.frames, c.stream));
+    HMMB_CUDA(cudaStreamSynchronize(c.stream));
+    return HMMB_OK;
+}
+
+// ---------------------------------------------------------------- connected-word decoding
+template <int SPT, typename SymT>
+static int launch_words_generic(SeqSet &s, int W, int N, double log_penalty, const double *d_lpi, const double *d_lA,
+                                const double *d_lE, double *d_score, int2 *d_rec) {
+    Ctx &c = ctx();
+    const int K = W * N;
+    const int threads = (int)std::min<int64_t>(WORDS_MAX_THREADS, ((K + SPT - 1) / SPT + 31) / 32 * 32);
+    const size_t smem = (size_t)K * 24 + 2 * 32 * sizeof(WordEnd);
+    HMMB_CUDA(cudaFuncSetAttribute((k_wordsG<SPT, SymT>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    HMMB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (k_wordsG<SPT, SymT>), threads, smem));
+    const unsigned grid = (unsigned)std::min<int64_t>(s.R, (int64_t)c.sm_count * std::max(per_sm, 1));
+    HMMB_LAUNCH("words", (k_wordsG<SPT, SymT>), grid, threads, smem, (const SymT *)s.d_obs, s.d_off, s.d_len, s.d_order, s.R,
+                W, N, d_lpi, d_lA, d_lE, log_penalty, d_score, d_rec);
+    return HMMB_OK;
+}
+
+// the fewest states per thread that keep a CTA within WORDS_MAX_THREADS threads
+template <typename SymT>
+static int launch_words_spt(SeqSet &s, int W, int N, double log_penalty, const double *d_lpi, const double *d_lA,
+                            const double *d_lE, double *d_score, int2 *d_rec) {
+    const int K = W * N;
+    if (K <= WORDS_MAX_THREADS) return launch_words_generic<1, SymT>(s, W, N, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec);
+    if (K <= 2 * WORDS_MAX_THREADS) return launch_words_generic<2, SymT>(s, W, N, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec);
+    if (K <= 4 * WORDS_MAX_THREADS) return launch_words_generic<4, SymT>(s, W, N, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec);
+    return launch_words_generic<8, SymT>(s, W, N, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec);
+}
+static_assert(WORDS_MAX_STATES <= 8 * WORDS_MAX_THREADS, "launch_words_spt covers every W * N up to the bound");
+
+// lane = word (W <= 32): G lanes per utterance, 32 / G utterances per warp; the log-emission table in shared memory
+// when it fits the opt-in limit (the reference's shape: 256 x 10 x 4 x 8 B = 80 KB)
+template <int NS, bool BIDIAG, typename SymT>
+static int launch_words_blocked(SeqSet &s, int W, double log_penalty, const double *d_lpi, const double *d_lA,
+                                const double *d_lE, double *d_score, int2 *d_rec) {
+    Ctx &c = ctx();
+    int G = 1;
+    while (G < W) G <<= 1;
+    const int64_t warps_needed = (s.R + 32 / G - 1) / (32 / G);
+    const size_t tab = (size_t)s.M * W * NS * sizeof(double);
+    const bool smem = tab <= (size_t)c.smem_optin;
+    auto launch = [&](auto kern, size_t bytes) -> int {
+        if (bytes) HMMB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        int per_sm = 0;
+        HMMB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WORDSB_THREADS, bytes));
+        const int64_t want = (warps_needed + WORDSB_THREADS / 32 - 1) / (WORDSB_THREADS / 32);
+        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)c.sm_count * std::max(per_sm, 1)));
+        HMMB_LAUNCH("words", kern, grid, WORDSB_THREADS, bytes, (const SymT *)s.d_obs, s.d_off, s.d_len, s.d_order, s.R, W,
+                    G, s.M, d_lpi, d_lA, d_lE, log_penalty, d_score, d_rec);
+        return HMMB_OK;
+    };
+    return smem ? launch(k_wordsB<NS, BIDIAG, true, SymT>, tab) : launch(k_wordsB<NS, BIDIAG, false, SymT>, (size_t)0);
+}
+
+int hmmb_decode_words(const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets, int64_t U, int W, int N,
+                      int M, const double *pi, const double *A, const double *B, double log_penalty, double *score_out,
+                      int64_t *seg_offsets_out, int32_t *seg_word_out, int32_t *seg_start_out) {
+    HMMB_TRY(require_init());
+    if (!pi || !A || !B || W <= 0 || W > 65535 || !std::isfinite(log_penalty) || (!seg_word_out != !seg_start_out)) {
+        set_error("hmmb_decode_words: bad arguments (W=%d, log_penalty=%g; seg_word_out and seg_start_out go together)", W,
+                  log_penalty);
+        return HMMB_ERR_ARG;
+    }
+    if (N >= 1 && N <= HMMB_MAX_STATES && (int64_t)W * N > WORDS_MAX_STATES) {
+        set_error("hmmb_decode_words: W * N = %lld states above the limit of %d", (long long)W * N, WORDS_MAX_STATES);
+        return HMMB_ERR_UNSUPPORTED;
+    }
+    Ctx &c = ctx();
+    if (U == 0 && seg_offsets_out) seg_offsets_out[0] = 0;
+    SeqSet s;
+    CallGuard guard{s, {}};
+    // one codeword stream in length-descending order (a single "word": every utterance meets every model) for either
+    // kernel; the family decision of the scorer picks the lane-per-word kernel for the blocked shapes
+    const Family fam = pick_family(N, M, A, W);
+    const bool blocked = fam.layout() != LAYOUT_LANES && W <= 32;
+    HMMB_TRY(seqset_build(s, obs, idx_bytes, obs_on_device, offsets, nullptr, U, 1, N, M, LAYOUT_LANES));
+    if (U == 0) return HMMB_OK;
+    const size_t nE = (size_t)W * N * M, nA = (size_t)W * N * N, nP = (size_t)W * N;
+    double *tmp = nullptr, *d_lE = nullptr, *d_score = nullptr;
+    HMMB_TRY(dev_alloc_t(&tmp, nE + nA + nP)); guard.ptrs.push_back(tmp);
+    HMMB_TRY(dev_alloc_t(&d_lE, nE + nA + nP)); guard.ptrs.push_back(d_lE);
+    double *d_lA = d_lE + nE, *d_lpi = d_lA + nA;
+    HMMB_TRY(dev_alloc_t(&d_score, (size_t)U)); guard.ptrs.push_back(d_score);
+    HMMB_CUDA(cudaMemcpyAsync(tmp, B, nE * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    HMMB_CUDA(cudaMemcpyAsync(tmp + nE, A, nA * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    HMMB_CUDA(cudaMemcpyAsync(tmp + nE + nA, pi, nP * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+    HMMB_LAUNCH("words_load", k_words_logs, (unsigned)std::min<size_t>((nE + nA + nP + 255) / 256, (size_t)c.sm_count * 8), 256, 0,
+                tmp + 0, tmp + nE, tmp + nE + nA, W, N, M, d_lE, d_lA, d_lpi);
+    // word-end records: one (word, first frame) pair per frame at the frame's input position
+    const bool want_segments = seg_offsets_out || seg_word_out;
+    int2 *d_rec = nullptr;
+    if (want_segments) { HMMB_TRY(dev_alloc_t(&d_rec, (size_t)s.frames)); guard.ptrs.push_back(d_rec); }
+    if (blocked) {
+        auto run = [&](auto sym) -> int {
+            using SymT = decltype(sym);
+            if (N == 4) return fam.bidiag ? launch_words_blocked<4, true, SymT>(s, W, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec)
+                                          : launch_words_blocked<4, false, SymT>(s, W, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec);
+            return N == 8 ? launch_words_blocked<8, true, SymT>(s, W, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec)
+                          : launch_words_blocked<16, true, SymT>(s, W, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec);
+        };
+        HMMB_TRY(s.sym_bytes == 1 ? run(uint8_t{}) : run(uint16_t{}));
+    } else {
+        HMMB_TRY(s.sym_bytes == 1 ? launch_words_spt<uint8_t>(s, W, N, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec)
+                                  : launch_words_spt<uint16_t>(s, W, N, log_penalty, d_lpi, d_lA, d_lE, d_score, d_rec));
+    }
+    if (score_out) HMMB_TRY(d2h_big(score_out, d_score, (size_t)U * sizeof(double), c.stream));
+    if (!want_segments) {
+        HMMB_CUDA(cudaStreamSynchronize(c.stream));
+        return HMMB_OK;
+    }
+    // segment counts -> host, prefix sum, offsets -> device, the segments written at them and copied back
+    std::vector<int64_t> seg_off((size_t)U + 1);
+    int64_t *d_segoff = nullptr;
+    HMMB_TRY(dev_alloc_t(&d_segoff, (size_t)U + 1)); guard.ptrs.push_back(d_segoff);
+    const unsigned bt_grid = (unsigned)((U + WORDS_BT_THREADS - 1) / WORDS_BT_THREADS);
+    HMMB_LAUNCH("words_backtrace", k_words_count, bt_grid, WORDS_BT_THREADS, 0, U, s.d_off, s.d_len, s.d_order, d_score, d_rec,
+                d_segoff + 1);
+    HMMB_TRY(d2h_big(seg_off.data() + 1, d_segoff + 1, (size_t)U * sizeof(int64_t), c.stream));
+    HMMB_CUDA(cudaStreamSynchronize(c.stream));
+    seg_off[0] = 0;
+    for (int64_t u = 0; u < U; ++u) seg_off[u + 1] += seg_off[u];
+    const int64_t nseg = seg_off[U];
+    if (seg_offsets_out) std::copy(seg_off.begin(), seg_off.end(), seg_offsets_out);
+    if (!seg_word_out || nseg == 0) return HMMB_OK;
+    int32_t *d_seg = nullptr;
+    HMMB_TRY(dev_alloc_t(&d_seg, (size_t)nseg * 2)); guard.ptrs.push_back(d_seg);
+    HMMB_CUDA(cudaMemcpyAsync(d_segoff, seg_off.data(), ((size_t)U + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, c.stream));
+    HMMB_LAUNCH("words_backtrace", k_words_emit, bt_grid, WORDS_BT_THREADS, 0, U, s.d_off, s.d_len, s.d_order, d_segoff, d_rec,
+                d_seg, d_seg + nseg);
+    HMMB_TRY(d2h_big(seg_word_out, d_seg, (size_t)nseg * sizeof(int32_t), c.stream));
+    HMMB_TRY(d2h_big(seg_start_out, d_seg + nseg, (size_t)nseg * sizeof(int32_t), c.stream));
     HMMB_CUDA(cudaStreamSynchronize(c.stream));
     return HMMB_OK;
 }

@@ -332,3 +332,39 @@ def viterbi(obs, offsets, model_of_utt, N: int, M: int, pi, A, B, want_path: boo
     check(lib.hmmb_viterbi(op, ib, on_dev, ptr(offsets), U, ptr(model_of_utt), W, N, M, ptr(pi), ptr(A), ptr(B),
                            ptr(score), ptr(path)))
     return score[:U], (path[:frames] if want_path else None)
+
+
+def decode_words(obs, offsets, N: int, M: int, pi, A, B, log_penalty: float = 0.0, want_segments: bool = True,
+                 obs_dev_ptr: Optional[int] = None, idx_bytes: Optional[int] = None):
+    """Connected-word recognition (hmmb_decode_words; an extension, the reference recognises one word per
+    recording): the best word sequence of every utterance over a free loop of the W models pi [W,N], A [W,N,N],
+    B [W,N,M] (linear).  A word is entered in any state and left from its last state; log_penalty is added once per
+    recognised word.
+
+    Returns (score float64 [U], seg_offsets int64 [U+1], seg_word int32 [S], seg_start int32 [S]): the segments of
+    utterance u are [seg_offsets[u], seg_offsets[u+1]), in time order, each a word index and its first frame relative
+    to the utterance (the segment ends one frame before the next one starts).  score[u] is -inf, with no segments,
+    for an impossible utterance.  want_segments=False decodes the scores only and returns None for the other three."""
+    lib = _lib.load()
+    pi, A, B = c_f64(pi), c_f64(A), c_f64(B)
+    W = pi.shape[0]
+    if pi.shape != (W, N) or A.shape != (W, N, N) or B.shape != (W, N, M):
+        raise ValueError("model parameter shapes do not match (W, N, M)")
+    if not np.isfinite(log_penalty):
+        raise ValueError("log_penalty must be finite")
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+    U = len(offsets) - 1
+    op, on_dev, ib, obs = _codewords(obs, obs_dev_ptr, idx_bytes)
+    frames = int(offsets[-1] - offsets[0]) if U > 0 else 0
+    score = np.empty(max(U, 1))
+    seg_off = seg_word = seg_start = None
+    if want_segments:
+        seg_off = np.zeros(U + 1, dtype=np.int64)
+        seg_word = np.empty(max(frames, 1), dtype=np.int32)
+        seg_start = np.empty(max(frames, 1), dtype=np.int32)
+    check(lib.hmmb_decode_words(op, ib, on_dev, ptr(offsets), U, W, N, M, ptr(pi), ptr(A), ptr(B), float(log_penalty),
+                                ptr(score), ptr(seg_off), ptr(seg_word), ptr(seg_start)))
+    if not want_segments:
+        return score[:U], None, None, None
+    nseg = int(seg_off[-1])
+    return score[:U], seg_off, seg_word[:nseg].copy(), seg_start[:nseg].copy()

@@ -3,8 +3,10 @@
     calculate_log_likelihood   HMM/hmm_testing.py:49-104
     test_hmm                   HMM/hmm_testing.py:107-163
     create_confusion_matrix    HMM/hmm_testing.py:166-218
-plus ``score_all`` (every utterance against every model in one launch) and ``viterbi_align`` (the most
-likely state path of every utterance under a chosen model; an extension, the reference has no Viterbi).
+plus ``score_all`` (every utterance against every model in one launch), ``viterbi_align`` (the most
+likely state path of every utterance under a chosen model; an extension, the reference has no Viterbi) and
+``recognize_connected`` (the best word sequence of every utterance; an extension, the reference recognises one word
+per recording).
 """
 from __future__ import annotations
 
@@ -90,6 +92,32 @@ def viterbi_align(observations: Sequence[np.ndarray], all_hmm: Sequence[HMMTrain
         for k, u in enumerate(utts):
             paths[u] = path[offsets[k]:offsets[k + 1]].copy()
     return scores, paths
+
+
+def recognize_connected(observations: Sequence[np.ndarray], all_hmm: Sequence[HMMTrained], log_penalty: float = 0.0):
+    """Connected-word recognition: the best sequence of words from all_hmm (a free word loop, any word after any
+    other) for every utterance, in one decode on the GPU (engine.decode_words).  log_penalty (natural log) is added
+    once per recognised word: negative values favour fewer, longer words.
+
+    Returns (scores float64 [U], one list per utterance of (word, first_frame, last_frame) with the word named by
+    HMMTrained.word).  An utterance that no word sequence can produce gets -inf and an empty list.  One decode needs
+    one model shape, so models of different (states, symbols) raise ValueError."""
+    seqs = [np.asarray(o) for o in observations]
+    if any(len(o) == 0 for o in seqs):
+        raise IndexError("index 0 is out of bounds for axis 0 with size 0")  # as score_all (hmm_testing.py:75)
+    if len({(int(h.states), int(h.symbols)) for h in all_hmm}) > 1:
+        raise ValueError("connected-word recognition needs models of one (states, symbols) shape")
+    if not all_hmm:
+        raise ValueError("no word models")
+    N, M, pi, A, B = _stack_models(all_hmm)
+    obs, offsets = _lib.pack_sequences(seqs, M)
+    scores, seg_off, seg_word, seg_start = engine.decode_words(obs, offsets, N, M, pi, A, B, log_penalty)
+    words = []
+    for u, o in enumerate(seqs):
+        a, b = int(seg_off[u]), int(seg_off[u + 1])
+        ends = list(seg_start[a + 1:b] - 1) + [len(o) - 1]
+        words.append([(all_hmm[int(seg_word[k])].word, int(seg_start[k]), int(ends[k - a])) for k in range(a, b)])
+    return scores, words
 
 
 def calculate_log_likelihood(recording_observations: np.ndarray, hmm: HMMTrained) -> float:

@@ -242,6 +242,39 @@ int hmmb_viterbi(const void *obs, int idx_bytes, int obs_on_device, const int64_
                  const int32_t *model_of_utt, int W, int N, int M, const double *pi, const double *A,
                  const double *B, double *score_out, int8_t *path_out);
 
+/* ------------------------------------------------------------------ connected-word decoding
+ * An extension: the reference recognises one word per recording.  The best word sequence of every utterance over a
+ * free loop of W isolated-word models (one-pass dynamic programming: Vintsyuk; Bridle, Brown and Chamberlain; Rabiner &
+ * Juang ch. 7), from LINEAR pi [W,N], A [W,N,N], B [W,N,M] (entries <= 0 or NaN are structural zeros, log = -inf).
+ * A word is entered in any state j with log pi_j and left only from its last state N - 1 (the exit of a left-to-right
+ * model); a silence model may be passed as one more word.  log_penalty (natural log, any sign, finite) is added once per
+ * recognised word.  With lpi / lA / lb the logs, all additions happen in exactly this order:
+ *     delta_0(w,j) = lpi[w][j] + lb[w][j](o_0)                                   token_0(w,j) = 0
+ *     t >= 1:  in(w,j)      = max_i (delta_t-1(w,i) + lA[w][i][j])   (smallest i on ties)
+ *              en(w,j)      = E_t-1 + lpi[w][j]
+ *              delta_t(w,j) = (en > in ? en : in) + lb[w][j](o_t)    (the entry wins only when strictly larger)
+ *              token_t(w,j) = en > in ? t : token_t-1(w, argmax i)
+ *     e_t = max_w delta_t(w, N-1) (smallest w on ties),  E_t = e_t + log_penalty,  record_t = (argmax w, its token)
+ *     score_out[u] = E_T-1
+ * Backtrace: record_T-1 = (w, s) is the segment "word w on frames [s, T-1]"; it continues at t = s - 1 until t < 0.
+ * The segments' log-probability is the sum of their best in-word paths plus K * log_penalty for K words.  An
+ * utterance with score -inf is impossible and has no segments; T = 1 gives one segment.  For a one-word utterance the
+ * score is not hmmb_viterbi's, which lets any state end the utterance.  The recursion only adds and compares log values,
+ * so it needs no precision guard.
+ * Outputs (each nullable): score_out [U]; seg_offsets_out [U+1], the segments of u are [seg_offsets_out[u],
+ * seg_offsets_out[u+1]); seg_word_out / seg_start_out (both or neither) the word and the first frame (relative to the
+ * utterance) of every segment, compact and in time order, capacity offsets[U] - offsets[0] (a bound on the segment
+ * count); only seg_offsets_out[U] entries are written.  With all three segment outputs NULL no word-end records are
+ * stored and no backtrace runs; score_out is then bit-identical to the call with segments.
+ * obs / idx_bytes / obs_on_device / offsets as for hmmb_score.  1 <= N <= 32, 1 <= M <= 65536, 1 <= W <= 65535 and
+ * W * N <= 8192 (the decoder keeps 24 bytes of shared memory per state).
+ * Errors: HMMB_ERR_RANGE (codeword >= M), HMMB_ERR_EMPTY (empty utterance), HMMB_ERR_ARG (null parameters, W outside
+ * [1, 65535], non-finite log_penalty, only one of seg_word_out / seg_start_out), HMMB_ERR_UNSUPPORTED (N or M out of
+ * range, W * N > 8192), HMMB_ERR_OOM (the word-end records take 8 bytes per frame).                                 */
+int hmmb_decode_words(const void *obs, int idx_bytes, int obs_on_device, const int64_t *offsets, int64_t U,
+                      int W, int N, int M, const double *pi, const double *A, const double *B, double log_penalty,
+                      double *score_out, int64_t *seg_offsets_out, int32_t *seg_word_out, int32_t *seg_start_out);
+
 /* ------------------------------------------------------------------ MFCC front-end
  * Replaces RawDataMFCC.calculate_mfcc, CodeVector/codevector_classes.py:226-250, batched: F frames
  * of L samples each (Y [F,L] fp64, host or device) -> mfcc_out [F,13] (host), the coefficients of
